@@ -7,6 +7,7 @@ Metric (BASELINE.json): Lotka-Volterra two-level delayed-acceptance chain-steps/
   python bench.py --gpus 1 --steps K --warmup W            # our arm
   python bench.py --impl reference --steps K --warmup W    # CPU arm (oracle port, all host threads)
   torchrun ... bench.py --gpus N ...                        # one rank per GPU, NCCL
+  python bench.py ... --dump-outputs DIR                    # also write the timed path's final chain state as .npy
 
 A "step" is one pass of the hot path over the whole ensemble: one yg_run launch
 of `--transitions` (default 300) Metropolis-Hastings transitions of every chain, so that the
@@ -290,6 +291,9 @@ def run_gpu_arm(args):
     ms = [a.elapsed_time(b) for (a, b) in evs]
     total_ms = float(sum(ms))
     c1 = ens.counters()
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {k: v.double().cpu().numpy() for k, v in ens.state().items() if torch.is_tensor(v)},
+                     f"_rank{rank}" if world > 1 else "")
     launches = ens.last_launch()["launches"] - l0
     t = torch.tensor([total_ms], dtype=torch.float64, device=dev)
     evals = torch.tensor([c1["coarse_evals"] - c0["coarse_evals"], c1["fine_evals"] - c0["fine_evals"],
@@ -754,6 +758,25 @@ def measure_other_configs(device, fp64_peak, main_value, hbm_peak_gbs):
     return out
 
 
+DUMP_LIMIT_BYTES = 64 * 1024 * 1024
+
+
+def dump_outputs(out_dir, arrays, suffix=""):
+    """Writes the chain state the timed steps leave behind (ChainEnsemble.state(): theta [d, n], logpost [levels, n],
+    n_accept [n], Welford w_mean [d, n] and w_m2; chains on the last axis) as out_dir/<name><suffix>.npy in float64,
+    so that two builds can be compared output for output.  Above DUMP_LIMIT_BYTES in all, a fixed seeded sample of
+    the chains is written instead, and its chain indices as chain_index.npy."""
+    n = arrays["theta"].shape[-1]
+    per_chain = 8 * sum(a.size // n for a in arrays.values())
+    if n * per_chain > DUMP_LIMIT_BYTES:
+        keep = np.sort(np.random.default_rng(0).choice(n, DUMP_LIMIT_BYTES // (per_chain + 8), replace=False))
+        arrays = {k: a[..., keep] for k, a in arrays.items()}
+        arrays["chain_index"] = keep
+    os.makedirs(out_dir, exist_ok=True)
+    for k, a in arrays.items():
+        np.save(os.path.join(out_dir, k + suffix + ".npy"), np.ascontiguousarray(a, dtype=np.float64))
+
+
 _JSON_OUT = None
 
 
@@ -795,7 +818,13 @@ def main():
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-cpu", action="store_true")
     ap.add_argument("--no-configs", action="store_true", help="skip the brief timing of the other BASELINE.json configs")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write the chain state they computed "
+                    "(theta, log-posterior, accept counts, Welford moments) as DIR/<name>.npy, float64, at most 64 MB")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs applies to the GPU arm (the CPU arm sizes its sample from the measured rate)")
     if args.warmup < 3:
         args.warmup = 3 if args.impl == "b200" else args.warmup
     if args.impl == "reference":

@@ -37,6 +37,46 @@ def test_reference_arm_line():
     assert py["rk4_plugin"]["chain_steps_per_s_per_core"] > 0 and "NOT on this box" in py["measured_in"]
 
 
+def test_dump_outputs_are_float64_and_capped(tmp_path, monkeypatch):
+    """--dump-outputs writes one float64 .npy per array; above the cap, the same seeded sample of chains every time."""
+    import numpy as np
+    import bench
+    n = 1000
+    state = {"theta": np.arange(2.0 * n).reshape(2, n), "n_accept": np.arange(n, dtype=np.int64)}
+    bench.dump_outputs(str(tmp_path / "full"), state)
+    assert np.array_equal(np.load(tmp_path / "full" / "n_accept.npy"), np.arange(n))
+    assert sorted(p.name for p in (tmp_path / "full").iterdir()) == ["n_accept.npy", "theta.npy"]
+    monkeypatch.setattr(bench, "DUMP_LIMIT_BYTES", 8 * 1024)
+    for out in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / out), state, "_rank1")
+    files = {p.name: np.load(p) for p in (tmp_path / "a").iterdir()}
+    assert set(files) == {"theta_rank1.npy", "n_accept_rank1.npy", "chain_index_rank1.npy"}
+    assert all(a.dtype == np.float64 for a in files.values()) and sum(a.nbytes for a in files.values()) <= 8 * 1024
+    keep = files["chain_index_rank1.npy"].astype(np.int64)
+    assert len(keep) > 0 and np.array_equal(files["theta_rank1.npy"], state["theta"][:, keep])
+    assert np.array_equal(keep, np.load(tmp_path / "b" / "chain_index_rank1.npy"))
+
+
+@pytest.mark.gpu
+@pytest.mark.timeout(300)
+def test_b200_arm_dumps_the_same_outputs_for_the_same_arguments(tmp_path):
+    """Two runs with the same arguments compute the same chain state, bit for bit: what --dump-outputs writes can
+    compare two builds of the project."""
+    import numpy as np
+    args = ["--steps", "2", "--warmup", "3", "--chains", "8192", "--transitions", "10",
+            "--no-ess", "--no-e2e", "--no-cpu", "--no-configs", "--dump-outputs"]
+    for out in ("a", "b"):
+        d = _run(args + [str(tmp_path / out)], 280)
+        assert d["steps"] == 2
+    names = sorted(p.name for p in (tmp_path / "a").iterdir())
+    assert names == ["logpost.npy", "n_accept.npy", "theta.npy", "w_m2.npy", "w_mean.npy"]
+    for name in names:
+        a, b = np.load(tmp_path / "a" / name), np.load(tmp_path / "b" / name)
+        assert a.dtype == np.float64 and a.shape[-1] == 8192 and np.array_equal(a, b, equal_nan=True), name
+    theta = np.load(tmp_path / "a" / "theta.npy")
+    assert theta.shape == (2, 8192) and np.isfinite(theta).all()
+
+
 @pytest.mark.gpu
 @pytest.mark.timeout(300)
 def test_b200_arm_line():
