@@ -69,3 +69,31 @@ def test_no_cpu_fallback():
         prop_L=[[1.0]], L0_g_mean=[0.0], L0_g_prec=[[1.0]], L0_g_logconst=0.0))
     with pytest.raises(_lib.BackendUnavailable):
         ChainEnsemble(pb, 4)
+
+
+def test_state_layout_names_every_yg_state_field():
+    from yagre_mcmc_b200.ensemble import state_layout
+    lay = state_layout(6, 3, 2, True, 4)
+    assert [k + "_dev" for k in lay] == [f for f, _ in _lib.YgState._fields_]
+
+
+def test_check_state_accepts_exactly_the_layout():
+    """What load_state checks before a pointer reaches yg_load_state, which copies the layout's byte count from each."""
+    import torch
+    from yagre_mcmc_b200.ensemble import check_state, state_layout
+    n, d = 6, 3
+    for lay in (state_layout(n, d, 2, True, 4), state_layout(n, 12, 1, False, 0)):
+        good = {k: torch.zeros(shape, dtype=dtype) for k, (shape, dtype) in lay.items()}
+        check_state(good, lay)
+        check_state(dict(theta=good["theta"], logpost=good["logpost"], step_index=3), lay)
+        for k in ("theta", "logpost"):
+            with pytest.raises(ValueError):
+                check_state({j: v for j, v in good.items() if j != k}, lay)
+        for k, v in good.items():
+            bad = [torch.zeros((v.shape[0] + 1,) + tuple(v.shape[1:]), dtype=v.dtype),      # oversized
+                   v.to(torch.float32), v.to(torch.float64 if v.dtype == torch.int64 else torch.int64), v.numpy()]
+            if v.dim() > 1:
+                bad.append(v.transpose(0, -1))
+            for b in bad:
+                with pytest.raises(ValueError, match=k):
+                    check_state(dict(good, **{k: b}), lay)

@@ -178,6 +178,46 @@ def test_checkpoint_files_and_trajectory_dump(tmp_path):
     assert np.array_equal(mm[-1], back[-1])
 
 
+def test_load_state_rejects_misshapen_arrays():
+    """load_state checks every array against the ensemble's layout before yg_load_state copies from it (each array
+    here is at least as large as that copy, so nothing reads out of bounds whatever the check does)."""
+    meta, arrays = bp.linear_problem(True)
+    nc = 64
+    a = _ens(meta, arrays, nc, seed=8)
+    a.set_state(np.zeros((nc, 2)))
+    a.run(5, samples=False)
+    st = a.state()
+    b = _ens(meta, arrays, nc, seed=8)
+    for theta in (st["theta"].t().contiguous(), torch.zeros(3, nc, dtype=torch.float64, device=st["theta"].device)):
+        with pytest.raises(ValueError, match="theta"):
+            b.load_state(dict(st, theta=theta))
+    with pytest.raises(ValueError, match="logpost"):
+        b.load_state({k: v for k, v in st.items() if k != "logpost"})
+    b.load_state(st)
+    assert torch.equal(b.state()["theta"], st["theta"])
+
+
+def test_failed_set_problem_leaves_the_handle_unchanged():
+    """A tensor-path handle (data_dim 16) given a one-chain-per-thread problem that fails validation keeps its problem:
+    the same log-posteriors, and it still runs."""
+    import ctypes as C
+    from yagre_mcmc_b200 import _lib
+    from yagre_mcmc_b200.ensemble import LoweredProblem
+    meta, arrays = bp.big_linear_problem(2, 16, 1)
+    nc = 64
+    ens = _ens(meta, arrays, nc, seed=12)
+    pts = np.random.default_rng(0).standard_normal((8, 2))
+    before = ens.logpost(0, pts)
+    small_meta, small_arrays = bp.linear_problem(False)
+    small = LoweredProblem(dict(small_meta, proposal="pcn", pcn_step=0.7), small_arrays)
+    pb = small.c_struct()
+    assert ens.lib.yg_set_problem(ens._h, C.byref(pb)) == _lib.YG_ERR_INVALID
+    assert torch.equal(ens.logpost(0, pts), before)
+    ens.set_state(np.zeros((nc, 2)))
+    ens.run(10, samples=False)
+    assert ens.counters()["transitions"] == nc * 10
+
+
 def test_thinning_and_outputs():
     meta, arrays = bp.lv_problem(True, Nc=16, Nf=64)
     nc = 200

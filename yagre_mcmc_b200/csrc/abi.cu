@@ -24,6 +24,55 @@ namespace {
 
 constexpr int POOL_PARTS = 64;
 
+// The per-chain state buffers, one row per StateBuf: the yg_state field, the bytes of one element, the elements per
+// chain as a function of the parameter dimension d and the adaptive error model's data dimension dd, and the group.
+// ALWAYS and DIAG buffers exist in every handle, AM buffers if cfg.adaptive, AEM buffers if cfg.aem (allocated by
+// yg_set_problem, which learns dd).  yg_set_state zeroes DIAG unless YG_KEEP_DIAGNOSTICS, AM and AEM unless
+// YG_KEEP_ADAPTATION.
+enum Group { ALWAYS, DIAG, AM, AEM };
+struct StateSpec {
+    size_t field;                               // offsetof(yg_state, ..._dev)
+    size_t elem;
+    size_t (*per_chain)(size_t d, size_t dd);
+    Group group;
+};
+const StateSpec kState[SB_COUNT] = {
+    {offsetof(yg_state, theta_dev), sizeof(double), [](size_t d, size_t) { return d; }, ALWAYS},
+    {offsetof(yg_state, logpost_dev), sizeof(double), [](size_t, size_t) { return (size_t)YG_MAX_LEVELS; }, ALWAYS},
+    {offsetof(yg_state, n_accept_dev), sizeof(unsigned long long), [](size_t, size_t) { return (size_t)1; }, DIAG},
+    {offsetof(yg_state, w_mean_dev), sizeof(double), [](size_t d, size_t) { return d; }, DIAG},
+    // the large linear model keeps the diagonal of the Welford M2 only (big_linear.h)
+    {offsetof(yg_state, w_m2_dev), sizeof(double), [](size_t d, size_t) { return d > YG_MAX_DIM ? d : d * d; }, DIAG},
+    {offsetof(yg_state, prop_L_dev), sizeof(double), [](size_t d, size_t) { return d * d; }, AM},
+    {offsetof(yg_state, am_mean_dev), sizeof(double), [](size_t d, size_t) { return d; }, AM},
+    {offsetof(yg_state, am_m2_dev), sizeof(double), [](size_t d, size_t) { return d * d; }, AM},
+    {offsetof(yg_state, aem_n_dev), sizeof(unsigned long long), [](size_t, size_t) { return (size_t)1; }, AEM},
+    {offsetof(yg_state, aem_mean_dev), sizeof(double), [](size_t, size_t dd) { return dd; }, AEM},
+    {offsetof(yg_state, aem_m2_dev), sizeof(double), [](size_t, size_t dd) { return dd; }, AEM},
+    {offsetof(yg_state, aem_cache_dev), sizeof(double), [](size_t d, size_t) { return 3 * (d + 1) + 1; }, AEM},
+};
+
+bool has_group(const yg_ensemble *e, Group g) { return g == AM ? e->cfg.adaptive : (g == AEM ? e->cfg.aem : true); }
+
+size_t buf_bytes(const yg_ensemble *e, int b)
+{
+    const StateSpec &s = kState[b];
+    return s.elem * s.per_chain((size_t)e->cfg.dim, (size_t)e->aem_data_dim) * (size_t)e->cfg.n_chains;
+}
+
+// Bytes yg_get_state / yg_load_state copy: the state holds n_levels of logpost's YG_MAX_LEVELS rows.
+size_t state_bytes(const yg_ensemble *e, int b)
+{
+    return b == SB_LOGPOST ? sizeof(double) * e->cfg.n_levels * e->cfg.n_chains : buf_bytes(e, b);
+}
+
+void *state_ptr(const yg_state *s, int b)
+{
+    void *p;
+    memcpy(&p, reinterpret_cast<const char *>(s) + kState[b].field, sizeof(p));
+    return p;
+}
+
 int check_handle(const yg_ensemble *e, bool need_problem, bool need_state)
 {
     if (!e) {
@@ -41,11 +90,23 @@ int check_handle(const yg_ensemble *e, bool need_problem, bool need_state)
     return YG_OK;
 }
 
-template <typename T>
-int dev_alloc(T **p, size_t n)
+int dev_alloc(void **p, size_t bytes)
 {
-    YG_CUDA_CHECK(cudaMalloc((void **)p, sizeof(T) * std::max<size_t>(n, 1)));
-    YG_CUDA_CHECK(cudaMemset(*p, 0, sizeof(T) * std::max<size_t>(n, 1)));
+    YG_CUDA_CHECK(cudaMalloc(p, bytes));
+    YG_CUDA_CHECK(cudaMemset(*p, 0, bytes));
+    return YG_OK;
+}
+
+// (Re)allocates the buffers of group g, zeroed.
+int alloc_group(yg_ensemble *e, Group g)
+{
+    for (int b = 0; b < SB_COUNT; b++) {
+        if (kState[b].group != g) continue;
+        cudaFree(e->buf[b]);
+        e->buf[b] = nullptr;
+        const int rc = dev_alloc(&e->buf[b], buf_bytes(e, b));
+        if (rc) return rc;
+    }
     return YG_OK;
 }
 
@@ -58,7 +119,7 @@ RunArgs make_args(yg_ensemble *e)
 {
     RunArgs a;
     memset(&a, 0, sizeof(a));
-    a.problem = e->d_problem;
+    a.problem = static_cast<const DevProblemHeader *>(e->d_problem);    // the tensor path passes its header itself
     a.problem_bytes = (uint32_t)e->h_problem.size();
     a.thin = 1;
     a.n_chains = e->cfg.n_chains;
@@ -67,14 +128,14 @@ RunArgs make_args(yg_ensemble *e)
     a.step0 = e->step_index;
     a.welford_n0 = e->welford_n;
     a.am_t0 = e->am_steps;
-    a.theta = e->theta;
-    a.logpost = e->logpost;
-    a.n_accept = e->n_accept;
-    a.w_mean = e->w_mean;
-    a.w_m2 = e->w_m2;
-    a.am_mean = e->am_mean;
-    a.am_m2 = e->am_m2;
-    a.prop_L = e->prop_L;
+    a.theta = static_cast<double *>(e->buf[SB_THETA]);
+    a.logpost = static_cast<double *>(e->buf[SB_LOGPOST]);
+    a.n_accept = static_cast<unsigned long long *>(e->buf[SB_N_ACCEPT]);
+    a.w_mean = static_cast<double *>(e->buf[SB_W_MEAN]);
+    a.w_m2 = static_cast<double *>(e->buf[SB_W_M2]);
+    a.am_mean = static_cast<double *>(e->buf[SB_AM_MEAN]);
+    a.am_m2 = static_cast<double *>(e->buf[SB_AM_M2]);
+    a.prop_L = static_cast<double *>(e->buf[SB_PROP_L]);
     a.adaptive = e->cfg.adaptive;
     a.am_refresh = std::max(1, e->cfg.am_refresh);
     a.am_idle = e->cfg.am_idle_steps;
@@ -85,10 +146,10 @@ RunArgs make_args(yg_ensemble *e)
     a.aem_min_data = e->cfg.aem_min_data;
     a.aem_heuristic = e->cfg.aem_heuristic;
     a.welford = e->cfg.acceptance_only ? 0 : 1;
-    a.aem_n = e->aem_n;
-    a.aem_mean = e->aem_mean;
-    a.aem_m2 = e->aem_m2;
-    a.aem_cache = e->aem_cache;
+    a.aem_n = static_cast<unsigned long long *>(e->buf[SB_AEM_N]);
+    a.aem_mean = static_cast<double *>(e->buf[SB_AEM_MEAN]);
+    a.aem_m2 = static_cast<double *>(e->buf[SB_AEM_M2]);
+    a.aem_cache = static_cast<double *>(e->buf[SB_AEM_CACHE]);
     a.counters = e->counters;
     return a;
 }
@@ -100,6 +161,16 @@ __global__ void broadcast_L_kernel(const DevProblemHeader *pb, double *prop_L, i
         for (int k = 0; k < d * d; k++) prop_L[(int64_t)k * n + g] = pb->prop_L[k];
 }
 
+// Every chain of an adaptive ensemble restarts from the problem's proposal factor.
+int broadcast_prop_L(yg_ensemble *e, cudaStream_t st)
+{
+    const size_t n = (size_t)e->cfg.n_chains;
+    broadcast_L_kernel<<<(int)std::min<size_t>((n + 127) / 128, 2048), 128, 0, st>>>(
+        static_cast<const DevProblemHeader *>(e->d_problem), static_cast<double *>(e->buf[SB_PROP_L]), (int64_t)n);
+    YG_CUDA_CHECK(cudaGetLastError());
+    return YG_OK;
+}
+
 bool is_diagonal(const double *M, int n)
 {
     for (int i = 0; i < n; i++)
@@ -108,28 +179,17 @@ bool is_diagonal(const double *M, int n)
     return true;
 }
 
-// Large linear model: builds the DevBigHeader blob (big_linear.h) for linear_dmma_kernel.cu.
-int set_problem_big(yg_ensemble *e, const yg_problem *pb)
+// The blob builders read the configuration and the problem only.  yg_set_problem has checked the proposal kind, the
+// pCN rules and that prop_L is lower triangular.
+
+// Large linear model: the DevBigHeader blob (big_linear.h) of linear_dmma_kernel.cu.
+int build_big_blob(const yg_config &c, const yg_problem *pb, std::vector<char> &blob)
 {
-    const int d = e->cfg.dim, nl = e->cfg.n_levels;
-    if (e->cfg.adaptive || e->cfg.eq_mode != YG_EQ_EXACT || e->cfg.aem || nl > 2) {
+    const int d = c.dim, nl = c.n_levels;
+    if (c.adaptive || c.eq_mode != YG_EQ_EXACT || c.aem || nl > 2) {
         yg_set_error("large linear model (dim > %d or data_dim > %d): MRW / pCN / two-level delayed acceptance with exact "
                      "equality only (no adaptive proposal, adaptive error model or third level)", YG_MAX_DIM, YG_MAX_DATA_DIM);
         return YG_ERR_UNSUPPORTED;
-    }
-    if (pb->proposal != YG_PROPOSAL_MRW && pb->proposal != YG_PROPOSAL_PCN) {
-        yg_set_error("unknown proposal kind %d", pb->proposal);
-        return YG_ERR_INVALID;
-    }
-    if (pb->proposal == YG_PROPOSAL_PCN) {
-        if (!(pb->pcn_step > 0.0 && pb->pcn_step <= 0.5)) {       // pcn.py:42
-            yg_set_error("pCN step size must lie in (0, 0.5], got %g", pb->pcn_step);
-            return YG_ERR_INVALID;
-        }
-        if (nl != 1) {
-            yg_set_error("pCN is a single-level method (chain/method/pcn.py)");
-            return YG_ERR_UNSUPPORTED;
-        }
     }
     for (int l = 0; l < nl; l++)
         if (pb->level[l].tempered) {
@@ -137,12 +197,6 @@ int set_problem_big(yg_ensemble *e, const yg_problem *pb)
             return YG_ERR_UNSUPPORTED;
         }
     const bool dense_L = !is_diagonal(pb->prop_L, d);
-    for (int i = 0; i < d; i++)
-        for (int j = i + 1; j < d; j++)
-            if (pb->prop_L[(size_t)i * d + j] != 0.0) {
-                yg_set_error("prop_L must be lower triangular");
-                return YG_ERR_INVALID;
-            }
     const int kp = d <= 16 ? 16 : (d <= 32 ? 32 : 64), ks = kp + 4;
     size_t tail_len = 0;
     bool dense_prior[2] = {false, false};
@@ -203,11 +257,11 @@ int set_problem_big(yg_ensemble *e, const yg_problem *pb)
             return YG_ERR_UNSUPPORTED;
         }
     }
-    std::vector<char> blob(sizeof(DevBigHeader) + sizeof(double) * tail_len, 0);
+    blob.assign(sizeof(DevBigHeader) + sizeof(double) * tail_len, 0);
     DevBigHeader *h = reinterpret_cast<DevBigHeader *>(blob.data());
     double *tail = reinterpret_cast<double *>(blob.data() + sizeof(DevBigHeader));
     h->dim = d; h->kp = kp; h->ks = ks; h->n_levels = nl;
-    h->J = nl == 2 ? e->cfg.sub_chain_length : 1;
+    h->J = nl == 2 ? c.sub_chain_length : 1;
     h->tail_len = (int32_t)tail_len;
     h->proposal = pb->proposal;
     h->dense_L = dense_L ? 1 : 0;
@@ -275,19 +329,6 @@ int set_problem_big(yg_ensemble *e, const yg_problem *pb)
     if (dense_L)
         for (int r = 0; r < d; r++)
             for (int k = 0; k <= r; k++) tail[off + (size_t)r * ks + k] = pb->prop_L[(size_t)r * d + k];
-    YG_CUDA_CHECK(cudaSetDevice(e->cfg.device));
-    e->problem_set = false;
-    if (e->d_problem) cudaFree(e->d_problem);
-    e->d_problem = nullptr;
-    YG_CUDA_CHECK(cudaMalloc((void **)&e->d_problem, blob.size()));
-    YG_CUDA_CHECK(cudaMemcpy(e->d_problem, blob.data(), blob.size(), cudaMemcpyHostToDevice));
-    if (!e->big_done) {     // per-tile progress counters of the balanced (tile, step-range) schedule
-        int rc = dev_alloc(&e->big_done, ((size_t)e->cfg.n_chains + 7) / 8);
-        if (rc) return rc;
-    }
-    e->h_problem.swap(blob);
-    e->problem_set = true;
-    e->big = true;
     return YG_OK;
 }
 
@@ -378,21 +419,13 @@ extern "C" int yg_create(const yg_config *cfg, yg_ensemble **out)
         delete e;
         return YG_ERR_CUDA;
     }
-    const size_t n = (size_t)cfg->n_chains, d = (size_t)cfg->dim;
     int rc = YG_OK;
-    if ((rc = dev_alloc(&e->theta, d * n)) || (rc = dev_alloc(&e->logpost, YG_MAX_LEVELS * n)) ||
-        (rc = dev_alloc(&e->w_mean, d * n)) || (rc = dev_alloc(&e->w_m2, (cfg->dim > YG_MAX_DIM ? d : d * d) * n)) ||
-        (rc = dev_alloc(&e->n_accept, n)) || (rc = dev_alloc(&e->counters, 8)) ||
-        (rc = dev_alloc(&e->pool_partials, (size_t)POOL_PARTS * (size_t)yg_pooled_len(std::min(cfg->dim, YG_MAX_DIM))))) {
+    if ((rc = alloc_group(e, ALWAYS)) || (rc = alloc_group(e, DIAG)) || (cfg->adaptive && (rc = alloc_group(e, AM))) ||
+        (rc = dev_alloc((void **)&e->counters, sizeof(unsigned long long) * 8)) ||
+        (rc = dev_alloc((void **)&e->pool_partials,
+                        sizeof(double) * POOL_PARTS * (size_t)yg_pooled_len(std::min(cfg->dim, YG_MAX_DIM))))) {
         yg_destroy(e);
         return rc;
-    }
-    if (cfg->adaptive) {
-        if ((rc = dev_alloc(&e->am_mean, d * n)) || (rc = dev_alloc(&e->am_m2, d * d * n)) ||
-            (rc = dev_alloc(&e->prop_L, d * d * n))) {
-            yg_destroy(e);
-            return rc;
-        }
     }
     *out = e;
     return YG_OK;
@@ -402,19 +435,8 @@ extern "C" int yg_destroy(yg_ensemble *e)
 {
     if (!e) return YG_OK;
     cudaSetDevice(e->cfg.device);
+    for (void *p : e->buf) cudaFree(p);
     cudaFree(e->d_problem);
-    cudaFree(e->theta);
-    cudaFree(e->logpost);
-    cudaFree(e->w_mean);
-    cudaFree(e->w_m2);
-    cudaFree(e->am_mean);
-    cudaFree(e->am_m2);
-    cudaFree(e->prop_L);
-    cudaFree(e->aem_n);
-    cudaFree(e->aem_mean);
-    cudaFree(e->aem_m2);
-    cudaFree(e->aem_cache);
-    cudaFree(e->n_accept);
     cudaFree(e->counters);
     cudaFree(e->pool_partials);
     cudaFree(e->big_done);
@@ -422,35 +444,12 @@ extern "C" int yg_destroy(yg_ensemble *e)
     return YG_OK;
 }
 
-extern "C" int yg_set_problem(yg_ensemble *e, const yg_problem *pb)
+namespace {
+
+// One-chain-per-thread and LV kernels: the DevProblemHeader blob (common.cuh).
+int build_blob(const yg_config &c, const yg_problem *pb, std::vector<char> &blob)
 {
-    int rc = check_handle(e, false, false);
-    if (rc) return rc;
-    if (!pb || !pb->prop_L) {
-        yg_set_error("yg_set_problem: problem / prop_L is null");
-        return YG_ERR_INVALID;
-    }
-    const int d = e->cfg.dim, nl = e->cfg.n_levels, model = e->cfg.model;
-    if (model == YG_MODEL_LINEAR) {
-        bool big = d > YG_MAX_DIM;
-        for (int l = 0; l < nl; l++) big = big || pb->level[l].data_dim > YG_MAX_DATA_DIM;
-        if (big) return set_problem_big(e, pb);
-    }
-    e->big = false;
-    if (pb->proposal != YG_PROPOSAL_MRW && pb->proposal != YG_PROPOSAL_PCN) {
-        yg_set_error("unknown proposal kind %d", pb->proposal);
-        return YG_ERR_INVALID;
-    }
-    if (pb->proposal == YG_PROPOSAL_PCN) {
-        if (!(pb->pcn_step > 0.0 && pb->pcn_step <= 0.5)) {       // pcn.py:42
-            yg_set_error("pCN step size must lie in (0, 0.5], got %g", pb->pcn_step);
-            return YG_ERR_INVALID;
-        }
-        if (nl != 1 || e->cfg.adaptive) {
-            yg_set_error("pCN is a single-level, non-adaptive method (chain/method/pcn.py)");
-            return YG_ERR_UNSUPPORTED;
-        }
-    }
+    const int d = c.dim, nl = c.n_levels, model = c.model;
     // tail: per level data + design
     size_t tail_len = 0;
     for (int l = 0; l < nl; l++) {
@@ -482,14 +481,14 @@ extern "C" int yg_set_problem(yg_ensemble *e, const yg_problem *pb)
         if (model == YG_MODEL_LV_RK4) tail_len += (size_t)L.n_data * 2;
     }
     tail_len = (tail_len + 1) & ~size_t(1);        // keep the blob a multiple of 16 bytes
-    std::vector<char> blob(sizeof(DevProblemHeader) + sizeof(double) * tail_len, 0);
+    blob.assign(sizeof(DevProblemHeader) + sizeof(double) * tail_len, 0);
     DevProblemHeader *h = reinterpret_cast<DevProblemHeader *>(blob.data());
     double *tail = reinterpret_cast<double *>(blob.data() + sizeof(DevProblemHeader));
     h->model = model;
     h->dim = d;
     h->n_levels = nl;
-    h->J = nl >= 2 ? e->cfg.sub_chain_length : 1;
-    h->eq_mode = e->cfg.eq_mode;
+    h->J = nl >= 2 ? c.sub_chain_length : 1;
+    h->eq_mode = c.eq_mode;
     h->tail_len = (int32_t)tail_len;
     h->proposal = pb->proposal;
     if (pb->proposal == YG_PROPOSAL_PCN) {
@@ -499,12 +498,6 @@ extern "C" int yg_set_problem(yg_ensemble *e, const yg_problem *pb)
         if (pb->pcn_mean) copy_mat(h->pcn_mean, pb->pcn_mean, 1, d);
     }
     copy_mat(h->prop_L, pb->prop_L, d, d);
-    for (int i = 0; i < d; i++)
-        for (int j = i + 1; j < d; j++)
-            if (h->prop_L[i * d + j] != 0.0) {
-                yg_set_error("prop_L must be lower triangular");
-                return YG_ERR_INVALID;
-            }
     size_t off = 0;
     for (int l = 0; l < nl; l++) {
         const yg_level &L = pb->level[l];
@@ -544,7 +537,7 @@ extern "C" int yg_set_problem(yg_ensemble *e, const yg_problem *pb)
             off += (size_t)L.n_data * 2;
         }
     }
-    if (e->cfg.aem) {
+    if (c.aem) {
         const yg_level &Lc = pb->level[0], &Lf = pb->level[1];
         if (Lc.data_dim != Lf.data_dim || pb->proposal != YG_PROPOSAL_MRW) {
             yg_set_error("adaptive error model: both levels must share the data dimension (MRW proposal)");
@@ -558,21 +551,63 @@ extern "C" int yg_set_problem(yg_ensemble *e, const yg_problem *pb)
                     return YG_ERR_UNSUPPORTED;
                 }
     }
-    YG_CUDA_CHECK(cudaSetDevice(e->cfg.device));
-    e->problem_set = false;                     // stays false if anything below fails
-    if (e->d_problem) cudaFree(e->d_problem);
+    return YG_OK;
+}
+
+}  // namespace
+
+extern "C" int yg_set_problem(yg_ensemble *e, const yg_problem *pb)
+{
+    int rc = check_handle(e, false, false);
+    if (rc) return rc;
+    if (!pb || !pb->prop_L) {
+        yg_set_error("yg_set_problem: problem / prop_L is null");
+        return YG_ERR_INVALID;
+    }
+    const yg_config &c = e->cfg;
+    const int d = c.dim, nl = c.n_levels;
+    if (pb->proposal != YG_PROPOSAL_MRW && pb->proposal != YG_PROPOSAL_PCN) {
+        yg_set_error("unknown proposal kind %d", pb->proposal);
+        return YG_ERR_INVALID;
+    }
+    if (pb->proposal == YG_PROPOSAL_PCN) {
+        if (!(pb->pcn_step > 0.0 && pb->pcn_step <= 0.5)) {       // pcn.py:42
+            yg_set_error("pCN step size must lie in (0, 0.5], got %g", pb->pcn_step);
+            return YG_ERR_INVALID;
+        }
+        if (nl != 1 || c.adaptive) {
+            yg_set_error("pCN is a single-level, non-adaptive method (chain/method/pcn.py)");
+            return YG_ERR_UNSUPPORTED;
+        }
+    }
+    for (int i = 0; i < d; i++)
+        for (int j = i + 1; j < d; j++)
+            if (pb->prop_L[(size_t)i * d + j] != 0.0) {
+                yg_set_error("prop_L must be lower triangular");
+                return YG_ERR_INVALID;
+            }
+    bool big = false;
+    if (c.model == YG_MODEL_LINEAR) {
+        big = d > YG_MAX_DIM;
+        for (int l = 0; l < nl; l++) big = big || pb->level[l].data_dim > YG_MAX_DATA_DIM;
+    }
+    std::vector<char> blob;
+    if ((rc = big ? build_big_blob(c, pb, blob) : build_blob(c, pb, blob))) return rc;
+    // Commit.  The handle changes from here on only, and holds no problem unless every step below succeeds.
+    YG_CUDA_CHECK(cudaSetDevice(c.device));
+    e->problem_set = false;
+    cudaFree(e->d_problem);
     e->d_problem = nullptr;
-    YG_CUDA_CHECK(cudaMalloc((void **)&e->d_problem, blob.size()));
+    YG_CUDA_CHECK(cudaMalloc(&e->d_problem, blob.size()));
     YG_CUDA_CHECK(cudaMemcpy(e->d_problem, blob.data(), blob.size(), cudaMemcpyHostToDevice));
     e->h_problem.swap(blob);
-    if (e->cfg.aem) {
-        const size_t n = (size_t)e->cfg.n_chains, dd = (size_t)pb->level[0].data_dim;
-        cudaFree(e->aem_n); cudaFree(e->aem_mean); cudaFree(e->aem_m2); cudaFree(e->aem_cache);
-        e->aem_n = nullptr; e->aem_mean = e->aem_m2 = e->aem_cache = nullptr;
-        e->aem_data_dim = (int)dd;
-        if ((rc = dev_alloc(&e->aem_n, n)) || (rc = dev_alloc(&e->aem_mean, dd * n)) ||
-            (rc = dev_alloc(&e->aem_m2, dd * n)) || (rc = dev_alloc(&e->aem_cache, (size_t)(3 * (d + 1) + 1) * n)))
-            return rc;
+    e->big = big;
+    if (big && !e->big_done) {      // per-tile progress counters of the balanced (tile, step-range) schedule
+        if ((rc = dev_alloc((void **)&e->big_done, sizeof(long long) * (((size_t)c.n_chains + 7) / 8)))) return rc;
+    }
+    if (c.aem) {
+        e->aem_data_dim = pb->level[0].data_dim;
+        if ((rc = alloc_group(e, AEM))) return rc;
     }
     e->problem_set = true;
     return YG_OK;
@@ -587,36 +622,29 @@ extern "C" int yg_set_state(yg_ensemble *e, const double *theta0_dev, int32_t fl
         return YG_ERR_INVALID;
     }
     cudaStream_t st = (cudaStream_t)stream;
-    const size_t n = (size_t)e->cfg.n_chains, d = (size_t)e->cfg.dim;
+    const size_t n = (size_t)e->cfg.n_chains;
     // a handle that never held a state has nothing to keep
     const bool keep_diag = (flags & YG_KEEP_DIAGNOSTICS) && e->state_set;
     const bool keep_adapt = (flags & YG_KEEP_ADAPTATION) && e->state_set;
     YG_CUDA_CHECK(cudaSetDevice(e->cfg.device));
-    YG_CUDA_CHECK(cudaMemcpyAsync(e->theta, theta0_dev, sizeof(double) * d * n, cudaMemcpyDeviceToDevice, st));
+    YG_CUDA_CHECK(cudaMemcpyAsync(e->buf[SB_THETA], theta0_dev, buf_bytes(e, SB_THETA), cudaMemcpyDeviceToDevice, st));
+    for (int b = 0; b < SB_COUNT; b++) {      // prop_L restarts from the problem's factor below, not from zeros
+        const Group g = kState[b].group;
+        const bool reset = g == DIAG ? !keep_diag : (g != ALWAYS && has_group(e, g) && !keep_adapt);
+        if (reset && b != SB_PROP_L) YG_CUDA_CHECK(cudaMemsetAsync(e->buf[b], 0, buf_bytes(e, b), st));
+    }
     if (!keep_diag) {
-        YG_CUDA_CHECK(cudaMemsetAsync(e->w_mean, 0, sizeof(double) * d * n, st));
-        YG_CUDA_CHECK(cudaMemsetAsync(e->w_m2, 0, sizeof(double) * (d > YG_MAX_DIM ? d : d * d) * n, st));
-        YG_CUDA_CHECK(cudaMemsetAsync(e->n_accept, 0, sizeof(unsigned long long) * n, st));
         YG_CUDA_CHECK(cudaMemsetAsync(e->counters, 0, sizeof(unsigned long long) * 8, st));
         e->welford_n = 0;
     }
     if (e->cfg.adaptive && !keep_adapt) {
-        YG_CUDA_CHECK(cudaMemsetAsync(e->am_mean, 0, sizeof(double) * d * n, st));
-        YG_CUDA_CHECK(cudaMemsetAsync(e->am_m2, 0, sizeof(double) * d * d * n, st));
-        broadcast_L_kernel<<<(int)std::min<size_t>((n + 127) / 128, 2048), 128, 0, st>>>(e->d_problem, e->prop_L,
-                                                                                      (int64_t)n);
-        YG_CUDA_CHECK(cudaGetLastError());
+        if ((rc = broadcast_prop_L(e, st))) return rc;
         e->am_steps = 0;
     }
-    if (e->cfg.aem && !keep_adapt) {       // empty cache, no error realisations yet
-        YG_CUDA_CHECK(cudaMemsetAsync(e->aem_n, 0, sizeof(unsigned long long) * n, st));
-        YG_CUDA_CHECK(cudaMemsetAsync(e->aem_mean, 0, sizeof(double) * (size_t)e->aem_data_dim * n, st));
-        YG_CUDA_CHECK(cudaMemsetAsync(e->aem_m2, 0, sizeof(double) * (size_t)e->aem_data_dim * n, st));
-        YG_CUDA_CHECK(cudaMemsetAsync(e->aem_cache, 0, sizeof(double) * (3 * (d + 1) + 1) * n, st));
-    }
+    double *theta = static_cast<double *>(e->buf[SB_THETA]), *logpost = static_cast<double *>(e->buf[SB_LOGPOST]);
     for (int l = 0; l < e->cfg.n_levels; l++) {
-        rc = e->big ? yg_launch_logpost_big(e, l, e->theta, (int64_t)n, e->logpost + (size_t)l * n, st)
-                    : yg_launch_logpost(e, l, e->theta, (int64_t)n, e->logpost + (size_t)l * n, st);
+        rc = e->big ? yg_launch_logpost_big(e, l, theta, (int64_t)n, logpost + (size_t)l * n, st)
+                    : yg_launch_logpost(e, l, theta, (int64_t)n, logpost + (size_t)l * n, st);
         if (rc) return rc;
     }
     // e->step_index (the Philox stream position) is deliberately left alone: the reference's numpy
@@ -671,7 +699,7 @@ extern "C" int yg_set_proposal_factor(yg_ensemble *e, const double *L_host, void
         }
         double *tail = reinterpret_cast<double *>(e->h_problem.data() + sizeof(DevBigHeader));
         for (int k = 0; k < d; k++) tail[h->propL_off + k] = L_host[(size_t)k * d + k];
-        char *base = reinterpret_cast<char *>(e->d_problem) + sizeof(DevBigHeader);
+        char *base = static_cast<char *>(e->d_problem) + sizeof(DevBigHeader);
         YG_CUDA_CHECK(cudaMemcpyAsync(base + sizeof(double) * h->propL_off, tail + h->propL_off, sizeof(double) * d,
                                       cudaMemcpyHostToDevice, st));
         if (h->dense_L) {
@@ -688,14 +716,9 @@ extern "C" int yg_set_proposal_factor(yg_ensemble *e, const double *L_host, void
         return YG_ERR_UNSUPPORTED;
     }
     copy_mat(h->prop_L, L_host, d, d);
-    YG_CUDA_CHECK(cudaMemcpyAsync(reinterpret_cast<char *>(e->d_problem) + offsetof(DevProblemHeader, prop_L), h->prop_L,
+    YG_CUDA_CHECK(cudaMemcpyAsync(static_cast<char *>(e->d_problem) + offsetof(DevProblemHeader, prop_L), h->prop_L,
                                   sizeof(h->prop_L), cudaMemcpyHostToDevice, st));
-    if (e->cfg.adaptive && e->prop_L) {
-        const size_t n = (size_t)e->cfg.n_chains;
-        broadcast_L_kernel<<<(int)std::min<size_t>((n + 127) / 128, 2048), 128, 0, st>>>(e->d_problem, e->prop_L, (int64_t)n);
-        YG_CUDA_CHECK(cudaGetLastError());
-    }
-    return YG_OK;
+    return e->cfg.adaptive ? broadcast_prop_L(e, st) : YG_OK;
 }
 
 extern "C" int yg_run(yg_ensemble *e, int64_t n_steps, int32_t thin, const yg_outputs *out, const yg_noise *noise,
@@ -752,41 +775,20 @@ extern "C" int yg_get_state(yg_ensemble *e, const yg_state *dst, void *stream)
     int rc = check_handle(e, true, true);
     if (rc) return rc;
     if (!dst) return YG_ERR_INVALID;
+    for (int b = 0; b < SB_COUNT; b++) {
+        const Group g = kState[b].group;
+        if (state_ptr(dst, b) && !has_group(e, g)) {
+            yg_set_error("%s per-chain state of %s ensembles only",
+                         b == SB_PROP_L ? "prop_L_dev is" : (g == AM ? "am_mean_dev / am_m2_dev are" : "aem_*_dev are"),
+                         g == AM ? "adaptive" : "adaptive-error-model");
+            return YG_ERR_INVALID;
+        }
+    }
     cudaStream_t st = (cudaStream_t)stream;
-    const size_t n = (size_t)e->cfg.n_chains, d = (size_t)e->cfg.dim, nl = (size_t)e->cfg.n_levels;
     YG_CUDA_CHECK(cudaSetDevice(e->cfg.device));
-    const cudaMemcpyKind k = cudaMemcpyDeviceToDevice;
-    if (dst->theta_dev) YG_CUDA_CHECK(cudaMemcpyAsync(dst->theta_dev, e->theta, 8 * d * n, k, st));
-    if (dst->logpost_dev) YG_CUDA_CHECK(cudaMemcpyAsync(dst->logpost_dev, e->logpost, 8 * nl * n, k, st));
-    if (dst->n_accept_dev) YG_CUDA_CHECK(cudaMemcpyAsync(dst->n_accept_dev, e->n_accept, 8 * n, k, st));
-    if (dst->w_mean_dev) YG_CUDA_CHECK(cudaMemcpyAsync(dst->w_mean_dev, e->w_mean, 8 * d * n, k, st));
-    if (dst->w_m2_dev) YG_CUDA_CHECK(cudaMemcpyAsync(dst->w_m2_dev, e->w_m2, 8 * (d > YG_MAX_DIM ? d : d * d) * n, k, st));
-    if (dst->prop_L_dev) {
-        if (!e->cfg.adaptive) {
-            yg_set_error("prop_L_dev is per-chain state of adaptive ensembles only");
-            return YG_ERR_INVALID;
-        }
-        YG_CUDA_CHECK(cudaMemcpyAsync(dst->prop_L_dev, e->prop_L, 8 * d * d * n, k, st));
-    }
-    if (dst->am_mean_dev || dst->am_m2_dev) {
-        if (!e->cfg.adaptive) {
-            yg_set_error("am_mean_dev / am_m2_dev are per-chain state of adaptive ensembles only");
-            return YG_ERR_INVALID;
-        }
-        if (dst->am_mean_dev) YG_CUDA_CHECK(cudaMemcpyAsync(dst->am_mean_dev, e->am_mean, 8 * d * n, k, st));
-        if (dst->am_m2_dev) YG_CUDA_CHECK(cudaMemcpyAsync(dst->am_m2_dev, e->am_m2, 8 * d * d * n, k, st));
-    }
-    if (dst->aem_n_dev || dst->aem_mean_dev || dst->aem_m2_dev || dst->aem_cache_dev) {
-        if (!e->cfg.aem) {
-            yg_set_error("aem_*_dev are per-chain state of adaptive-error-model ensembles only");
-            return YG_ERR_INVALID;
-        }
-        const size_t dd = (size_t)e->aem_data_dim;
-        if (dst->aem_n_dev) YG_CUDA_CHECK(cudaMemcpyAsync(dst->aem_n_dev, e->aem_n, 8 * n, k, st));
-        if (dst->aem_mean_dev) YG_CUDA_CHECK(cudaMemcpyAsync(dst->aem_mean_dev, e->aem_mean, 8 * dd * n, k, st));
-        if (dst->aem_m2_dev) YG_CUDA_CHECK(cudaMemcpyAsync(dst->aem_m2_dev, e->aem_m2, 8 * dd * n, k, st));
-        if (dst->aem_cache_dev) YG_CUDA_CHECK(cudaMemcpyAsync(dst->aem_cache_dev, e->aem_cache, 8 * (3 * (d + 1) + 1) * n, k, st));
-    }
+    for (int b = 0; b < SB_COUNT; b++)
+        if (void *p = state_ptr(dst, b))
+            YG_CUDA_CHECK(cudaMemcpyAsync(p, e->buf[b], state_bytes(e, b), cudaMemcpyDeviceToDevice, st));
     return YG_OK;
 }
 
@@ -800,26 +802,11 @@ extern "C" int yg_load_state(yg_ensemble *e, const yg_state *src, int64_t step_i
         return YG_ERR_INVALID;
     }
     cudaStream_t st = (cudaStream_t)stream;
-    const size_t n = (size_t)e->cfg.n_chains, d = (size_t)e->cfg.dim, nl = (size_t)e->cfg.n_levels;
     YG_CUDA_CHECK(cudaSetDevice(e->cfg.device));
-    const cudaMemcpyKind k = cudaMemcpyDeviceToDevice;
-    YG_CUDA_CHECK(cudaMemcpyAsync(e->theta, src->theta_dev, 8 * d * n, k, st));
-    YG_CUDA_CHECK(cudaMemcpyAsync(e->logpost, src->logpost_dev, 8 * nl * n, k, st));
-    if (src->n_accept_dev) YG_CUDA_CHECK(cudaMemcpyAsync(e->n_accept, src->n_accept_dev, 8 * n, k, st));
-    if (src->w_mean_dev) YG_CUDA_CHECK(cudaMemcpyAsync(e->w_mean, src->w_mean_dev, 8 * d * n, k, st));
-    if (src->w_m2_dev) YG_CUDA_CHECK(cudaMemcpyAsync(e->w_m2, src->w_m2_dev, 8 * (d > YG_MAX_DIM ? d : d * d) * n, k, st));
-    if (src->prop_L_dev && e->cfg.adaptive)
-        YG_CUDA_CHECK(cudaMemcpyAsync(e->prop_L, src->prop_L_dev, 8 * d * d * n, k, st));
-    if (src->am_mean_dev && e->cfg.adaptive)
-        YG_CUDA_CHECK(cudaMemcpyAsync(e->am_mean, src->am_mean_dev, 8 * d * n, k, st));
-    if (src->am_m2_dev && e->cfg.adaptive)
-        YG_CUDA_CHECK(cudaMemcpyAsync(e->am_m2, src->am_m2_dev, 8 * d * d * n, k, st));
-    if (e->cfg.aem) {
-        const size_t dd = (size_t)e->aem_data_dim;
-        if (src->aem_n_dev) YG_CUDA_CHECK(cudaMemcpyAsync(e->aem_n, src->aem_n_dev, 8 * n, k, st));
-        if (src->aem_mean_dev) YG_CUDA_CHECK(cudaMemcpyAsync(e->aem_mean, src->aem_mean_dev, 8 * dd * n, k, st));
-        if (src->aem_m2_dev) YG_CUDA_CHECK(cudaMemcpyAsync(e->aem_m2, src->aem_m2_dev, 8 * dd * n, k, st));
-        if (src->aem_cache_dev) YG_CUDA_CHECK(cudaMemcpyAsync(e->aem_cache, src->aem_cache_dev, 8 * (3 * (d + 1) + 1) * n, k, st));
+    for (int b = 0; b < SB_COUNT; b++) {
+        const void *p = state_ptr(src, b);
+        if (p && has_group(e, kState[b].group))       // pointers for groups the handle lacks are ignored
+            YG_CUDA_CHECK(cudaMemcpyAsync(e->buf[b], p, state_bytes(e, b), cudaMemcpyDeviceToDevice, st));
     }
     e->step_index = step_index;
     e->welford_n = welford_n;
@@ -873,8 +860,9 @@ extern "C" int yg_pooled_stats(yg_ensemble *e, double *out_dev, void *stream)
         return YG_ERR_UNSUPPORTED;
     }
     YG_CUDA_CHECK(cudaSetDevice(e->cfg.device));
-    return yg_pooled_impl(e->w_mean, e->w_m2, e->n_accept, e->cfg.dim, e->cfg.n_chains, e->welford_n,
-                          e->pool_partials, POOL_PARTS, out_dev, (cudaStream_t)stream);
+    return yg_pooled_impl(static_cast<const double *>(e->buf[SB_W_MEAN]), static_cast<const double *>(e->buf[SB_W_M2]),
+                          static_cast<const unsigned long long *>(e->buf[SB_N_ACCEPT]), e->cfg.dim, e->cfg.n_chains,
+                          e->welford_n, e->pool_partials, POOL_PARTS, out_dev, (cudaStream_t)stream);
 }
 
 extern "C" int yg_last_launch(yg_ensemble *e, int32_t *grid, int32_t *block, int32_t *smem_bytes, int64_t *launches)
@@ -893,16 +881,3 @@ extern "C" int yg_fp64_tensor_peak(int32_t device, double ms, double *tflops_out
     return yg_dmma_peak(device, ms, tflops_out);
 }
 
-#ifdef YG_BOUNDS_CHECK
-// Bounds-checked development build only (not part of include/yagre_b200.h): proves that YG_CHK is live in THIS
-// library by violating it on purpose.  Returns 1 when the device assert fired (the CUDA context is unusable
-// afterwards: call it last, in a process of its own), 0 when the launch completed, i.e. the checks are compiled out.
-namespace {
-__global__ void bounds_selftest_kernel(int limit) { YG_CHK(threadIdx.x + 1, limit); }
-}  // namespace
-extern "C" int yg_bounds_check_selftest(void)
-{
-    bounds_selftest_kernel<<<1, 32>>>(1);
-    return cudaDeviceSynchronize() == cudaErrorAssert ? 1 : 0;
-}
-#endif

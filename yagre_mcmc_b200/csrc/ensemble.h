@@ -48,19 +48,22 @@ struct RunArgs {
     unsigned long long *counters;
 };
 
+// The per-chain state buffers, in the order of yg_state; their sizes and groups are the table in abi.cu.
+enum StateBuf {
+    SB_THETA, SB_LOGPOST, SB_N_ACCEPT, SB_W_MEAN, SB_W_M2, SB_PROP_L, SB_AM_MEAN, SB_AM_M2,
+    SB_AEM_N, SB_AEM_MEAN, SB_AEM_M2, SB_AEM_CACHE, SB_COUNT
+};
+
 struct yg_ensemble {
     yg_config cfg;
     int sm_count = 0;
     bool problem_set = false, state_set = false;
     bool big = false;                  // large linear model: DevBigHeader blob, linear_dmma_kernel.cu
     std::vector<char> h_problem;
-    DevProblemHeader *d_problem = nullptr;
-    double *theta = nullptr, *logpost = nullptr, *w_mean = nullptr, *w_m2 = nullptr;
-    double *am_mean = nullptr, *am_m2 = nullptr, *prop_L = nullptr;
-    unsigned long long *aem_n = nullptr;
-    double *aem_mean = nullptr, *aem_m2 = nullptr, *aem_cache = nullptr;
+    void *d_problem = nullptr;         // DevBigHeader blob if big, else DevProblemHeader blob
+    void *buf[SB_COUNT] = {};          // per-chain state, chain index fastest (RunArgs lists the shapes)
     int aem_data_dim = 0;
-    unsigned long long *n_accept = nullptr, *counters = nullptr;
+    unsigned long long *counters = nullptr;
     double *pool_partials = nullptr;   // [POOL_PARTS][yg_pooled_len(d)] scratch of yg_pooled_stats
     long long *big_done = nullptr;     // [tiles] steps completed per 8-chain tile within a launch (linear_dmma_kernel.cu)
     int64_t step_index = 0, welford_n = 0, am_steps = 0;

@@ -956,7 +956,8 @@ int launch_logpost_t(yg_ensemble *e, int level, const double *theta, int64_t n, 
     const size_t smem = (e->h_problem.size() + 15) & ~size_t(15);
     auto kern = logpost_kernel<D, DD>;
     YG_CUDA_CHECK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    kern<<<grid, threads, smem, st>>>(e->d_problem, (uint32_t)e->h_problem.size(), level, theta, n, out);
+    kern<<<grid, threads, smem, st>>>(static_cast<const DevProblemHeader *>(e->d_problem), (uint32_t)e->h_problem.size(),
+                                      level, theta, n, out);
     YG_CUDA_CHECK(cudaGetLastError());
     e->launches += 1;
     return YG_OK;

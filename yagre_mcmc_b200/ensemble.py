@@ -23,6 +23,30 @@ def _f64(a):
     return np.ascontiguousarray(np.asarray(a, dtype=np.float64))
 
 
+def state_layout(n, d, levels, adaptive, aem_data_dim):
+    """{name: (shape, torch dtype)} of the per-chain state (yg_state) of n chains; aem_data_dim 0: no error model."""
+    f64, i64 = torch.float64, torch.int64
+    lay = dict(theta=((d, n), f64), logpost=((levels, n), f64), n_accept=((n,), i64), w_mean=((d, n), f64),
+               w_m2=((d, d, n) if d <= _lib.YG_MAX_DIM else (d, n), f64))        # large linear model: diagonal only
+    if adaptive:
+        lay.update(prop_L=((d, d, n), f64), am_mean=((d, n), f64), am_m2=((d, d, n), f64))
+    if aem_data_dim:
+        lay.update(aem_n=((n,), i64), aem_mean=((aem_data_dim, n), f64), aem_m2=((aem_data_dim, n), f64),
+                   aem_cache=((3 * (d + 1) + 1, n), f64))
+    return lay
+
+
+def check_state(r, layout):
+    """ValueError unless r has theta and logpost and each array the layout names is a tensor of its shape and dtype."""
+    if 'theta' not in r or 'logpost' not in r:
+        raise ValueError("a state needs at least theta and logpost")
+    for k, (shape, dtype) in layout.items():
+        v = r.get(k)
+        if v is not None and (not torch.is_tensor(v) or tuple(v.shape) != shape or v.dtype != dtype):
+            raise ValueError(f"state {k!r} must be a {dtype} tensor of shape {shape}, got {type(v).__name__} "
+                             f"{tuple(getattr(v, 'shape', ()))} {getattr(v, 'dtype', '')}")
+
+
 class LoweredProblem:
     """The plain-array form of a (hierarchy of) Bayesian model(s) + proposal, i.e.
     what ChainBuilder.build_method() (reference chain/builder.py:72-83) boils down to.
@@ -247,26 +271,13 @@ class ChainEnsemble:
         res['_keep'] = keep
         return res
 
+    def layout(self):
+        dd = int(np.asarray(self.problem.arrays['L0_data']).shape[1]) if self.cfg.aem else 0
+        return state_layout(self.n_chains, self.dim, self.levels, self.cfg.adaptive, dd)
+
     def state(self):
-        n, d = self.n_chains, self.dim
-        st = YgState()
-        # large linear model (d > YG_MAX_DIM): Welford M2 is diagonal only, [d, n]
-        w_m2 = self._empty(d, d, n) if d <= _lib.YG_MAX_DIM else self._empty(d, n)
-        r = dict(theta=self._empty(d, n), logpost=self._empty(self.levels, n),
-                 n_accept=self._empty(n, dtype=torch.int64), w_mean=self._empty(d, n), w_m2=w_m2)
-        st.theta_dev, st.logpost_dev, st.n_accept_dev = r['theta'].data_ptr(), r['logpost'].data_ptr(), r['n_accept'].data_ptr()
-        st.w_mean_dev, st.w_m2_dev = r['w_mean'].data_ptr(), r['w_m2'].data_ptr()
-        if self.cfg.adaptive:
-            r['prop_L'], r['am_mean'], r['am_m2'] = self._empty(d, d, n), self._empty(d, n), self._empty(d, d, n)
-            st.prop_L_dev, st.am_mean_dev, st.am_m2_dev = (r['prop_L'].data_ptr(), r['am_mean'].data_ptr(),
-                                                           r['am_m2'].data_ptr())
-        if self.cfg.aem:
-            dd = int(np.asarray(self.problem.arrays['L0_data']).shape[1])
-            r['aem_n'] = self._empty(n, dtype=torch.int64)
-            r['aem_mean'], r['aem_m2'] = self._empty(dd, n), self._empty(dd, n)
-            r['aem_cache'] = self._empty(3 * (d + 1) + 1, n)
-            st.aem_n_dev, st.aem_mean_dev = r['aem_n'].data_ptr(), r['aem_mean'].data_ptr()
-            st.aem_m2_dev, st.aem_cache_dev = r['aem_m2'].data_ptr(), r['aem_cache'].data_ptr()
+        r = {k: self._empty(*shape, dtype=dtype) for k, (shape, dtype) in self.layout().items()}
+        st = YgState(**{k + '_dev': v.data_ptr() for k, v in r.items()})
         with torch.cuda.device(self.device):
             check(self.lib.yg_get_state(self._h, C.byref(st), self._stream()))
         c = self.counters()
@@ -275,30 +286,18 @@ class ChainEnsemble:
 
     def accept_counts(self):
         """Per-chain accepted transitions since set_state: device tensor [n_chains] int64 (asynchronous)."""
-        st = YgState()
         out = self._empty(self.n_chains, dtype=torch.int64)
-        st.n_accept_dev = out.data_ptr()
+        st = YgState(n_accept_dev=out.data_ptr())
         with torch.cuda.device(self.device):
             check(self.lib.yg_get_state(self._h, C.byref(st), self._stream()))
         return out
 
     def load_state(self, r):
-        st = YgState()
-        keep = {k: r[k].to(self.device).contiguous() for k in
-                ('theta', 'logpost', 'n_accept', 'w_mean', 'w_m2', 'prop_L', 'am_mean', 'am_m2',
-                 'aem_n', 'aem_mean', 'aem_m2', 'aem_cache') if k in r}
-        st.theta_dev, st.logpost_dev = keep['theta'].data_ptr(), keep['logpost'].data_ptr()
-        if 'n_accept' in keep:
-            st.n_accept_dev = keep['n_accept'].data_ptr()
-        if 'w_mean' in keep:
-            st.w_mean_dev, st.w_m2_dev = keep['w_mean'].data_ptr(), keep['w_m2'].data_ptr()
-        if 'prop_L' in keep and self.cfg.adaptive:
-            st.prop_L_dev = keep['prop_L'].data_ptr()
-        if 'am_mean' in keep and 'am_m2' in keep and self.cfg.adaptive:
-            st.am_mean_dev, st.am_m2_dev = keep['am_mean'].data_ptr(), keep['am_m2'].data_ptr()
-        if self.cfg.aem and all(k in keep for k in ('aem_n', 'aem_mean', 'aem_m2', 'aem_cache')):
-            st.aem_n_dev, st.aem_mean_dev = keep['aem_n'].data_ptr(), keep['aem_mean'].data_ptr()
-            st.aem_m2_dev, st.aem_cache_dev = keep['aem_m2'].data_ptr(), keep['aem_cache'].data_ptr()
+        """Restores state(); theta and logpost are required, arrays of features this ensemble lacks are ignored."""
+        layout = self.layout()
+        check_state(r, layout)          # yg_load_state reads the layout's byte count from every pointer it is given
+        keep = {k: r[k].to(self.device).contiguous() for k in layout if k in r}
+        st = YgState(**{k + '_dev': v.data_ptr() for k, v in keep.items()})
         with torch.cuda.device(self.device):
             check(self.lib.yg_load_state(self._h, C.byref(st), int(r.get('step_index', 0)),
                                          int(r.get('welford_n', 0)),

@@ -19,8 +19,6 @@ import numpy as np
 import torch
 
 FORMAT_VERSION = 1
-_STATE_KEYS = ('theta', 'logpost', 'n_accept', 'w_mean', 'w_m2', 'prop_L', 'am_mean', 'am_m2',
-               'aem_n', 'aem_mean', 'aem_m2', 'aem_cache')
 
 
 def save_trajectory(path, samples, thin=1, chain_offset=0, meta=None):
@@ -58,7 +56,7 @@ def as_reference_layout(samples):
 def save_checkpoint(path, ensemble, extra=None):
     """Writes the complete per-chain state of a ChainEnsemble (this rank's chains)."""
     st = ensemble.state()
-    arrays = {k: st[k].cpu().numpy() for k in _STATE_KEYS if k in st}
+    arrays = {k: st[k].cpu().numpy() for k in ensemble.layout()}
     head = dict(format='yagre_mcmc_b200.checkpoint', version=FORMAT_VERSION, step_index=int(st['step_index']),
                 welford_n=int(st['welford_n']), am_steps=int(st.get('am_steps', 0)), n_chains=int(ensemble.n_chains), dim=int(ensemble.dim),
                 levels=int(ensemble.levels), seed=int(ensemble.cfg.seed), chain_offset=int(ensemble.cfg.chain_offset),
@@ -82,7 +80,7 @@ def load_checkpoint(path, ensemble):
         if head[key] != have:
             raise ValueError(f"checkpoint {key}={head[key]!r} does not match the ensemble ({have!r}): "
                              "a resumed run would not continue the saved chains")
-    st = {k: torch.from_numpy(np.ascontiguousarray(f[k])) for k in _STATE_KEYS if k in f.files}
+    st = {k: torch.from_numpy(np.ascontiguousarray(f[k])) for k in ensemble.layout() if k in f.files}
     st['step_index'], st['welford_n'] = head['step_index'], head['welford_n']
     st['am_steps'] = head.get('am_steps', head['welford_n'])
     ensemble.load_state(st)
