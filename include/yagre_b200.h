@@ -67,7 +67,7 @@
 extern "C" {
 #endif
 
-#define YG_ABI_VERSION 4u
+#define YG_ABI_VERSION 5u
 #define YG_MAX_LEVELS 3         /* densities per problem: up to two surrogates + the target */
 #define YG_MAX_DIM 8           /* parameter dimension of the one-chain-per-thread kernels */
 #define YG_MAX_DATA_DIM 8
@@ -176,7 +176,10 @@ typedef struct yg_config {
      * builders (chain/builder.py:14-16) -- : they stay zero.  Honoured by the tensor-path kernel, where the moments
      * live in L2 (d x 2 doubles per chain); the other kernels keep them in registers / shared memory for free. */
     int32_t acceptance_only;
-    int32_t reserved[1];
+    /* 1 = the LV kernel evaluates every design point of every proposal.  0 (default): at level 0 it skips the
+     * remaining integrations of a proposal whose partial misfit already certifies its rejection (diagonal noise
+     * precision only); results are bit-identical either way. */
+    int32_t early_reject_off;
 } yg_config;
 
 typedef struct yg_noise {
@@ -246,9 +249,11 @@ int yg_get_state(yg_ensemble *e, const yg_state *dst, void *stream);
 int yg_load_state(yg_ensemble *e, const yg_state *src, int64_t step_index, int64_t welford_n, int64_t am_steps,
                   void *stream);
 
-/* out_host[9] = {step index, transitions done (all chains), accepted, level-0 forward evals,
+/* out_host[10] = {step index, transitions done (all chains), accepted, level-0 forward evals,
  * target-level forward evals, welford n, am_steps, level-1 forward evals of a three-level hierarchy,
- * accepted coarse sub-steps (the acceptance the reference's surrogate diagnostics record, mlda.py:58-62)}.
+ * accepted coarse sub-steps (the acceptance the reference's surrogate diagnostics record, mlda.py:58-62),
+ * level-0 integrations (proposal, design point) the LV kernel skipped because the rejection was already
+ * certain}.  The last one depends on the launch geometry and the scheduling, the others do not.
  * Synchronises `stream`. */
 int yg_get_counters(yg_ensemble *e, int64_t *out_host, void *stream);
 

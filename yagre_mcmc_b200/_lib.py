@@ -10,7 +10,7 @@ _HERE = os.path.dirname(os.path.abspath(__file__))
 # YAGRE_B200_LIB: development override (an alternative build of the same library, e.g. tools/_build/...)
 LIB_PATH = os.environ.get("YAGRE_B200_LIB") or os.path.join(_HERE, "libyagre_b200.so")
 
-YG_ABI_VERSION = 4
+YG_ABI_VERSION = 5
 YG_MAX_LEVELS = 3
 KEEP_DIAGNOSTICS, KEEP_ADAPTATION = 1, 2
 YG_MAX_DIM = 8
@@ -55,7 +55,7 @@ class YgConfig(C.Structure):
                 ("am_eps", C.c_double), ("am_scale", C.c_double),
                 ("blocks_per_sm", C.c_int32), ("threads_per_block", C.c_int32),
                 ("rk4_segment", C.c_int32), ("aem", C.c_int32), ("aem_min_data", C.c_int32),
-                ("aem_heuristic", C.c_int32), ("acceptance_only", C.c_int32), ("reserved", C.c_int32 * 1)]
+                ("aem_heuristic", C.c_int32), ("acceptance_only", C.c_int32), ("early_reject_off", C.c_int32)]
 
 
 class YgNoise(C.Structure):

@@ -833,6 +833,7 @@ extern "C" int yg_get_counters(yg_ensemble *e, int64_t *out_host, void *stream)
     out_host[6] = e->am_steps;
     out_host[7] = (int64_t)c[4];
     out_host[8] = (int64_t)c[5];
+    out_host[9] = (int64_t)c[6];
     return YG_OK;
 }
 

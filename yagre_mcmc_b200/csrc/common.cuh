@@ -11,6 +11,7 @@
 #include "../../include/yagre_b200.h"
 
 #define YG_DEVFN __device__ __forceinline__
+#define YG_HDFN __host__ __device__ __forceinline__
 
 // Bounds-checked development build (`make -C yagre_mcmc_b200/csrc checked`, -DYG_BOUNDS_CHECK): every computed index
 // into a shared-memory carve-up or a caller-provided device buffer is asserted against the extent of that array
@@ -131,11 +132,28 @@ YG_DEVFN void philox_normal_pair(uint64_t seed, uint64_t chain, uint64_t step, u
 
 // mrw.py:54-57, mlda.py:148-154, metropolisHastings.py:68-73:
 //   r = exp(delta); a = r if r < 1. else 1.; accept iff u <= a   (NaN -> a = 1 -> accept)
-YG_DEVFN bool accept_rule(double delta, double u)
+YG_HDFN bool accept_rule(double delta, double u)
 {
     const double r = exp(delta);
     const double a = (r < 1.0) ? r : 1.0;
     return u <= a;
+}
+
+// Misfit budget of a proposal whose acceptance is accept_rule(t * (-S / 2) + lp - lps, u), S = sum of the
+// misfits q_n >= 0: a partial sum of q above the budget certifies the rejection, so the remaining forward
+// evaluations can be skipped.  The margin (relative 1e-9 of every term) covers the rounding of log / exp,
+// of the product by t, of the sums and of summing S in another order than np_sum_le128.  Returns +inf (never
+// skip) when the rule is not monotone in S or a term is not finite: u == 0 always accepts, and a NaN delta
+// (lps = -inf) accepts too.
+YG_HDFN double reject_budget(double lp, double lps, double u, double t)
+{
+    if (!(u > 0.0) || !(t > 0.0) || !isfinite(t)) return (double)INFINITY;
+    const double lu = log(u);
+    const double d = lp - lps - lu;
+    const double m = fabs(lp) + fabs(lps) + fabs(lu) + 1.0;
+    if (!isfinite(d) || !isfinite(m)) return (double)INFINITY;
+    const double b = 2.0 * (d + 1e-9 * m) / t;
+    return b > 0.0 ? b * (1.0 + 1e-9) : b;
 }
 
 // parameter/scalar.py:38-43: math.isclose(a, b) with rel_tol = 1e-9, abs_tol = 0
@@ -149,7 +167,7 @@ YG_DEVFN bool isclose_rule(double x, double y)
 
 // numpy's pairwise summation over a contiguous vector (np.sum in likelihood.py:80).
 // stride lets the caller walk a shared-memory column.
-YG_DEVFN double np_sum_le128(const double *a, int n, int stride)
+YG_HDFN double np_sum_le128(const double *a, int n, int stride)
 {
     if (n < 8) {
         double res = 0.0;

@@ -106,8 +106,21 @@ YG_DEVFN int fast_div(int u, int d, float inv)
     return q;
 }
 
+// Lane of the k-th (0-based) set bit of m; requires k < popc(m).
+YG_DEVFN int nth_set_bit(unsigned m, int k)
+{
+    int pos = 0;
+#pragma unroll
+    for (int w = 16; w > 0; w >>= 1) {
+        const int lo = __popc(m & ((1u << w) - 1u));
+        if (k >= lo) { k -= lo; pos += w; m >>= w; }
+    }
+    return pos;
+}
+
 template <bool TWO_LEVEL, int MAXT>
-__global__ void __launch_bounds__(MAXT, 1) lv_mh_kernel(const RunArgs a, const int cmax, const int seg_len)
+__global__ void __launch_bounds__(MAXT, 1) lv_mh_kernel(const RunArgs a, const int cmax, const int seg_len,
+                                                          const bool early_reject)
 {
     extern __shared__ __align__(16) unsigned char smem_raw[];
     const int tid = threadIdx.x, nthr = blockDim.x;
@@ -124,32 +137,59 @@ __global__ void __launch_bounds__(MAXT, 1) lv_mh_kernel(const RunArgs a, const i
     off += sizeof(double) * (size_t)nd_max * cmax;                         //   segments, indexed by item
     double *sy = reinterpret_cast<double *>(smem_raw + off);
     off += sizeof(double) * (size_t)nd_max * cmax;
-    double *nz = reinterpret_cast<double *>(smem_raw + off);               // [3][cmax] next z0, z1, uniform
-    off += sizeof(double) * 3 * cmax;
+    double *nz = reinterpret_cast<double *>(smem_raw + off);               // [4][cmax] z0, z1, uniform, next uniform
+    off += sizeof(double) * 4 * cmax;
+    double *qmax = reinterpret_cast<double *>(smem_raw + off);             // [cmax] misfit budget (reject_budget)
+    off += sizeof(double) * cmax;
+    double *qpart = reinterpret_cast<double *>(smem_raw + off);            // [cmax] misfit summed so far
+    off += sizeof(double) * cmax;
+    double *qsum = reinterpret_cast<double *>(smem_raw + off);             // [n_data] misfit per design point
+    off += sizeof(double) * nd_max;
     unsigned long long *nacc = reinterpret_cast<unsigned long long *>(smem_raw + off);   // [cmax]
     off += sizeof(unsigned long long) * cmax;
     int *list0 = reinterpret_cast<int *>(smem_raw + off);                  // [2][cmax]
     off += sizeof(int) * 2 * cmax;
     int *segdone = reinterpret_cast<int *>(smem_raw + off);                // [n_data * cmax] segments done per item
     off += sizeof(int) * (size_t)nd_max * cmax;
+    int *perm = reinterpret_cast<int *>(smem_raw + off);                   // [n_data] level-0 design points, heaviest first
+    off += sizeof(int) * nd_max;
     unsigned char *evald = smem_raw + off;                                 // [cmax]
     off += (cmax + 15) & ~15;
     off = (off + 15) & ~size_t(15);      // the int arrays above leave 4-byte alignment when n_data * cmax is odd
     uint64_t *mbar = reinterpret_cast<uint64_t *>(smem_raw + off);
     int *nact = reinterpret_cast<int *>(mbar + 1);                         // [2]
-    unsigned long long *blk_cnt = reinterpret_cast<unsigned long long *>(mbar + 2);   // [5]
-    int *qhead = reinterpret_cast<int *>(mbar + 7);                        // work-queue head of the current phase
+    unsigned long long *blk_cnt = reinterpret_cast<unsigned long long *>(mbar + 2);   // [6]
+    int *qhead = reinterpret_cast<int *>(mbar + 8);                        // work-queue head of the current phase
     YG_CHK(reinterpret_cast<unsigned char *>(qhead + 1) - smem_raw - 1, yg_dynamic_smem_bytes());   // the carve-up fits the launch
 
     tma_stage_blob(pb, a.problem, (uint32_t)((a.problem_bytes + 15u) & ~15u), mbar);
-    if (tid < 5) blk_cnt[tid] = 0ull;
+    if (tid < 6) blk_cnt[tid] = 0ull;
     if (tid < 2) nact[tid] = 0;
+    for (int i = tid; i < nd_max; i += nthr) perm[i] = i;
 
     const double *tail = dev_tail(pb);
     const int J = TWO_LEVEL ? pb->J : 1;
     const int n_lvl = TWO_LEVEL ? 2 : 1;
     const double L00 = pb->prop_L[0], L10 = pb->prop_L[LV_D], L11 = pb->prop_L[LV_D + 1];
     const bool pcn = pb->proposal == YG_PROPOSAL_PCN;
+    const int n_phases = TWO_LEVEL ? J + 1 : 1;
+
+    // Early rejection at level 0 (the coarse level, or the only one): a proposal whose partial misfit sum
+    // passed its budget is rejected whatever the remaining design points give, so their integrations are
+    // skipped.  Exact only when every q_n >= 0 and never NaN: diagonal noise precision with positive finite
+    // entries and finite data (a non-finite forward output then gives q = +inf).  Only for levels of one
+    // segment per item, where a skipped unit has no successor waiting on it.
+    bool skip_lvl0 = false;
+    {
+        const DevLevel &L0 = pb->lvl[0];
+        const double *P = L0.noise_prec;
+        bool ok = early_reject && L0.data_dim == 2 && L0.rk4_steps <= seg_len && P[1] == 0.0 && P[2] == 0.0 &&
+                  P[0] > 0.0 && P[3] > 0.0 && isfinite(P[0]) && isfinite(P[3]);
+        for (int i = 0; ok && i < 2 * L0.n_data; i++) ok = isfinite(tail[L0.data_off + i]);
+        skip_lvl0 = ok;
+    }
+    // design-point order of the level-0 queue: learned from the misfits of the launch's first level-0 phase
+    bool perm_ready = false;
 
 #ifdef YG_BOUNDS_CHECK
     auto ch_at = [&](const int field, const int c) -> double & {
@@ -176,7 +216,13 @@ __global__ void __launch_bounds__(MAXT, 1) lv_mh_kernel(const RunArgs a, const i
     // predecessor left in sx/sy; the predecessor has a smaller queue index, so it was grabbed
     // earlier and never waits on anything later: the spin on segdone[item] cannot deadlock.
     // A batch never holds two segments of one item (batch size <= nItems).
-    auto eval_phase = [&](const int lvl, const int cur, const double h, const LvStepConsts &kc) {
+    //
+    // With early rejection (skip_lvl0, level 0) a warp drops the units of proposals whose rejection is already
+    // certain when it takes them, and keeps taking units until its 32 lanes hold live ones: FP64 instructions
+    // issue per warp, so a skipped lane saves nothing unless its slot is refilled.  Design points are visited
+    // in the order `perm`; q stays indexed by the design point, so results do not depend on the order.
+    auto eval_phase = [&](const int lvl, const int cur, const double h, const LvStepConsts &kc,
+                          unsigned long long &n_skip) {
         const DevLevel &Lv = pb->lvl[lvl];
         const int na = nact[cur];
         const int nD = Lv.n_data;
@@ -194,6 +240,70 @@ __global__ void __launch_bounds__(MAXT, 1) lv_mh_kernel(const RunArgs a, const i
         if (tid == 0) {
             nact[cur ^ 1] = 0;
             blk_cnt[2 + lvl] += (unsigned long long)na;
+        }
+        auto integrate = [&](const int steps, const LvRates &r, double &x, double &y) {
+#ifdef YG_TIMERS
+            lv_integrate(kc, r, a.thin == 7 ? 0 : steps, x, y);   // thin == 7: overhead-only run
+#else
+            lv_integrate(kc, r, steps, x, y);
+#endif
+        };
+        // misfit of design point n from the forward output (x, y)
+        auto misfit = [&](const int n, double x, double y) {
+            // non-finite forward output -> +inf (policy of the oracle's RK4 plugin)
+            x = isfinite(x) ? x : CUDART_INF;
+            y = isfinite(y) ? y : CUDART_INF;
+            const double r0 = x - data[2 * n], r1 = y - data[2 * n + 1];
+            // r' P r with P applied first; exact zeros skipped (diagonal noise, inf-safe)
+            double t0 = P00 * r0;
+            if (P01 != 0.0) t0 = fma(P01, r1, t0);
+            double t1 = (P10 != 0.0) ? P10 * r0 : 0.0;
+            t1 = (P10 != 0.0) ? fma(P11, r1, t1) : P11 * r1;
+            return fma(r1, t1, r0 * t0);
+        };
+        if (lvl == 0 && skip_lvl0) {      // one segment per item: unit == item, design-point major
+            int mine = 0, pend = 0;        // this lane's unit; lanes [0, pend) hold one
+            bool drained = false;
+            for (;;) {
+                while (pend < 32 && !drained) {
+                    const int want = 32 - pend;
+                    int u0 = 0;
+                    if (lane == 0) u0 = atomicAdd(qhead, want);
+                    u0 = __shfl_sync(0xffffffffu, u0, 0);
+                    if (u0 >= nUnits) { drained = true; break; }
+                    const int u = u0 + lane;
+                    bool live = false;
+                    if (lane < want && u < nUnits) {
+                        const int nq = fast_div(u, na, inv_na), ai = u - nq * na;
+                        YG_CHK(ai, cmax); YG_CHK(nq, nD);
+                        const int c = lst[ai];
+                        YG_CHK(c, cmax);
+                        live = !(qpart[c] > qmax[c]);
+                        if (!live) n_skip += 1ull;
+                    }
+                    const unsigned m = __ballot_sync(0xffffffffu, live);
+                    const int k = lane - pend, nl = __popc(m);
+                    const int v = __shfl_sync(0xffffffffu, u, (k >= 0 && k < nl) ? nth_set_bit(m, k) : lane);
+                    if (k >= 0 && k < nl) mine = v;
+                    pend += nl;
+                }
+                if (pend == 0) break;
+                if (lane < pend) {
+                    const int nq = fast_div(mine, na, inv_na), ai = mine - nq * na;
+                    YG_CHK(ai, cmax); YG_CHK(nq, nD);
+                    const int n = perm[nq], c = lst[ai];
+                    YG_CHK(n, nD); YG_CHK(c, cmax);
+                    const LvRates r = lv_rates(h, CH(BETA, c), CH(DELTA, c));
+                    double x = design[2 * n], y = design[2 * n + 1];
+                    integrate(Nrk, r, x, y);
+                    const double qn = misfit(n, x, y);
+                    q[n * cmax + c] = qn;
+                    atomicAdd(&qpart[c], qn);
+                }
+                pend = 0;
+                __syncwarp();
+            }
+            return;
         }
         for (;;) {
             int u = 0;
@@ -216,26 +326,13 @@ __global__ void __launch_bounds__(MAXT, 1) lv_mh_kernel(const RunArgs a, const i
                     __threadfence_block();
                     x = sx[it]; y = sy[it];
                 }
-#ifdef YG_TIMERS
-                lv_integrate(kc, r, a.thin == 7 ? 0 : min(seg_len, Nrk - seg * seg_len), x, y);   // thin == 7: overhead-only run
-#else
-                lv_integrate(kc, r, min(seg_len, Nrk - seg * seg_len), x, y);
-#endif
+                integrate(min(seg_len, Nrk - seg * seg_len), r, x, y);
                 if (seg + 1 < nSeg) {
                     sx[it] = x; sy[it] = y;
                     __threadfence_block();
                     *(volatile int *)(segdone + it) = seg + 1;
                 } else {
-                    // non-finite forward output -> +inf (policy of the oracle's RK4 plugin)
-                    x = isfinite(x) ? x : CUDART_INF;
-                    y = isfinite(y) ? y : CUDART_INF;
-                    const double r0 = x - data[2 * n], r1 = y - data[2 * n + 1];
-                    // r' P r with P applied first; exact zeros skipped (diagonal noise, inf-safe)
-                    double t0 = P00 * r0;
-                    if (P01 != 0.0) t0 = fma(P01, r1, t0);
-                    double t1 = (P10 != 0.0) ? P10 * r0 : 0.0;
-                    t1 = (P10 != 0.0) ? fma(P11, r1, t1) : P11 * r1;
-                    q[n * cmax + c] = fma(r1, t1, r0 * t0);
+                    q[n * cmax + c] = misfit(n, x, y);
                 }
             }
             __syncwarp();
@@ -255,8 +352,10 @@ __global__ void __launch_bounds__(MAXT, 1) lv_mh_kernel(const RunArgs a, const i
     };
 
     // noise: injected arrays are indexed by (step, sub-step), never by call count.  draw_z /
-    // draw_u fill the chain's slot of nz one sub-step ahead of its use, always from the thread
-    // that owns the chain (producer == consumer, no barrier needed).
+    // draw_u fill the chain's slot of nz one phase ahead of its use, always from the thread
+    // that owns the chain (producer == consumer, no barrier needed).  The uniform goes to slot 3:
+    // the owners' phase moves it to slot 2 after slot 2 decided the previous sub-step, so the
+    // budget of the proposals about to be evaluated is known before the barrier.
     auto draw_z = [&](int c, int64_t g, int64_t n, int j) {
         const uint64_t gid = (uint64_t)(a.chain_offset + g);
         const int64_t zi = ((n * J + j) * LV_D) * N + g;
@@ -283,7 +382,7 @@ __global__ void __launch_bounds__(MAXT, 1) lv_mh_kernel(const RunArgs a, const i
             u = philox_uniform(a.seed, gid, (uint64_t)(a.step0 + n), fine ? YG_SUB_FINE : (uint32_t)j);
             if (a.noise_mode == YG_NOISE_RECORD) arr[i] = u;
         }
-        nz[2 * cmax + c] = u;
+        nz[3 * cmax + c] = u;
     };
 
     // Adaptive Metropolis (chain/adaptive.py:55-60: update() before every proposal of the MRW chain it drives,
@@ -332,6 +431,7 @@ __global__ void __launch_bounds__(MAXT, 1) lv_mh_kernel(const RunArgs a, const i
     const long long dbg_start = dbg_last;
 #endif
     int cur = 0;
+    unsigned long long my_skip = 0ull;      // level-0 integrations skipped by early rejection
     for (int64_t cb = cta_lo; cb < cta_hi; cb += cmax) {
         const int C = (int)min((int64_t)cmax, cta_hi - cb);
         __syncthreads();
@@ -350,7 +450,10 @@ __global__ void __launch_bounds__(MAXT, 1) lv_mh_kernel(const RunArgs a, const i
             CH(W10, c) = a.w_m2[2 * N + g];
             CH(W11, c) = a.w_m2[3 * N + g];
             nacc[c] = a.n_accept[g];
-            if (a.n_steps > 0) draw_z(c, g, 0, 0);
+            if (a.n_steps > 0) {
+                draw_u(c, g, 0, 0, n_phases == 1);
+                draw_z(c, g, 0, 0);
+            }
         }
         unsigned long long my_acc = 0ull, my_cacc = 0ull;      // accepted transitions / accepted coarse sub-steps
 
@@ -363,7 +466,6 @@ __global__ void __launch_bounds__(MAXT, 1) lv_mh_kernel(const RunArgs a, const i
             // Phases j = 0..J-1: decide sub-step j-1, propose sub-step j, evaluate level 0.
             // Two level only, phase j = J: decide sub-step J-1, evaluate level 1 where the
             // sub-chain moved.  Then the commit below decides the transition.
-            const int n_phases = TWO_LEVEL ? J + 1 : 1;
             for (int j = 0; j < n_phases; j++) {
                 // =============== owners' phase ===================================
                 if (tid == 0) *qhead = 0;
@@ -386,15 +488,19 @@ __global__ void __launch_bounds__(MAXT, 1) lv_mh_kernel(const RunArgs a, const i
                         // coarse decision of sub-step j-1 (mrw.py:51-57)
                         s0 = CH(S0, c); s1 = CH(S1, c); lps = CH(LPS, c);
                         if (evald[c]) {
-                            const double p0 = CH(P0, c), p1 = CH(P1, c);
-                            const double lpp = log_post_from_q(0, c, p0, p1);
-                            if (accept_rule(lpp - lps, nz[2 * cmax + c])) {      // u_c(n, j-1)
-                                s0 = p0; s1 = p1; lps = lpp;
-                                my_cacc += 1ull;
+                                const double p0 = CH(P0, c), p1 = CH(P1, c);
+                            YG_CHK(c, cmax);
+                            if (!(skip_lvl0 && qpart[c] > qmax[c])) {           // else rejection certified
+                                const double lpp = log_post_from_q(0, c, p0, p1);
+                                if (accept_rule(lpp - lps, nz[2 * cmax + c])) {      // u_c(n, j-1)
+                                    s0 = p0; s1 = p1; lps = lpp;
+                                    my_cacc += 1ull;
+                                }
                             }
                         }
                     }
                     CH(S0, c) = s0; CH(S1, c) = s1; CH(LPS, c) = lps;
+                    nz[2 * cmax + c] = nz[3 * cmax + c];      // the uniform that decides this phase's proposals
                     if (j < J) {
                         double l00 = L00, l10 = L10, l11 = L11;
                         if (a.adaptive) am_update(cb + c, (a.am_t0 + n) * J + j, s0, s1, l00, l10, l11);
@@ -417,6 +523,12 @@ __global__ void __launch_bounds__(MAXT, 1) lv_mh_kernel(const RunArgs a, const i
                         if (!eq) {
                             CH(BETA, c) = exp(p0);     // LotkaVolterraParameter.evaluate, testSetup.py:57-58
                             CH(DELTA, c) = exp(p1);
+                            if (skip_lvl0) {
+                                qpart[c] = 0.0;
+                                qmax[c] = perm_ready ? reject_budget(log_prior(0, p0, p1), lps, nz[2 * cmax + c],
+                                                                     pb->lvl[0].tempering)
+                                                     : CUDART_INF;
+                            }
                             list_append(list0 + cur * cmax, &nact[cur], c, cmax);
                         }
                     } else {
@@ -443,15 +555,19 @@ __global__ void __launch_bounds__(MAXT, 1) lv_mh_kernel(const RunArgs a, const i
                 dbg_t[1] += tA - dbg_own;
                 if (tid == 0) dbg_t[6 + ((TWO_LEVEL && j == J) ? 1 : 0)] += nact[cur] * pb->lvl[(TWO_LEVEL && j == J) ? 1 : 0].n_data;
 #endif
-                // noise one sub-step ahead: the uniform that decides the proposals being evaluated
-                // now, and the normals of the next proposal
+                // noise one phase ahead: the uniform that decides the proposals of the next phase,
+                // and the normals of the next proposal
                 {
                     const bool last = (j == n_phases - 1);
                     for (int c = tid; c < C; c += nthr) {
                         const int64_t g = cb + c;
-                        draw_u(c, g, n, j, last);
-                        if (!last) { if (j + 1 < J) draw_z(c, g, n, j + 1); }
-                        else if (n + 1 < a.n_steps) draw_z(c, g, n + 1, 0);
+                        if (!last) {
+                            draw_u(c, g, n, j + 1, j + 1 == n_phases - 1);
+                            if (j + 1 < J) draw_z(c, g, n, j + 1);
+                        } else if (n + 1 < a.n_steps) {
+                            draw_u(c, g, n + 1, 0, n_phases == 1);
+                            draw_z(c, g, n + 1, 0);
+                        }
                     }
                 }
 #ifdef YG_TIMERS
@@ -459,8 +575,8 @@ __global__ void __launch_bounds__(MAXT, 1) lv_mh_kernel(const RunArgs a, const i
                 dbg_t[2] += dbg_nz - tA;
 #endif
                 // two inlined copies so that h and the chain-independent rates are constant-bank operands
-                if (TWO_LEVEL && j == J) eval_phase(1, cur, a.lv_h[1], a.lv_k[1]);
-                else eval_phase(0, cur, a.lv_h[0], a.lv_k[0]);
+                if (TWO_LEVEL && j == J) eval_phase(1, cur, a.lv_h[1], a.lv_k[1], my_skip);
+                else eval_phase(0, cur, a.lv_h[0], a.lv_k[0], my_skip);
 #ifdef YG_TIMERS
                 const long long dbg_ev = yg_clk();
                 dbg_t[3] += dbg_ev - dbg_nz;
@@ -470,6 +586,30 @@ __global__ void __launch_bounds__(MAXT, 1) lv_mh_kernel(const RunArgs a, const i
                 dbg_last = yg_clk();
                 dbg_t[4] += dbg_last - dbg_ev;
 #endif
+                if (skip_lvl0 && !perm_ready) {
+                    // first level-0 phase of the launch, evaluated in full: design points by total misfit,
+                    // largest first (ties by index), so that rejections are certified after fewer of them
+                    const int nD = pb->lvl[0].n_data, na = nact[cur];
+                    const int *lst = list0 + cur * cmax;
+                    for (int i = tid; i < nD; i += nthr) {
+                        double sum = 0.0;
+                        for (int k = 0; k < na; k++) {
+                            YG_CHK(lst[k], cmax);
+                            sum += q[i * cmax + lst[k]];
+                        }
+                        YG_CHK(i, nd_max);
+                        qsum[i] = sum;
+                    }
+                    __syncthreads();
+                    for (int i = tid; i < nD; i += nthr) {
+                        int rank = 0;
+                        for (int k = 0; k < nD; k++) rank += (qsum[k] > qsum[i] || (qsum[k] == qsum[i] && k < i)) ? 1 : 0;
+                        YG_CHK(rank, nd_max);
+                        perm[rank] = i;
+                    }
+                    __syncthreads();
+                    perm_ready = true;
+                }
                 cur ^= 1;
             }
             // =============== commit the transition ===============================
@@ -487,7 +627,7 @@ __global__ void __launch_bounds__(MAXT, 1) lv_mh_kernel(const RunArgs a, const i
                             CH(LP0, c) = CH(LPS, c); CH(LP1, c) = lpf_s;
                             accepted = true;
                         }
-                    } else {
+                    } else if (!(skip_lvl0 && qpart[c] > qmax[c])) {               // else rejection certified
                         const double p0 = CH(P0, c), p1 = CH(P1, c);
                         const double lpp = log_post_from_q(0, c, p0, p1);
                         if (accept_rule(lpp - CH(LP0, c), nz[2 * cmax + c])) {       // u_f(n)
@@ -536,6 +676,8 @@ __global__ void __launch_bounds__(MAXT, 1) lv_mh_kernel(const RunArgs a, const i
         }
         if (my_acc) atomicAdd(&blk_cnt[1], my_acc);
         if (my_cacc) atomicAdd(&blk_cnt[4], my_cacc);
+        if (my_skip) atomicAdd(&blk_cnt[5], my_skip);
+        my_skip = 0ull;
         if (tid == 0) blk_cnt[0] += (unsigned long long)C * (unsigned long long)a.n_steps;
     }
     __syncthreads();
@@ -549,6 +691,7 @@ __global__ void __launch_bounds__(MAXT, 1) lv_mh_kernel(const RunArgs a, const i
 #endif
     if (tid < 4 && blk_cnt[tid]) atomicAdd(&a.counters[tid], blk_cnt[tid]);
     if (tid == 4 && blk_cnt[4]) atomicAdd(&a.counters[5], blk_cnt[4]);       // [4] is the middle level of three-level problems
+    if (tid == 5 && blk_cnt[5]) atomicAdd(&a.counters[6], blk_cnt[5]);       // skipped level-0 integrations
 #undef CH
 }
 
@@ -557,13 +700,16 @@ size_t lv_smem_bytes(const yg_ensemble *e, int cmax, int nd_max)
     size_t off = (e->h_problem.size() + 15u) & ~size_t(15);
     off += sizeof(double) * SmemLayout::NDBL * cmax;
     off += sizeof(double) * (size_t)nd_max * cmax * 3;     // q, sx, sy
-    off += sizeof(double) * 3 * cmax;                      // nz
+    off += sizeof(double) * 4 * cmax;                      // nz
+    off += sizeof(double) * 2 * cmax;                      // qmax, qpart
+    off += sizeof(double) * nd_max;                        // qsum
     off += sizeof(unsigned long long) * cmax;
     off += sizeof(int) * 2 * cmax;
     off += sizeof(int) * (size_t)nd_max * cmax;           // segdone
+    off += sizeof(int) * nd_max;                           // perm
     off += (cmax + 15) & ~15;
     off = (off + 15) & ~size_t(15);
-    off += 8 + 8 + 40 + 8;
+    off += 8 + 8 + 48 + 8;
     return (off + 15) & ~size_t(15);
 }
 
@@ -596,7 +742,7 @@ int yg_launch_lv(yg_ensemble *e, const RunArgs &a, bool, cudaStream_t st)
     int64_t share = (a.n_chains + grid - 1) / grid;
     const size_t budget = (size_t)(220 * 1024) / bps;
     const size_t fixed = lv_smem_bytes(e, 0, nd_max);
-    const size_t per_chain = sizeof(double) * (SmemLayout::NDBL + 3 * nd_max + 3) + 4 * nd_max + 8 + 8 + 1;
+    const size_t per_chain = sizeof(double) * (SmemLayout::NDBL + 3 * nd_max + 6) + 4 * nd_max + 8 + 8 + 1;
     int64_t cap = fixed < budget ? (int64_t)((budget - fixed) / per_chain) : 0;
     if (cap < 1) {
         yg_set_error("problem blob too large for shared memory (%zu bytes)", fixed);
@@ -615,7 +761,7 @@ int yg_launch_lv(yg_ensemble *e, const RunArgs &a, bool, cudaStream_t st)
                                  : (two ? lv_mh_kernel<true, 1024> : lv_mh_kernel<false, 1024>);
     YG_CUDA_CHECK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     const int seg_len = e->cfg.rk4_segment > 0 ? e->cfg.rk4_segment : 128;
-    kern<<<grid, threads, smem, st>>>(args, cmax, seg_len);
+    kern<<<grid, threads, smem, st>>>(args, cmax, seg_len, e->cfg.early_reject_off == 0);
     YG_CUDA_CHECK(cudaGetLastError());
     e->last_grid = grid;
     e->last_block = threads;

@@ -111,7 +111,8 @@ class ChainEnsemble:
     """n_chains independent chains of one problem on one device."""
 
     def __init__(self, problem, n_chains, device=0, seed=0, chain_offset=0,
-                 adaptive=None, blocks_per_sm=0, threads_per_block=0, rk4_segment=0, aem=None, welford=True):
+                 adaptive=None, blocks_per_sm=0, threads_per_block=0, rk4_segment=0, aem=None, welford=True,
+                 early_reject=True):
         self.lib = _lib.load()
         if not torch.cuda.is_available():
             raise _lib.BackendUnavailable("no CUDA device visible: the batched-chain backend has no CPU fallback")
@@ -138,6 +139,8 @@ class ChainEnsemble:
         # welford=False: AcceptanceRateDiagnostics only (the reference builders' default, chain/builder.py:14-16);
         # honoured by the tensor-path kernel, whose Welford moments live in L2
         cfg.acceptance_only = 0 if welford else 1
+        # early_reject=False: the LV kernel integrates every design point of every proposal (same results)
+        cfg.early_reject_off = 0 if early_reject else 1
         self.aem = None
         if aem:             # adaptive error model: dict(min_data=..., heuristic=...)
             cfg.aem = 1
@@ -305,16 +308,24 @@ class ChainEnsemble:
             torch.cuda.current_stream(self.device).synchronize()
         return self
 
-    def counters(self):
-        buf = (C.c_int64 * 9)()
+    def _counters(self):
+        buf = (C.c_int64 * 10)()
         with torch.cuda.device(self.device):
             check(self.lib.yg_get_counters(self._h, buf, self._stream()))
+        return [int(x) for x in buf]
+
+    def counters(self):
         keys = ('step_index', 'transitions', 'accepted', 'coarse_evals', 'fine_evals', 'welford_n', 'am_steps',
                 'mid_evals', 'coarse_accepted')
-        c = dict(zip(keys, [int(x) for x in buf]))
+        c = dict(zip(keys, self._counters()))
         if self.levels == 1:        # single level: level 0 IS the target
             c['fine_evals'], c['coarse_evals'] = c['coarse_evals'], 0
         return c
+
+    def skipped_evals(self):
+        """Level-0 integrations (proposal, design point) skipped since set_state because the proposal's rejection
+        was already certain.  Unlike counters(), it depends on the launch geometry and the scheduling."""
+        return self._counters()[9]
 
     def logpost(self, level, theta):
         t = torch.as_tensor(theta, dtype=torch.float64).to(self.device)
