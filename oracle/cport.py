@@ -123,7 +123,8 @@ class Problem:
 
 
 def run_injected(problem, theta0, z, u_c, u_f, n_threads=0):
-    """theta0[nc,d] z[nc,ns,J,d] u_c[nc,ns,J] u_f[nc,ns] -> dict of outputs (chain-major)."""
+    """theta0[nc,d] z[nc,ns,J,d] u_c[nc,ns,J] u_f[nc,ns] -> dict of outputs (chain-major).
+    coarse_accepted[nc]: accepted sub-steps of the coarse sub-chain per chain (zero for a single level)."""
     theta0, z, u_c, u_f = _arr(theta0), _arr(z), _arr(u_c), _arr(u_f)
     nc, ns = u_f.shape
     d = problem.dim
@@ -139,13 +140,15 @@ def run_injected(problem, theta0, z, u_c, u_f, n_threads=0):
     dd = int(problem.pb.level[0].data_dim)
     aem = np.zeros((nc, 2 + 2 * max(dd, 1)))
     am = np.zeros((nc, d + 2 * d * d))
+    cacc = np.zeros(nc, dtype=np.int64)
     rc = lib().yo_run_injected(C.byref(problem.pb), C.c_int64(nc), C.c_int64(ns),
                                _ptr(theta0), _ptr(z), _ptr(u_c), _ptr(u_f), _ptr(traj),
                                acc.ctypes.data_as(C.c_void_p), _ptr(lp0), _ptr(lp1), _ptr(lp2), _ptr(wm), _ptr(wv),
-                               ev.ctypes.data_as(C.c_void_p), C.c_int(n_threads), _ptr(aem), _ptr(am))
+                               ev.ctypes.data_as(C.c_void_p), C.c_int(n_threads), _ptr(aem), _ptr(am),
+                               cacc.ctypes.data_as(C.c_void_p))
     assert rc == 0
     out = dict(traj=traj, accepted=acc, logpost_L0=lp0, logpost_L1=lp1, logpost_L2=lp2,
-               welford_mean=wm, welford_var=wv, n_evals=ev)
+               welford_mean=wm, welford_var=wv, n_evals=ev, coarse_accepted=cacc)
     if problem.pb.adaptive:
         out.update(am_mean=am[:, :d].copy(), am_m2=am[:, d:d + d * d].reshape(nc, d, d).copy(),
                    am_L=am[:, d + d * d:].reshape(nc, d, d).copy())

@@ -341,6 +341,7 @@ typedef struct {
     double theta[YO_MAX_DIM];
     double lp[3];                  /* log-posterior of theta per level */
     int64_t n_accept;
+    int64_t n_coarse_accept;       /* accepted coarse sub-steps (the device's coarse_accepted counter) */
     int64_t n_evals[3];
     int64_t w_n;                   /* Welford (estimation.py:36-53), fed the PRE-transition state */
     double w_mean[YO_MAX_DIM], w_m2[YO_MAX_DIM];
@@ -541,7 +542,10 @@ static int chain_step_aem(const yo_problem *pb, chain_state *cs, const noise_src
         if (param_equal(pb, p, s)) continue;
         const double lpp = aem_query_coarse(pb, cs, p);      /* mrw.py:53: proposal first, then state */
         const double lps = aem_query_coarse(pb, cs, s);
-        if (accept_rule(lpp - lps, get_uc(pb, ns, n, j))) memcpy(s, p, sizeof(double) * d);
+        if (accept_rule(lpp - lps, get_uc(pb, ns, n, j))) {
+            memcpy(s, p, sizeof(double) * d);
+            cs->n_coarse_accept++;
+        }
     }
     if (param_equal(pb, s, cs->theta)) return 0;
     /* mlda.py:148-152: pi_f(P) + pi_c(theta) - pi_c(P) - pi_f(theta), evaluated in this order */
@@ -602,6 +606,7 @@ static int chain_step(const yo_problem *pb, chain_state *cs, const noise_src *ns
         if (accept_rule(lpp - lpc_s, get_uc(pb, ns, n, j))) {
             memcpy(s, p, sizeof(double) * d);
             lpc_s = lpp;
+            cs->n_coarse_accept++;
         }
     }
     if (param_equal(pb, s, cs->theta)) return 0;         /* no fine evaluation, no uniform */
@@ -641,9 +646,11 @@ static int chain_step(const yo_problem *pb, chain_state *cs, const noise_src *ns
 int yo_run_injected(const yo_problem *pb, int64_t nc, int64_t ns,
                     const double *theta0, const double *z, const double *u_c, const double *u_f,
                     double *traj, uint8_t *accepted, double *lp0, double *lp1, double *lp2,
-                    double *w_mean, double *w_var, int64_t *n_evals, int n_threads, double *aem_out, double *am_out)
+                    double *w_mean, double *w_var, int64_t *n_evals, int n_threads, double *aem_out, double *am_out,
+                    int64_t *coarse_accepted)
 {   /* aem_out[nc, 2 + 2 data_dim]: error samples, coarse model evaluations, error mean, error variance
-     * am_out[nc, d + 2 d d]: adaptive Metropolis mean, M2, proposal factor L after the last transition */
+     * am_out[nc, d + 2 d d]: adaptive Metropolis mean, M2, proposal factor L after the last transition
+     * coarse_accepted[nc] (may be NULL): accepted sub-steps of the coarse sub-chain, summed over all transitions */
     const int d = pb->dim, J = pb->J;
     if (d > YO_MAX_DIM || pb->n_levels < 1 || pb->n_levels > 3) return -1;
     for (int l = 0; l < pb->n_levels; l++) if (pb->model != YO_GAUSS && pb->level[l].data_dim > YO_MAX_DATA) return -1;
@@ -670,6 +677,7 @@ int yo_run_injected(const yo_problem *pb, int64_t nc, int64_t ns,
             if (w_var) w_var[c * d + i] = cs.w_n > 1 ? cs.w_m2[i] / (double)(cs.w_n - 1) : NAN;
         }
         ev0 += cs.n_evals[0]; ev1 += cs.n_evals[1]; ev2 += cs.n_evals[2];
+        if (coarse_accepted) coarse_accepted[c] = cs.n_coarse_accept;
         if (am_out && pb->adaptive) {
             double *o = am_out + (size_t)c * (d + 2 * d * d);
             memcpy(o, cs.am_mean, sizeof(double) * d);

@@ -7,6 +7,7 @@ import pytest
 import torch
 
 import bench_problems as bp
+from diag_reference import check_replay_diagnostics, pre_states
 from golden_io import load, rel_err
 
 pytestmark = pytest.mark.gpu
@@ -70,6 +71,7 @@ def test_philox_run_replayed_through_oracle(name):
     if meta["levels"] == 2:
         # nc evaluations per level belong to the initial state in the oracle's count
         assert (c["coarse_evals"], c["fine_evals"]) == (int(ev[0]) - nc, int(ev[1]) - nc)
+    check_replay_diagnostics(ens.state(), c, ref, pre_states(th0, [out["samples"].cpu().numpy()]), name)
     z = out["z"].cpu().numpy()
     assert abs(z.mean()) < 0.02 and abs(z.var() - 1.0) < 0.03          # the recorded draws are N(0,1)
 

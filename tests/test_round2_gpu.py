@@ -5,6 +5,7 @@ import pytest
 import torch
 
 import bench_problems as bp
+from diag_reference import check_replay_diagnostics, pre_states
 from golden_io import load, rel_err
 
 pytestmark = pytest.mark.gpu
@@ -573,6 +574,13 @@ def test_seeded_shape_sweep_replayed_through_oracle(k):
         assert rel_err(lp[:, :, 1], ref["logpost_L1"][:, thin::thin]).max() <= LOGPOST_RTOL, label
     c = ens.counters()
     assert c["transitions"] == nc * ns and c["accepted"] == int(acc.sum()), label
+    # the diagnostics: Welford over every step even when the output is thinned (then the reference is built from the
+    # replay's trajectory, equal to the device's to 1e-12), coarse_accepted against the oracle's count
+    if thin == 1:
+        pre, traj_rtol = pre_states(th0, [out["samples"].cpu().numpy()]), 0.0
+    else:
+        pre, traj_rtol = ref["traj"][:, :ns], 1e-12
+    check_replay_diagnostics(ens.state(), c, ref, pre, label, traj_rtol)
     ens.close()
 
 
