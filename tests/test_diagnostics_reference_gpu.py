@@ -247,7 +247,7 @@ def test_adaptive_error_model_kernel_diagnostics():
 def _tensor_path_launch(d, rows, dense_L):
     """(wsm, dynamic shared memory) of linear_dmma_kernel.cu's launch_t for a model with d parameters and `rows` operand
     rows per level (data_dim, + d for a dense prior): the problem blob (abi.cu's tail), then as many warps as fit
-    (12 at most for d > 32, else 16), each with its state and noise tiles (big_warp_bytes), plus the two Welford tiles
+    (12 at most for d > 32, else 16), each with its state and noise tiles (smem_plan.h), plus the two Welford tiles
     per warp when the blob leaves room for them at that warp count -- the shared-memory side of `wsm`; otherwise the
     moments are read and written in L2 at every flush."""
     kp = 16 if d <= 16 else (32 if d <= 32 else 64)

@@ -65,6 +65,15 @@ def _near_zero_tensor():
     return meta, dict(arrays, L0_noise_prec=np.full((1, 1), 1e-6), L0_prior_prec=1e-6 * np.eye(9))
 
 
+def _tensor_4_warps():
+    """d = 64, two levels of 176 and 192 rows: the blob (206,208 bytes) and four warps' tiles take 232,320 bytes, within
+    the 227 KiB of one block."""
+    meta, arrays = bp.big_linear_problem(64, 192, 1, two_level=True, J=2, seed=9)
+    r = slice(0, 176)
+    return meta, dict(arrays, L0_data=arrays["L0_data"][:, r], L0_G=arrays["L0_G"][r], L0_b=arrays["L0_b"][r],
+                      L0_noise_prec=arrays["L0_noise_prec"][r, r])
+
+
 def _theta(meta, n, seed, scale=0.3):
     if meta["model"] == "lv":
         return bp.lv_initial_states(n, seed=seed) + np.random.default_rng(seed).uniform(-1, 1, (n, 2)) * 0.5
@@ -158,6 +167,7 @@ TENSOR = {
     "dense_prior": _dense_prior_tensor,
     "q_const_dominated": _qconst_tensor,
     "near_zero": _near_zero_tensor,
+    "64x176_192_four_warps": _tensor_4_warps,
 }
 
 

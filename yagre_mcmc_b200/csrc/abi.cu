@@ -2,6 +2,7 @@
 // Plain pointers and sizes only; no torch types, no exceptions across the boundary.
 #include "ensemble.h"
 #include "big_linear.h"
+#include "smem_plan.h"
 #include <cstdarg>
 #include <cstdio>
 #include <cstring>
@@ -250,12 +251,9 @@ int build_big_blob(const yg_config &c, const yg_problem *pb, std::vector<char> &
     }
     tail_len += 2 * (size_t)kp + (dense_L ? (size_t)kp * ks : 0);
     tail_len = (tail_len + 1) & ~size_t(1);
-    {   // the blob and the tiles of at least four warps (state tile, noise tile, + a scratch tile for a dense factor)
-        const size_t per_warp = sizeof(double) * 8 * (size_t)ks * (dense_L ? 2 : 1) + sizeof(float) * 8 * (size_t)(kp + 4);
-        if (sizeof(double) * tail_len + 4 * per_warp > 226 * 1024) {
-            yg_set_error("large linear model: %zu bytes of G / data do not fit the shared memory of one SM", sizeof(double) * tail_len);
-            return YG_ERR_UNSUPPORTED;
-        }
+    if (big_smem_plan((int)tail_len, ks, kp / 4, dense_L, false).warps < BIG_MIN_WARPS) {
+        yg_set_error("large linear model: %zu bytes of G / data do not fit the shared memory of one SM", sizeof(double) * tail_len);
+        return YG_ERR_UNSUPPORTED;
     }
     blob.assign(sizeof(DevBigHeader) + sizeof(double) * tail_len, 0);
     DevBigHeader *h = reinterpret_cast<DevBigHeader *>(blob.data());
@@ -761,8 +759,8 @@ extern "C" int yg_run(yg_ensemble *e, int64_t n_steps, int32_t thin, const yg_ou
     }
     YG_CUDA_CHECK(cudaSetDevice(e->cfg.device));
     rc = e->big ? yg_launch_linear_big(e, a, (cudaStream_t)stream)
-         : (e->cfg.model == YG_MODEL_LV_RK4) ? yg_launch_lv(e, a, false, (cudaStream_t)stream)
-                                             : yg_launch_generic(e, a, false, (cudaStream_t)stream);
+         : (e->cfg.model == YG_MODEL_LV_RK4) ? yg_launch_lv(e, a, (cudaStream_t)stream)
+                                             : yg_launch_generic(e, a, (cudaStream_t)stream);
     if (rc) return rc;
     e->step_index += n_steps;
     e->welford_n += n_steps;

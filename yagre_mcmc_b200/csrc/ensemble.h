@@ -72,8 +72,8 @@ struct yg_ensemble {
 };
 
 // kernels' host launchers (lv_kernel.cu, generic_kernel.cu, diag_kernels.cu)
-int yg_launch_lv(yg_ensemble *e, const RunArgs &a, bool init_only, cudaStream_t st);
-int yg_launch_generic(yg_ensemble *e, const RunArgs &a, bool init_only, cudaStream_t st);
+int yg_launch_lv(yg_ensemble *e, const RunArgs &a, cudaStream_t st);
+int yg_launch_generic(yg_ensemble *e, const RunArgs &a, cudaStream_t st);
 int yg_launch_logpost(yg_ensemble *e, int level, const double *theta, int64_t n, double *out, cudaStream_t st);
 int yg_launch_linear_big(yg_ensemble *e, const RunArgs &a, cudaStream_t st);
 int yg_launch_logpost_big(yg_ensemble *e, int level, const double *theta, int64_t n, double *out, cudaStream_t st);

@@ -14,7 +14,7 @@ namespace {
 int cap_of(int n) { return n <= 2 ? 2 : (n <= 4 ? 4 : 8); }
 }  // namespace
 
-int yg_launch_generic(yg_ensemble *e, const RunArgs &a, bool, cudaStream_t st)
+int yg_launch_generic(yg_ensemble *e, const RunArgs &a, cudaStream_t st)
 {
     const DevProblemHeader *hp = reinterpret_cast<const DevProblemHeader *>(e->h_problem.data());
     const int cd = cap_of(hp->dim);

@@ -23,6 +23,7 @@
 #pragma once
 #include "ensemble.h"
 #include "lv_model.cuh"
+#include "smem_plan.h"
 #include <math_constants.h>
 #include <algorithm>
 
@@ -185,7 +186,6 @@ YG_DEVFN bool cholesky_lower(const double (&C)[D][D], double (&L)[D][D], int d)
 // warps 1 and 2 PRODUCE the normals and uniforms of the coming sub-steps into a shared-memory ring, warp 0
 // CONSUMES them and runs only the state-dependent half.  Same streams, same arithmetic: trajectories are
 // bit-identical to the unspecialised kernel (tests/test_backend_gpu.py).
-constexpr int WS_RING = 16;                // ring entries; one entry = (z0, z1, u) of one sub-step for 32 chains
 constexpr int WS_THREADS = 64;             // 1 consumer warp + 1 producer warp (more producers measured no gain)
 constexpr int64_t WS_MAX_CHAINS = 32768;   // beyond this the plain kernel has enough warps per sub-partition
 
@@ -199,6 +199,7 @@ __global__ void __launch_bounds__(WS ? WS_THREADS : 128) generic_mh_kernel(const
         ws_ring = reinterpret_cast<double *>(smem_raw + ((a.problem_bytes + 15u) & ~15u));       // [WS_RING][3][32]
         ws_ready = reinterpret_cast<volatile unsigned long long *>(ws_ring + WS_RING * 96);     // [WS_RING]
         ws_consumed = ws_ready + WS_RING;
+        YG_CHK(((a.problem_bytes + 15u) & ~15u) + WS_RING_BYTES - 1, yg_dynamic_smem_bytes());  // the ring fits the launch
         if (threadIdx.x <= WS_RING) ws_ready[threadIdx.x] = 0ull;                               // incl. ws_consumed
     }
     stage_blob(smem_raw, a.problem, a.problem_bytes);
@@ -935,7 +936,7 @@ int launch_generic_t(yg_ensemble *e, const RunArgs &a, cudaStream_t st)
         kern = e->cfg.n_levels >= 2 ? generic_mh_kernel<D, DD, true, D == 2> : generic_mh_kernel<D, DD, false, D == 2>;
         threads = WS_THREADS;
         grid = (int)((a.n_chains + 31) / 32);
-        smem += sizeof(double) * WS_RING * 96 + sizeof(unsigned long long) * (WS_RING + 1);
+        smem += WS_RING_BYTES;
     }
     YG_CUDA_CHECK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     kern<<<grid, threads, smem, st>>>(a);

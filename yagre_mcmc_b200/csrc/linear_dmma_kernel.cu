@@ -45,6 +45,7 @@
 //     the FP64 pipe would cost as much as a fifth of the GEMM.
 #include "ensemble.h"
 #include "big_linear.h"
+#include "smem_plan.h"
 #include <math_constants.h>
 
 namespace {
@@ -262,29 +263,13 @@ YG_DEVFN double logpost_tile(const SmemLevel &L, const int ks, const double (&a)
     return -0.5 * (q + L.q_const) + (-0.5 * quad_sum(pr));
 }
 
-constexpr int BIG_WARPS = 16;      // most warps per CTA (8 chains each, <= 128 registers per thread); fewer when shared memory is short
-// d > 32 (KQ = 16): G of a 256-row model leaves shared memory for 13 warps; 12 are used -- three per sub-partition may
-// take 168 registers each (a fourth warp on one sub-partition caps everybody at 128: the register file is per
-// sub-partition), which the 64-parameter operand tiles need: no spills, 25.2 against 20.7 TFLOP/s with 13 x 128.
-#ifndef YG_BIG_WARPS_KQ16
-#define YG_BIG_WARPS_KQ16 12
-#endif
-__host__ __device__ constexpr int big_max_warps(int kq) { return kq == 16 ? YG_BIG_WARPS_KQ16 : BIG_WARPS; }
-// per-warp shared memory: the state tile [8][ks] doubles and the noise tile [8][4 KQ + 4] floats of the next proposal
-__host__ __device__ constexpr int big_zs(int kq) { return 4 * kq + 4; }
-// (+ a second [8][ks] tile when the proposal factor is dense: the transpose buffer of L z)
-inline size_t big_warp_bytes(int ks, int kq, bool dense_L, bool wsm)
-{
-    return sizeof(double) * 8 * (size_t)ks * (1 + (dense_L ? 1 : 0) + (wsm ? 2 : 0)) + sizeof(float) * 8 * (size_t)big_zs(kq);
-}
-
 // FREE_NOISE = true: the production instance (Philox noise, diagonal proposal factor).  The injected / recorded noise
 // paths of the parity tests and the DENSE proposal factor (p = s + L z with L z as a second small GEMM) live in the
 // FREE_NOISE = false instance, which keeps the step loop of the production one small enough for the instruction cache
 // (stall reason no_instruction in profiles/r01_linear_dmma.md).
 template <int KQ, bool TWO_LEVEL, bool FREE_NOISE>
 __global__ void __launch_bounds__(big_max_warps(KQ) * 32, 1) linear_dmma_mh_kernel(const RunArgs a, const DevBigHeader *gh,
-                                                                          long long *tile_done, const int wsm)
+                                                                          long long *tile_done, const BigSmemPlan sp)
 {
     const int noise_mode = FREE_NOISE ? (int)YG_NOISE_PHILOX : a.noise_mode;
     extern __shared__ __align__(16) double smem[];
@@ -315,16 +300,16 @@ __global__ void __launch_bounds__(big_max_warps(KQ) * 32, 1) linear_dmma_mh_kern
     const int n_warps = blockDim.x >> 5;
     const bool dense_L = !FREE_NOISE && H.dense_L;
     const double *Ld = smem + H.Ld_off;            // [kp][ks] lower-triangular proposal factor (dense_L only)
-    // per-warp tiles: state [8][ks]; (dense factor only) the transpose buffer of L z [8][ks]; (wsm: when shared memory
-    // allows) the Welford mean and second moment of the tile, 2 x [8][ks]; the noise tile [8][ZS] floats
-    const int n_dtiles = 1 + (dense_L ? 1 : 0) + (wsm ? 2 : 0);
-    double *ths = smem + ((H.tail_len + 1) & ~1) + (size_t)warp * (8 * ks * n_dtiles + 4 * ZS);   // 8 ZS floats = 4 ZS doubles
-    double *scr = ths + 8 * ks;                    // (dense_L only)
-    double *wmt = ths + 8 * ks * (dense_L ? 2 : 1), *wvt = wmt + 8 * ks;      // (wsm only)
-    float *zb = reinterpret_cast<float *>(ths + 8 * ks * n_dtiles);
+    // the warp's tiles (smem_plan.h): state, transpose buffer of L z (dense_L only), Welford moments (wsm only), noise
+    const int wsm = sp.wsm;
+    unsigned char *wreg = reinterpret_cast<unsigned char *>(smem) + sp.blob + (size_t)warp * sp.stride;
+    double *ths = reinterpret_cast<double *>(wreg);
+    double *scr = reinterpret_cast<double *>(wreg + sp.scr);
+    double *wmt = reinterpret_cast<double *>(wreg + sp.wm), *wvt = reinterpret_cast<double *>(wreg + sp.wv);
+    float *zb = reinterpret_cast<float *>(wreg + sp.zb);
 #ifdef YG_BOUNDS_CHECK
     // every per-warp tile is [8][ks] doubles; the warp's region must end inside the dynamic shared memory of the launch
-    YG_CHK(reinterpret_cast<unsigned char *>(zb + 8 * ZS) - reinterpret_cast<unsigned char *>(smem) - 1, yg_dynamic_smem_bytes());
+    YG_CHK(sp.blob + (size_t)(warp + 1) * sp.stride - 1, yg_dynamic_smem_bytes());
     auto tile_at = [&](double *tile, const int i) -> double & {
         YG_CHK(g * ks + 4 * i + t, 8 * ks);
         return tile[g * ks + 4 * i + t];
@@ -733,35 +718,24 @@ template <int KQ>
 int launch_t(yg_ensemble *e, const RunArgs &a, cudaStream_t st)
 {
     const DevBigHeader *hh = reinterpret_cast<const DevBigHeader *>(e->h_problem.data());
-    // warps per CTA: as many as the shared memory left by the problem blob holds (13 at d = 64 x 256, else 16)
-    const bool dense_L = hh->dense_L != 0;
-    const size_t blob = sizeof(double) * (((size_t)hh->tail_len + 1) & ~size_t(1));
-    const size_t budget = 227 * 1024;
-    // Welford moments of the tiles in shared memory when that costs no warp (and FullDiagnostics asked for them at all)
-    size_t per_warp = big_warp_bytes(hh->ks, KQ, dense_L, false);
-    int warps = blob < budget ? (int)std::min<size_t>(big_max_warps(KQ), (budget - blob) / per_warp) : 0;
-    const size_t per_warp_w = big_warp_bytes(hh->ks, KQ, dense_L, true);
-    const bool wsm = a.welford && warps >= 4 && blob + (size_t)warps * per_warp_w <= budget;
-    if (wsm) per_warp = per_warp_w;
-    if (warps < 4) {
-        yg_set_error("large linear model: %zu bytes of G / data leave no room for the per-warp tiles", blob);
-        return YG_ERR_UNSUPPORTED;
-    }
-    const size_t smem = blob + (size_t)warps * per_warp;
-    const bool free_noise = a.noise_mode == YG_NOISE_PHILOX && !dense_L;      // the general instance also knows dense factors
+    // warps per CTA: as many as the shared memory left by the problem blob holds (13 at d = 64 x 256, else 16; yg_set_problem
+    // refused a blob that leaves fewer than BIG_MIN_WARPS); Welford moments of the tiles in shared memory when that costs no
+    // warp (and FullDiagnostics asked for them at all)
+    const BigSmemPlan sp = big_smem_plan(hh->tail_len, hh->ks, KQ, hh->dense_L != 0, a.welford != 0);
+    const bool free_noise = a.noise_mode == YG_NOISE_PHILOX && !hh->dense_L;      // the general instance also knows dense factors
     auto kern = e->cfg.n_levels == 2
                     ? (free_noise ? linear_dmma_mh_kernel<KQ, true, true> : linear_dmma_mh_kernel<KQ, true, false>)
                     : (free_noise ? linear_dmma_mh_kernel<KQ, false, true> : linear_dmma_mh_kernel<KQ, false, false>);
-    YG_CUDA_CHECK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    YG_CUDA_CHECK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sp.total));
     const int64_t tiles = (a.n_chains + 7) / 8;
     // persistent grid, every CTA resident (one per SM): the balanced schedule lets warps wait on one another
-    const int grid = (int)std::max<int64_t>(1, std::min<int64_t>((tiles + warps - 1) / warps, e->sm_count));
+    const int grid = (int)std::max<int64_t>(1, std::min<int64_t>((tiles + sp.warps - 1) / sp.warps, e->sm_count));
     YG_CUDA_CHECK(cudaMemsetAsync(e->big_done, 0, sizeof(long long) * (size_t)tiles, st));
-    kern<<<grid, warps * 32, smem, st>>>(a, reinterpret_cast<const DevBigHeader *>(e->d_problem), e->big_done, wsm ? 1 : 0);
+    kern<<<grid, sp.warps * 32, sp.total, st>>>(a, reinterpret_cast<const DevBigHeader *>(e->d_problem), e->big_done, sp);
     YG_CUDA_CHECK(cudaGetLastError());
     e->last_grid = grid;
-    e->last_block = warps * 32;
-    e->last_smem = (int)smem;
+    e->last_block = sp.warps * 32;
+    e->last_smem = (int)sp.total;
     e->launches += 1;
     return YG_OK;
 }
@@ -771,9 +745,9 @@ int launch_t(yg_ensemble *e, const RunArgs &a, cudaStream_t st)
 int yg_launch_linear_big(yg_ensemble *e, const RunArgs &a, cudaStream_t st)
 {
     const DevBigHeader *hh = reinterpret_cast<const DevBigHeader *>(e->h_problem.data());
-    switch (hh->kp / 4) {
-    case 1: case 2: case 3: case 4: return launch_t<4>(e, a, st);
-    case 5: case 6: case 7: case 8: return launch_t<8>(e, a, st);
+    switch (hh->kp) {       // 16, 32 or 64 (build_big_blob)
+    case 16: return launch_t<4>(e, a, st);
+    case 32: return launch_t<8>(e, a, st);
     default: return launch_t<16>(e, a, st);
     }
 }

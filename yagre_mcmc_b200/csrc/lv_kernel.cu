@@ -32,16 +32,12 @@
 //     work of the warps that are already integrating.
 #include "ensemble.h"
 #include "lv_model.cuh"
+#include "smem_plan.h"
 #include <math_constants.h>
 
 namespace {
 
 constexpr int LV_D = 2;
-
-struct SmemLayout {
-    // doubles per chain slot
-    enum { TH0, TH1, LP0, LP1, S0, S1, LPS, P0, P1, BETA, DELTA, WM0, WM1, W00, W01, W10, W11, NDBL };
-};
 
 #ifdef YG_TIMERS
 YG_DEVFN long long yg_clk()
@@ -119,48 +115,33 @@ YG_DEVFN int nth_set_bit(unsigned m, int k)
 }
 
 template <bool TWO_LEVEL, int MAXT>
-__global__ void __launch_bounds__(MAXT, 1) lv_mh_kernel(const RunArgs a, const int cmax, const int seg_len,
+__global__ void __launch_bounds__(MAXT, 1) lv_mh_kernel(const RunArgs a, const LvSmemPlan sp, const int seg_len,
                                                           const bool early_reject)
 {
     extern __shared__ __align__(16) unsigned char smem_raw[];
     const int tid = threadIdx.x, nthr = blockDim.x;
 
-    // ---- shared memory carve-up ------------------------------------------------
+    // ---- shared memory carve-up (smem_plan.h) ------------------------------------
+    const int cmax = sp.cmax, nd_max = sp.nd_max;
     DevProblemHeader *pb = reinterpret_cast<DevProblemHeader *>(smem_raw);
-    size_t off = (a.problem_bytes + 15u) & ~size_t(15);
-    double *chain = reinterpret_cast<double *>(smem_raw + off);            // [NDBL][cmax]
-    off += sizeof(double) * SmemLayout::NDBL * cmax;
-    const int nd_max = max(a.problem->lvl[0].n_data, TWO_LEVEL ? a.problem->lvl[1].n_data : 0);
-    double *q = reinterpret_cast<double *>(smem_raw + off);                // [n_data][cmax]
-    off += sizeof(double) * (size_t)nd_max * cmax;
-    double *sx = reinterpret_cast<double *>(smem_raw + off);               // [n_data * cmax] ODE state between
-    off += sizeof(double) * (size_t)nd_max * cmax;                         //   segments, indexed by item
-    double *sy = reinterpret_cast<double *>(smem_raw + off);
-    off += sizeof(double) * (size_t)nd_max * cmax;
-    double *nz = reinterpret_cast<double *>(smem_raw + off);               // [4][cmax] z0, z1, uniform, next uniform
-    off += sizeof(double) * 4 * cmax;
-    double *qmax = reinterpret_cast<double *>(smem_raw + off);             // [cmax] misfit budget (reject_budget)
-    off += sizeof(double) * cmax;
-    double *qpart = reinterpret_cast<double *>(smem_raw + off);            // [cmax] misfit summed so far
-    off += sizeof(double) * cmax;
-    double *qsum = reinterpret_cast<double *>(smem_raw + off);             // [n_data] misfit per design point
-    off += sizeof(double) * nd_max;
-    unsigned long long *nacc = reinterpret_cast<unsigned long long *>(smem_raw + off);   // [cmax]
-    off += sizeof(unsigned long long) * cmax;
-    int *list0 = reinterpret_cast<int *>(smem_raw + off);                  // [2][cmax]
-    off += sizeof(int) * 2 * cmax;
-    int *segdone = reinterpret_cast<int *>(smem_raw + off);                // [n_data * cmax] segments done per item
-    off += sizeof(int) * (size_t)nd_max * cmax;
-    int *perm = reinterpret_cast<int *>(smem_raw + off);                   // [n_data] level-0 design points, heaviest first
-    off += sizeof(int) * nd_max;
-    unsigned char *evald = smem_raw + off;                                 // [cmax]
-    off += (cmax + 15) & ~15;
-    off = (off + 15) & ~size_t(15);      // the int arrays above leave 4-byte alignment when n_data * cmax is odd
-    uint64_t *mbar = reinterpret_cast<uint64_t *>(smem_raw + off);
-    int *nact = reinterpret_cast<int *>(mbar + 1);                         // [2]
-    unsigned long long *blk_cnt = reinterpret_cast<unsigned long long *>(mbar + 2);   // [6]
-    int *qhead = reinterpret_cast<int *>(mbar + 8);                        // work-queue head of the current phase
-    YG_CHK(reinterpret_cast<unsigned char *>(qhead + 1) - smem_raw - 1, yg_dynamic_smem_bytes());   // the carve-up fits the launch
+    double *chain = reinterpret_cast<double *>(smem_raw + sp.off[LV_CHAIN]);
+    double *q = reinterpret_cast<double *>(smem_raw + sp.off[LV_Q]);
+    double *sx = reinterpret_cast<double *>(smem_raw + sp.off[LV_SX]);
+    double *sy = reinterpret_cast<double *>(smem_raw + sp.off[LV_SY]);
+    double *nz = reinterpret_cast<double *>(smem_raw + sp.off[LV_NZ]);
+    double *qmax = reinterpret_cast<double *>(smem_raw + sp.off[LV_QMAX]);
+    double *qpart = reinterpret_cast<double *>(smem_raw + sp.off[LV_QPART]);
+    double *qsum = reinterpret_cast<double *>(smem_raw + sp.off[LV_QSUM]);
+    unsigned long long *nacc = reinterpret_cast<unsigned long long *>(smem_raw + sp.off[LV_NACC]);
+    int *list0 = reinterpret_cast<int *>(smem_raw + sp.off[LV_LIST0]);
+    int *segdone = reinterpret_cast<int *>(smem_raw + sp.off[LV_SEGDONE]);
+    int *perm = reinterpret_cast<int *>(smem_raw + sp.off[LV_PERM]);
+    unsigned char *evald = smem_raw + sp.off[LV_EVALD];
+    uint64_t *mbar = reinterpret_cast<uint64_t *>(smem_raw + sp.mbar);
+    int *nact = reinterpret_cast<int *>(smem_raw + sp.nact);
+    unsigned long long *blk_cnt = reinterpret_cast<unsigned long long *>(smem_raw + sp.blk_cnt);
+    int *qhead = reinterpret_cast<int *>(smem_raw + sp.qhead);        // work-queue head of the current phase
+    YG_CHK(sp.total - 1, yg_dynamic_smem_bytes());                     // the plan fits the launch
 
     tma_stage_blob(pb, a.problem, (uint32_t)((a.problem_bytes + 15u) & ~15u), mbar);
     if (tid < 6) blk_cnt[tid] = 0ull;
@@ -196,9 +177,9 @@ __global__ void __launch_bounds__(MAXT, 1) lv_mh_kernel(const RunArgs a, const i
         YG_CHK(c, cmax);
         return chain[field * cmax + c];
     };
-#define CH(field, c) ch_at(SmemLayout::field, (c))
+#define CH(field, c) ch_at(LvSlot::field, (c))
 #else
-#define CH(field, c) chain[(SmemLayout::field) * cmax + (c)]
+#define CH(field, c) chain[(LvSlot::field) * cmax + (c)]
 #endif
 
     // chains of this CTA: even split of [0, n_chains) over the grid
@@ -695,61 +676,24 @@ __global__ void __launch_bounds__(MAXT, 1) lv_mh_kernel(const RunArgs a, const i
 #undef CH
 }
 
-size_t lv_smem_bytes(const yg_ensemble *e, int cmax, int nd_max)
-{
-    size_t off = (e->h_problem.size() + 15u) & ~size_t(15);
-    off += sizeof(double) * SmemLayout::NDBL * cmax;
-    off += sizeof(double) * (size_t)nd_max * cmax * 3;     // q, sx, sy
-    off += sizeof(double) * 4 * cmax;                      // nz
-    off += sizeof(double) * 2 * cmax;                      // qmax, qpart
-    off += sizeof(double) * nd_max;                        // qsum
-    off += sizeof(unsigned long long) * cmax;
-    off += sizeof(int) * 2 * cmax;
-    off += sizeof(int) * (size_t)nd_max * cmax;           // segdone
-    off += sizeof(int) * nd_max;                           // perm
-    off += (cmax + 15) & ~15;
-    off = (off + 15) & ~size_t(15);
-    off += 8 + 8 + 48 + 8;
-    return (off + 15) & ~size_t(15);
-}
-
 }  // namespace
 
-int yg_launch_lv(yg_ensemble *e, const RunArgs &a, bool, cudaStream_t st)
+int yg_launch_lv(yg_ensemble *e, const RunArgs &a, cudaStream_t st)
 {
     const DevProblemHeader *hp = reinterpret_cast<const DevProblemHeader *>(e->h_problem.data());
     const bool two = e->cfg.n_levels == 2;
     const int nd_max = std::max(hp->lvl[0].n_data, two ? hp->lvl[1].n_data : 0);
-    // Default geometry (profiles/r01_lv_tuning.md): ONE persistent CTA per SM with up to 768 threads
-    // (6 warps per sub-partition saturate the FP64 pipe, and 768 threads leave 80 registers per thread:
-    // fewer spills in the owners' phases than the 64 of 1024 threads, +2 %).  Several smaller CTAs per SM
-    // finish at very different times because the FP64 issue arbiter is not fair between CTAs, which
-    // leaves SMs half empty towards the end.
-    int bps = e->cfg.blocks_per_sm > 0 ? e->cfg.blocks_per_sm : 1;
-    int threads = e->cfg.threads_per_block;
-    if (threads <= 0) {
-        const int64_t ctas = std::min<int64_t>((int64_t)e->sm_count * bps, a.n_chains);
-        const int64_t items = ((a.n_chains + ctas - 1) / ctas) * nd_max;
-        threads = (int)std::min<int64_t>((bps == 1 ? 768 : 1024) / bps, std::max<int64_t>(128, (items + 31) / 32 * 32));
-    }
+    const LvGeometry g = lv_geometry(a.problem_bytes, nd_max, a.n_chains, e->sm_count, e->cfg.blocks_per_sm,
+                                     e->cfg.threads_per_block);
+    const int threads = g.threads;
     if (threads % 32 || threads > 1024) {
         yg_set_error("threads_per_block must be a multiple of 32 and <= 1024 (got %d)", threads);
         return YG_ERR_INVALID;
     }
-    int64_t grid64 = std::min<int64_t>((int64_t)e->sm_count * bps, a.n_chains);
-    int grid = (int)std::max<int64_t>(grid64, 1);
-    // chains per chunk: the CTA's share, capped so that shared memory fits bps CTAs per SM
-    int64_t share = (a.n_chains + grid - 1) / grid;
-    const size_t budget = (size_t)(220 * 1024) / bps;
-    const size_t fixed = lv_smem_bytes(e, 0, nd_max);
-    const size_t per_chain = sizeof(double) * (SmemLayout::NDBL + 3 * nd_max + 6) + 4 * nd_max + 8 + 8 + 1;
-    int64_t cap = fixed < budget ? (int64_t)((budget - fixed) / per_chain) : 0;
-    if (cap < 1) {
-        yg_set_error("problem blob too large for shared memory (%zu bytes)", fixed);
+    if (g.cmax < 1) {
+        yg_set_error("problem blob too large for shared memory (%u bytes)", g.plan.total);
         return YG_ERR_UNSUPPORTED;
     }
-    const int cmax = (int)std::max<int64_t>(1, std::min<int64_t>(share, std::min<int64_t>(cap, 1024)));
-    const size_t smem = lv_smem_bytes(e, cmax, nd_max);
     RunArgs args = a;
     for (int l = 0; l < e->cfg.n_levels; l++) {
         args.lv_h[l] = hp->lvl[l].T / (double)hp->lvl[l].rk4_steps;
@@ -759,13 +703,13 @@ int yg_launch_lv(yg_ensemble *e, const RunArgs &a, bool, cudaStream_t st)
     auto kern = threads <= 512 ? (two ? lv_mh_kernel<true, 512> : lv_mh_kernel<false, 512>)
                 : threads <= 768 ? (two ? lv_mh_kernel<true, 768> : lv_mh_kernel<false, 768>)
                                  : (two ? lv_mh_kernel<true, 1024> : lv_mh_kernel<false, 1024>);
-    YG_CUDA_CHECK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    YG_CUDA_CHECK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)g.plan.total));
     const int seg_len = e->cfg.rk4_segment > 0 ? e->cfg.rk4_segment : 128;
-    kern<<<grid, threads, smem, st>>>(args, cmax, seg_len, e->cfg.early_reject_off == 0);
+    kern<<<g.grid, threads, g.plan.total, st>>>(args, g.plan, seg_len, e->cfg.early_reject_off == 0);
     YG_CUDA_CHECK(cudaGetLastError());
-    e->last_grid = grid;
+    e->last_grid = g.grid;
     e->last_block = threads;
-    e->last_smem = (int)smem;
+    e->last_smem = (int)g.plan.total;
     e->launches += 1;
     return YG_OK;
 }
