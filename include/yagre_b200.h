@@ -39,6 +39,8 @@
  *                            ESS idiom example_inference_lotkaVolterra_twoLevel.py:117-118,132
  *   yg_pooled_stats          (new) sufficient statistics for pooled moments / R-hat, summed over local
  *                            chains; the host all-reduces them across GPUs (NCCL, torch.distributed)
+ *   yg_pooled_samples_workspace_len / yg_pooled_samples
+ *                            (new) the same sufficient statistics from a stored sample buffer, any d <= 64
  *   yg_set_proposal_factor   (new) pooled proposal covariance; cf. AdaptiveMRWProposal.set_state
  *                            chain/adaptive.py:55-60
  *   yg_logpost               DensityInterface.evaluate_log statistics/interface.py:6-10
@@ -275,6 +277,18 @@ int yg_iat_ess(const double *samples_dev, int64_t n_samples, int32_t d, int64_t 
  * Every entry is a plain sum over chains, so an all-reduce(sum) pools GPUs. */
 int64_t yg_pooled_len(int32_t d);
 int yg_pooled_stats(yg_ensemble *e, double *out_dev, void *stream);
+
+/* The same vector from a stored sample buffer samples_dev[n_samples, d, n_chains] (yg_run's samples layout), for any
+ * 1 <= d <= YG_BIG_MAX_DIM: with mean_c the mean of chain c's stored samples and M2_c = sum_t (x_ct - mean_c)(x_ct - mean_c)':
+ *   [0] n_chains  [1] n_samples  [2] 0 (the caller fills in the accepts it wants pooled)
+ *   then sum_c mean_c [d], sum_c mean_c mean_c' [d*d], sum_c M2_c [d*d] (symmetric), sum_c diag(M2_c)/(n_samples-1) [d]
+ *   (0 for n_samples == 1).
+ * M2_c is formed from data shifted by each chain's first sample, so a large common offset costs no accuracy.  One read
+ * of the buffer; deterministic (fixed-order sums, bitwise repeatable).  workspace_dev holds at least
+ * yg_pooled_samples_workspace_len(d, n_chains) doubles.  Asynchronous on `stream`, no allocation, no synchronisation. */
+int64_t yg_pooled_samples_workspace_len(int32_t d, int64_t n_chains);   /* doubles; 0 if d < 1 or n_chains < 1 */
+int yg_pooled_samples(const double *samples_dev, int64_t n_samples, int32_t d, int64_t n_chains,
+                      double *workspace_dev, int64_t workspace_len, double *out_dev, void *stream);
 
 /* Per-chain mean and unbiased variance of each half of samples_dev[n_samples, d, n_chains]
  * -> half_mean_dev[2, d, n_chains], half_var_dev[2, d, n_chains] (split-R-hat inputs). */

@@ -95,6 +95,9 @@ SYMBOLS = {
     "yg_pooled_len": (C.c_int64, [C.c_int32]),
     "yg_pooled_stats": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p]),
     "yg_split_moments": (C.c_int, [C.c_void_p, C.c_int64, C.c_int32, C.c_int64, C.c_void_p, C.c_void_p, C.c_void_p]),
+    "yg_pooled_samples_workspace_len": (C.c_int64, [C.c_int32, C.c_int64]),
+    "yg_pooled_samples": (C.c_int, [C.c_void_p, C.c_int64, C.c_int32, C.c_int64, C.c_void_p, C.c_int64, C.c_void_p,
+                                    C.c_void_p]),
     "yg_fp64_peak": (C.c_int, [C.c_int32, C.c_double, C.POINTER(C.c_double)]),
     "yg_rk4_loop_rate": (C.c_int, [C.c_int32, C.c_double, C.POINTER(C.c_double)]),
     "yg_fp64_tensor_peak": (C.c_int, [C.c_int32, C.c_double, C.POINTER(C.c_double)]),

@@ -11,6 +11,7 @@ Same surface -- run(chainLength, initialState, verbose), .chain.trajectory, .dia
 import numpy as np
 import torch
 
+from .._lib import YG_MAX_DIM
 from ..ensemble import ChainEnsemble
 from .chain import Chain, Trajectory
 from .verbosity import VerbosityController
@@ -52,6 +53,8 @@ class MetropolisHastings:
                                        chain_offset=self._offset, adaptive=adaptive, aem=aem,
                                        welford=self._wants_moments(diagnostics), **(launch or {}))
         self._last = None
+        self._accepted = 0              # accepted transitions (all local chains) since the device counters were reset
+        self._lastRun = None            # (accepted, transitions per chain) of the last run()
         self._ran = False               # a run() has set the device state at least once
         self._diagnosticsCleared = True  # clear() was called since the last run(): restart the device accumulators
 
@@ -117,8 +120,9 @@ class MetropolisHastings:
         # (metropolisHastings.py:107-108,122-125), adaptation state persists, and the noise stream keeps
         # advancing (numpy's global generator there, the Philox step index here) -- two runs from the same
         # state are different realisations.
-        ens.set_state(np.ascontiguousarray(theta0), keep_diagnostics=self._ran and not self._diagnosticsCleared,
-                      keep_adaptation=self._ran)
+        keep = self._ran and not self._diagnosticsCleared
+        ens.set_state(np.ascontiguousarray(theta0), keep_diagnostics=keep, keep_adaptation=self._ran)
+        accepted0 = self._accepted if keep else 0
         self._ran, self._diagnosticsCleared = True, False
         self._verbosityController.on = bool(verbose)
         nTrans = chainLength - 1
@@ -147,6 +151,9 @@ class MetropolisHastings:
         if self._store:
             traj = torch.cat(pieces, dim=0) if len(pieces) > 1 else pieces[0]
             self._chain.set(Trajectory(traj, squeeze=(self._nGlobal == 1)))
+            if d > YG_MAX_DIM:          # the acceptance of the run pooled() pools (_stored_samples)
+                self._accepted = ens.counters()['accepted']
+                self._lastRun = (self._accepted - accepted0, nTrans)
         return self
 
     # ---- internals ----------------------------------------------------------------------------
@@ -163,16 +170,36 @@ class MetropolisHastings:
         self._last = st
         self._diagnostics.process_ensemble(stats)
 
+    def _stored_samples(self):
+        """(samples [length, d, nLocal], accepted, transitions per chain) of the last run(): the pooled path for
+        d > YG_MAX_DIM, where the device keeps no full second moment per chain."""
+        if not self._store or self._lastRun is None or not isinstance(self._chain.trajectory, Trajectory):
+            raise NotImplementedError(
+                f"pooled statistics at dim > {YG_MAX_DIM} are computed from the stored trajectory of the last run(): "
+                "build the chain with storeTrajectory = True (and a thin that keeps it affordable), then run()")
+        return (self._chain.trajectory.device_tensor,) + self._lastRun
+
     def pooled(self):
-        """Pooled moments and R-hat over ALL chains (all ranks): see yagre_mcmc_b200.parallel."""
+        """Pooled moments and R-hat over ALL chains (all ranks): see yagre_mcmc_b200.parallel.
+
+        dim <= 8: from the chains' Welford moments, i.e. every pre-transition state since clear().  dim > 8 (the
+        tensor path keeps a diagonal second moment only): from the trajectory of the LAST run() as stored, i.e. its
+        initial state and every thin-th state after it; the acceptance rate is that run's.  Needs storeTrajectory."""
+        if self._lowered.dim > YG_MAX_DIM:
+            from ..parallel import pooled_diagnostics_from_samples
+            return pooled_diagnostics_from_samples(*self._stored_samples())
         from ..parallel import pooled_diagnostics
         return pooled_diagnostics(self._ensemble)
 
     def pool_proposal_covariance(self, scale=None, eps=1e-8):
         """Optional pooled proposal covariance: replaces the proposal covariance of every chain (all ranks) by
-        scale * (covariance pooled over all chains since the diagnostics were last cleared + eps I), scale =
-        2.4^2 / d by default.  The idiom mirrors the reference's burn-in restart
-        (example_inference_linearModel_twoLevel.py:228,236): run a burn-in, pool, run again from
-        chain.trajectory[-1].  Returns the pooled moments with the new factor under 'prop_L'."""
+        scale * (pooled covariance + eps I), scale = 2.4^2 / d by default.  The covariance is pooled as pooled()
+        does: since clear() for dim <= 8, over the stored trajectory of the last run() for dim > 8 -- where a handle
+        built with a diagonal proposal factor switches to the dense kernel instance.  The idiom mirrors the
+        reference's burn-in restart (example_inference_linearModel_twoLevel.py:228,236): run a burn-in, pool, run
+        again from chain.trajectory[-1].  Returns the pooled moments with the new factor under 'prop_L'."""
+        if self._lowered.dim > YG_MAX_DIM:
+            from ..parallel import pooled_proposal_covariance_from_samples
+            return pooled_proposal_covariance_from_samples(self._ensemble, *self._stored_samples(), scale, eps)
         from ..parallel import pooled_proposal_covariance
         return pooled_proposal_covariance(self._ensemble, scale, eps)

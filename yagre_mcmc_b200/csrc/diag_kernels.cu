@@ -186,12 +186,259 @@ __global__ void __launch_bounds__(POOL_THREADS) pooled_stage1(const double *w_me
 
 __global__ void pooled_stage2(const double *partials, int n_part, int len, double *out)
 {
-    for (int q = threadIdx.x; q < len; q += blockDim.x) {
+    for (int q = blockIdx.x * blockDim.x + threadIdx.x; q < len; q += gridDim.x * blockDim.x) {
         double s = 0.0;
         if (q == 1) s = partials[q];
         else for (int b = 0; b < n_part; b++) s += partials[(int64_t)b * len + q];
         out[q] = s;
     }
+}
+
+// Pooled sufficient statistics of a stored sample buffer x[ns, d, nc] (yg_pooled_samples), for any d <= 64.
+//
+// Each warp takes groups of 4 consecutive chains; the K dimension of a symmetric rank-K update is the (sample, chain)
+// pairs of a group, 4 per m16n8k4 DMMA.  Lane (g = lane / 4, q = lane % 4) holds coordinates 8 m + g (m < G) of chain
+// 4 gi + q, which is at once its A fragment (rows 16 I + g and 16 I + 8 + g: values m = 2 I, 2 I + 1) and its B fragment
+// (column 8 J + g: value m = J) -- no shuffles, no shared-memory staging.  Only the output tiles (I, J) with
+// J <= 2 I + 1 are issued: those cover the lower triangle (20 of 32 at d = 64); the diagonal tiles' upper halves are
+// computed and dropped, the lower triangle is mirrored on write.
+//
+// Centred one-pass form: chain c is shifted by its first stored sample s_c, y = x - s_c, and
+//   M2_c = sum_t y y' - S1_c S1_c' / ns,  S1_c = sum_t y,  mean_c = s_c + S1_c / ns,
+// so the cancellation is relative to the chain's own spread, not to |x| (tests/pooled_samples_reference.py derives
+// the bound).  The correction is one more DMMA step per group with B = -S1 / ns.
+//
+// Pass 1 reads the buffer once and writes each chain's mean to the workspace; pass 2 re-reads the means (d doubles
+// per chain: 1 / ns of pass 1) for sum_c mean_c mean_c' with the same accumulator registers.  ns == 1 skips pass 1:
+// the means are row 0 of the buffer.  Per-CTA partial vectors, warps added in a fixed order, then pooled_stage2:
+// deterministic, no atomics.
+constexpr int PS_WARPS = 4;
+constexpr int PS_CHAINS_PER_CTA = 4 * PS_WARPS;
+constexpr int PS_MAX_PARTS = 4 * 148;       // at most 4 CTAs on each of the B200's 148 SMs
+
+YG_DEVFN void dmma_m16n8k4(double (&c)[4], double a0, double a1, double b0)
+{
+    asm volatile("mma.sync.aligned.m16n8k4.row.col.f64.f64.f64.f64 {%0,%1,%2,%3}, {%4,%5}, {%6}, {%0,%1,%2,%3};"
+                 : "+d"(c[0]), "+d"(c[1]), "+d"(c[2]), "+d"(c[3])
+                 : "d"(a0), "d"(a1), "d"(b0));
+}
+
+// acc[I][J] += A B over the 4 pairs of one k-step, lower tiles only.
+template <int G>
+YG_DEVFN void syrk_step(double (&acc)[(G + 1) / 2][G][4], const double (&a)[G], const double (&b)[G])
+{
+#pragma unroll
+    for (int I = 0; I < (G + 1) / 2; I++)
+#pragma unroll
+        for (int J = 0; J < G; J++)
+            if (J <= 2 * I + 1) dmma_m16n8k4(acc[I][J], a[2 * I], 2 * I + 1 < G ? a[2 * I + 1] : 0.0, b[J]);
+}
+
+// R[r * d + col] (col <= r) = sum over the CTA's warps, in warp order, of the accumulators.
+template <int G>
+YG_DEVFN void flush_lower(double (&acc)[(G + 1) / 2][G][4], double *R, int d, int smem_len)
+{
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, g = lane >> 2, q = lane & 3;
+    for (int w = 0; w < PS_WARPS; w++) {
+        if (warp == w) {
+#pragma unroll
+            for (int I = 0; I < (G + 1) / 2; I++)
+#pragma unroll
+                for (int J = 0; J < G; J++)
+                    if (J <= 2 * I + 1) {
+#pragma unroll
+                        for (int e = 0; e < 4; e++) {
+                            const int r = 16 * I + g + (e >= 2 ? 8 : 0), col = 8 * J + 2 * q + (e & 1);
+                            if (r < d && col <= r) {
+                                YG_CHK(r * d + col, smem_len);
+                                R[r * d + col] = (w == 0 ? 0.0 : R[r * d + col]) + acc[I][J][e];
+                            }
+                        }
+                    }
+        }
+        __syncthreads();
+    }
+}
+
+template <int G>
+__global__ void __launch_bounds__(PS_WARPS * 32) pooled_samples_kernel(const double *__restrict__ x, int64_t ns, int d,
+                                                                       int64_t nc, double *partials, int len,
+                                                                       double *means)
+{
+    constexpr int RB = (G + 1) / 2;
+    constexpr int U = G >= 8 ? 1 : 8 / G;          // samples per iteration: about 8 loads in flight per lane
+    constexpr int DP = 8 * G;
+    extern __shared__ double sm[];                  // R[d * d] | sum of means [warp][q][DP] | sum of variances, same
+    [[maybe_unused]] const int smem_len = d * d + 2 * PS_WARPS * 4 * DP;
+    const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5, g = lane >> 2, q = lane & 3;
+    double *R = sm;
+    const int slot = d * d + (warp * 4 + q) * DP;   // this lane's slots (coordinates 8 m + g of its chains)
+    const int vslot = slot + PS_WARPS * 4 * DP;
+#pragma unroll
+    for (int m = 0; m < G; m++) {
+        YG_CHK(vslot + 8 * m + g, smem_len);
+        sm[slot + 8 * m + g] = 0.0;
+        sm[vslot + 8 * m + g] = 0.0;
+    }
+    __syncthreads();
+    const int64_t n_groups = (nc + 3) / 4, tw = (int64_t)gridDim.x * PS_WARPS;
+    [[maybe_unused]] const int64_t x_len = ns * d * nc, m_len = (int64_t)d * nc;     // YG_CHK extents
+    double *part = partials + (int64_t)blockIdx.x * len;
+    [[maybe_unused]] const int part_len = gridDim.x * len;
+    const int o_mean = 3, o_mm = o_mean + d, o_m2 = o_mm + d * d, o_var = o_m2 + d * d;
+    double acc[RB][G][4];
+
+    if (ns > 1) {
+#pragma unroll
+        for (int I = 0; I < RB; I++)
+#pragma unroll
+            for (int J = 0; J < G; J++) acc[I][J][0] = acc[I][J][1] = acc[I][J][2] = acc[I][J][3] = 0.0;
+        const double inv_n = 1.0 / (double)ns;
+        for (int64_t gi = (int64_t)blockIdx.x * PS_WARPS + warp; gi < n_groups; gi += tw) {
+            const int64_t c = 4 * gi + q;
+            const bool ok = c < nc;
+            double s[G], S1[G], Q[G];
+#pragma unroll
+            for (int m = 0; m < G; m++) {
+                const int i = 8 * m + g;
+                if (ok && i < d) YG_CHK((int64_t)i * nc + c, x_len);
+                s[m] = (ok && i < d) ? __ldg(x + (int64_t)i * nc + c) : 0.0;
+                S1[m] = Q[m] = 0.0;
+            }
+            // software pipeline: the loads of iteration t + U are in flight during the DMMAs of iteration t
+            double xn[U][G];
+            auto load = [&](int64_t t0) {
+#pragma unroll
+                for (int u = 0; u < U; u++)
+#pragma unroll
+                    for (int m = 0; m < G; m++) {
+                        const int i = 8 * m + g;
+                        const int64_t idx = ((t0 + u) * d + i) * nc + c;
+                        const bool in = ok && i < d && t0 + u < ns;
+                        if (in) YG_CHK(idx, x_len);
+                        xn[u][m] = in ? __ldg(x + idx) : s[m];
+                    }
+            };
+            load(0);
+            for (int64_t t = 0; t < ns; t += U) {
+                double y[U][G];
+#pragma unroll
+                for (int u = 0; u < U; u++)
+#pragma unroll
+                    for (int m = 0; m < G; m++) y[u][m] = xn[u][m] - s[m];
+                load(t + U);
+#pragma unroll
+                for (int u = 0; u < U; u++) {
+#pragma unroll
+                    for (int m = 0; m < G; m++) {
+                        S1[m] += y[u][m];
+                        Q[m] = fma(y[u][m], y[u][m], Q[m]);
+                    }
+                    syrk_step<G>(acc, y[u], y[u]);
+                }
+            }
+            double nS[G];
+#pragma unroll
+            for (int m = 0; m < G; m++) nS[m] = -(S1[m] * inv_n);
+            syrk_step<G>(acc, S1, nS);                              // - sum_c S1_c S1_c' / ns
+#pragma unroll
+            for (int m = 0; m < G; m++) {
+                const int i = 8 * m + g;
+                if (ok && i < d) {
+                    YG_CHK((int64_t)i * nc + c, m_len);
+                    means[(int64_t)i * nc + c] = s[m] + S1[m] * inv_n;
+                    sm[vslot + 8 * m + g] += (Q[m] - S1[m] * (S1[m] * inv_n)) / (double)(ns - 1);
+                }
+            }
+        }
+        flush_lower<G>(acc, R, d, smem_len);
+    }
+    for (int k = tid; k < d * d; k += blockDim.x) {
+        const int r = max(k / d, k % d), col = min(k / d, k % d);
+        YG_CHK(r * d + col, smem_len);
+        YG_CHK((int64_t)blockIdx.x * len + o_m2 + k, part_len);
+        part[o_m2 + k] = ns > 1 ? R[r * d + col] : 0.0;
+    }
+    for (int i = tid; i < d; i += blockDim.x) {
+        double v = 0.0;
+        for (int w = 0; w < PS_WARPS * 4; w++) {
+            YG_CHK(d * d + PS_WARPS * 4 * DP + w * DP + i, smem_len);
+            v += sm[d * d + PS_WARPS * 4 * DP + w * DP + i];
+        }
+        YG_CHK((int64_t)blockIdx.x * len + o_var + i, part_len);
+        part[o_var + i] = v;
+    }
+    __syncthreads();                                    // R is reused below
+
+    // pass 2: sum_c mean_c mean_c' and sum_c mean_c
+    const double *mb = ns > 1 ? means : x;             // [d, nc]; for ns == 1 row 0 of the buffer
+#pragma unroll
+    for (int I = 0; I < RB; I++)
+#pragma unroll
+        for (int J = 0; J < G; J++) acc[I][J][0] = acc[I][J][1] = acc[I][J][2] = acc[I][J][3] = 0.0;
+    for (int64_t gi = (int64_t)blockIdx.x * PS_WARPS + warp; gi < n_groups; gi += tw) {
+        const int64_t c = 4 * gi + q;
+        const bool ok = c < nc;
+        double mv[G];
+#pragma unroll
+        for (int m = 0; m < G; m++) {
+            const int i = 8 * m + g;
+            if (ok && i < d) YG_CHK((int64_t)i * nc + c, m_len);
+            mv[m] = (ok && i < d) ? mb[(int64_t)i * nc + c] : 0.0;     // pass 1 of this thread wrote `means`
+            if (ok && i < d) sm[slot + 8 * m + g] += mv[m];
+        }
+        syrk_step<G>(acc, mv, mv);
+    }
+    flush_lower<G>(acc, R, d, smem_len);
+    for (int k = tid; k < d * d; k += blockDim.x) {
+        const int r = max(k / d, k % d), col = min(k / d, k % d);
+        YG_CHK(r * d + col, smem_len);
+        YG_CHK((int64_t)blockIdx.x * len + o_mm + k, part_len);
+        part[o_mm + k] = R[r * d + col];
+    }
+    for (int i = tid; i < d; i += blockDim.x) {
+        double v = 0.0;
+        for (int w = 0; w < PS_WARPS * 4; w++) {
+            YG_CHK(d * d + w * DP + i, smem_len);
+            v += sm[d * d + w * DP + i];
+        }
+        YG_CHK((int64_t)blockIdx.x * len + o_mean + i, part_len);
+        part[o_mean + i] = v;
+    }
+    if (tid == 0) {
+        YG_CHK((int64_t)blockIdx.x * len + 2, part_len);
+        int64_t chains = 0;
+        for (int w = 0; w < PS_WARPS; w++)
+            for (int64_t gi = (int64_t)blockIdx.x * PS_WARPS + w; gi < n_groups; gi += tw)
+                chains += min((int64_t)4, nc - 4 * gi);
+        part[0] = (double)chains;
+        part[1] = (double)ns;
+        part[2] = 0.0;
+    }
+}
+
+int64_t ps_parts_max(int64_t nc)
+{
+    return std::min<int64_t>(PS_MAX_PARTS, (nc + PS_CHAINS_PER_CTA - 1) / PS_CHAINS_PER_CTA);
+}
+
+template <int G>
+int launch_pooled_samples(const double *x, int64_t ns, int d, int64_t nc, double *ws, double *out, cudaStream_t st)
+{
+    const int len = (int)yg_pooled_len(d);
+    const size_t smem = sizeof(double) * ((size_t)d * d + 2 * PS_WARPS * 4 * 8 * G);     // <= 48 KiB at d = 64
+    int dev = 0, sms = 148, per_sm = 1;
+    YG_CUDA_CHECK(cudaGetDevice(&dev));
+    YG_CUDA_CHECK(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
+    YG_CUDA_CHECK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, pooled_samples_kernel<G>, PS_WARPS * 32, smem));
+    const int64_t parts_max = ps_parts_max(nc);
+    const int grid = (int)std::max<int64_t>(1, std::min<int64_t>(parts_max, (int64_t)sms * std::min(per_sm, 4)));
+    double *means = ws + parts_max * len;
+    pooled_samples_kernel<G><<<grid, PS_WARPS * 32, smem, st>>>(x, ns, d, nc, ws, len, means);
+    YG_CUDA_CHECK(cudaGetLastError());
+    pooled_stage2<<<(len + 127) / 128, 128, 0, st>>>(ws, grid, len, out);
+    YG_CUDA_CHECK(cudaGetLastError());
+    return YG_OK;
 }
 
 // FP64-pipe micro-benchmarks, 1024 resident threads/SM.  Variant 0: eight independent
@@ -316,6 +563,41 @@ int yg_pooled_impl(const double *w_mean, const double *w_m2, const unsigned long
     pooled_stage2<<<1, 128, 0, st>>>(partials, n_part, len, out_dev);
     YG_CUDA_CHECK(cudaGetLastError());
     return YG_OK;
+}
+
+extern "C" int64_t yg_pooled_samples_workspace_len(int32_t d, int64_t n_chains)
+{
+    if (d < 1 || n_chains < 1) return 0;
+    return ps_parts_max(n_chains) * yg_pooled_len(d) + (int64_t)d * n_chains;
+}
+
+extern "C" int yg_pooled_samples(const double *samples_dev, int64_t n_samples, int32_t d, int64_t n_chains,
+                                 double *workspace_dev, int64_t workspace_len, double *out_dev, void *stream)
+{
+    if (!samples_dev || !workspace_dev || !out_dev || n_samples < 1 || n_chains < 1 || d < 1) {
+        yg_set_error("yg_pooled_samples: invalid arguments");
+        return YG_ERR_INVALID;
+    }
+    if (d > YG_BIG_MAX_DIM) {
+        yg_set_error("yg_pooled_samples: dim %d exceeds %d", d, YG_BIG_MAX_DIM);
+        return YG_ERR_UNSUPPORTED;
+    }
+    if (workspace_len < yg_pooled_samples_workspace_len(d, n_chains)) {
+        yg_set_error("yg_pooled_samples: workspace of %lld doubles, %lld needed", (long long)workspace_len,
+                     (long long)yg_pooled_samples_workspace_len(d, n_chains));
+        return YG_ERR_INVALID;
+    }
+    cudaStream_t st = (cudaStream_t)stream;
+    switch ((d + 7) / 8) {
+    case 1: return launch_pooled_samples<1>(samples_dev, n_samples, d, n_chains, workspace_dev, out_dev, st);
+    case 2: return launch_pooled_samples<2>(samples_dev, n_samples, d, n_chains, workspace_dev, out_dev, st);
+    case 3: return launch_pooled_samples<3>(samples_dev, n_samples, d, n_chains, workspace_dev, out_dev, st);
+    case 4: return launch_pooled_samples<4>(samples_dev, n_samples, d, n_chains, workspace_dev, out_dev, st);
+    case 5: return launch_pooled_samples<5>(samples_dev, n_samples, d, n_chains, workspace_dev, out_dev, st);
+    case 6: return launch_pooled_samples<6>(samples_dev, n_samples, d, n_chains, workspace_dev, out_dev, st);
+    case 7: return launch_pooled_samples<7>(samples_dev, n_samples, d, n_chains, workspace_dev, out_dev, st);
+    default: return launch_pooled_samples<8>(samples_dev, n_samples, d, n_chains, workspace_dev, out_dev, st);
+    }
 }
 
 extern "C" int yg_fp64_peak(int32_t device, double ms, double *tflops_out)

@@ -4,6 +4,7 @@ PyTorch is plumbing only (device memory, streams); every computation happens in
 the hand-written sm_100a kernels behind the C-ABI.  Layout on the device is
 struct-of-arrays with the chain index fastest (theta[d, n], samples[n_out, d, n]).
 """
+import copy
 import ctypes as C
 
 import numpy as np
@@ -215,6 +216,27 @@ class ChainEnsemble:
             check(self.lib.yg_set_proposal_factor(self._h, Lh.ctypes.data_as(C.c_void_p), self._stream()))
         return self
 
+    def rebuild_proposal_factor(self, L):
+        """Replaces the proposal factor by re-issuing yg_set_problem with the problem's prop_L replaced by L (lower
+        triangular [d, d], positive diagonal).  Unlike set_proposal_factor it may switch the kind of factor: a
+        tensor-path handle built with a diagonal factor takes a dense one and runs the dense kernel instance from then
+        on.  The chains' state is kept (the target does not change).  Refused for pCN, whose factor is the prior's
+        (pcn.py:23-35)."""
+        if self.problem.proposal == 'pcn':
+            raise NotImplementedError("the proposal factor of a pCN chain is the prior's (pcn.py:23-35) and cannot be "
+                                      "replaced")
+        Lh = _f64(L)
+        if Lh.shape != (self.dim, self.dim):
+            raise ValueError(f"proposal factor must be [{self.dim}, {self.dim}], got {Lh.shape}")
+        if not np.all(np.isfinite(Lh)) or np.any(np.triu(Lh, 1) != 0.0) or not np.all(np.diag(Lh) > 0.0):
+            raise ValueError("proposal factor must be finite, lower triangular with a positive diagonal")
+        problem = copy.copy(self.problem)
+        problem.arrays = dict(self.problem.arrays, prop_L=Lh)
+        with torch.cuda.device(self.device):
+            check(self.lib.yg_set_problem(self._h, C.byref(problem.c_struct())))
+        self.problem = problem
+        return self
+
     def run(self, n_steps, thin=1, samples=True, accepted=False, logpost=False, inject=None, record=False,
             samples_out=None):
         """Runs n_steps transitions of every chain.
@@ -379,6 +401,24 @@ def split_moments(samples):
         check(lib.yg_split_moments(C.c_void_p(samples.data_ptr()), ns, d, n, C.c_void_p(hm.data_ptr()),
                                    C.c_void_p(hv.data_ptr()), st))
     return hm, hv
+
+
+def pooled_sample_stats(samples):
+    """samples: device tensor [n_samples, d, n_chains] float64 (yg_run's samples layout, d <= 64) -> device vector of
+    the pooled sufficient statistics (parallel.py's layout, yg_pooled_samples) over the stored samples of every chain.
+    Entry [2] (accepts) is 0.  Asynchronous on the current stream; the workspace is allocated here."""
+    lib = _lib.load()
+    if not (torch.is_tensor(samples) and samples.is_cuda and samples.dtype == torch.float64 and samples.dim() == 3):
+        raise ValueError("samples must be a float64 CUDA tensor [n_samples, d, n_chains]")
+    samples = samples.contiguous()
+    ns, d, n = samples.shape
+    ws = torch.empty(max(1, int(lib.yg_pooled_samples_workspace_len(d, n))), dtype=torch.float64, device=samples.device)
+    out = torch.empty(int(lib.yg_pooled_len(d)), dtype=torch.float64, device=samples.device)
+    with torch.cuda.device(samples.device):
+        st = C.c_void_p(torch.cuda.current_stream(samples.device).cuda_stream)
+        check(lib.yg_pooled_samples(C.c_void_p(samples.data_ptr()), ns, d, n, C.c_void_p(ws.data_ptr()), ws.numel(),
+                                    C.c_void_p(out.data_ptr()), st))
+    return out
 
 
 def fp64_peak_tflops(device=0, ms=20.0):

@@ -7,6 +7,8 @@ pinned against a numpy restatement in the tests, not against the reference.
 Layout of the statistics vector (yg_pooled_stats, length 3 + d + 2 d^2 + d):
   [0] chains  [1] samples per chain n  [2] sum accepts
   sum_c mean_c [d] | sum_c mean_c mean_c' [d,d] | sum_c M2_c [d,d] | sum_c var_c [d]
+yg_pooled_stats builds it from the chains' Welford moments (d <= 8); yg_pooled_samples builds the same vector from a
+stored sample buffer for any d <= 64 (the tensor path keeps a diagonal Welford M2 only).
 """
 import numpy as np
 import torch
@@ -76,6 +78,29 @@ def pooled_proposal_covariance(ensemble, scale=None, eps=1e-8):
     out = pooled_diagnostics(ensemble)
     L = proposal_factor_from_covariance(out['covariance'], scale, eps)
     ensemble.set_proposal_factor(L)
+    out['prop_L'] = L
+    return out
+
+
+def pooled_diagnostics_from_samples(samples, accepted, transitions):
+    """Pooled moments and R-hat over all ranks from THIS rank's stored samples [n_samples, d, n_chains] (a device
+    tensor in yg_run's samples layout, e.g. Trajectory.device_tensor; d <= 64).  accepted: accepted transitions summed
+    over this rank's chains; transitions: transitions per chain, the same on every rank.  The acceptance entry is
+    written as accepted n_samples / transitions before the all-reduce, so 'acceptance_rate' is the pooled accepted
+    transitions over the pooled transitions."""
+    from .ensemble import pooled_sample_stats
+    vec = pooled_sample_stats(samples)
+    vec[2] = float(accepted) * samples.shape[0] / transitions if transitions > 0 else 0.0
+    return moments_from_stats(all_reduce_stats(vec), samples.shape[1])
+
+
+def pooled_proposal_covariance_from_samples(ensemble, samples, accepted, transitions, scale=None, eps=1e-8):
+    """pooled_proposal_covariance from stored samples (pooled_diagnostics_from_samples): the factor
+    L = chol(scale (Sigma_pooled + eps I)) is installed with ensemble.rebuild_proposal_factor, so a tensor-path
+    ensemble built with a diagonal factor switches to the dense one.  Returns the moments dict with 'prop_L'."""
+    out = pooled_diagnostics_from_samples(samples, accepted, transitions)
+    L = proposal_factor_from_covariance(out['covariance'], scale, eps)
+    ensemble.rebuild_proposal_factor(L)
     out['prop_L'] = L
     return out
 
