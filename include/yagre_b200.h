@@ -75,7 +75,9 @@ extern "C" {
 #define YG_MAX_DATA_DIM 8
 /* YG_MODEL_LINEAR beyond those sizes runs on the FP64 tensor path (DMMA GEMM, linear_dmma_kernel.cu): MRW, pCN and
  * two-level delayed acceptance; diagonal measurement noise; diagonal or dense prior precision and proposal factor;
- * any number of data rows; no adaptive Metropolis / adaptive error model / third level / tempering;
+ * every combination up to YG_BIG_MAX_DIM x YG_BIG_MAX_DATA_DIM (an operand that does not fit shared memory -- level
+ * 1's G, then the dense factor -- is read from L2; rates measured on a B200 in profiles/streamed_operand.md);
+ * no adaptive Metropolis / adaptive error model / third level / tempering;
  * Welford M2 is then diagonal only ([d, n_chains] instead of [d, d, n_chains]). */
 #define YG_BIG_MAX_DIM 64
 #define YG_BIG_MAX_DATA_DIM 256

@@ -199,7 +199,7 @@ int build_big_blob(const yg_config &c, const yg_problem *pb, std::vector<char> &
         }
     const bool dense_L = !is_diagonal(pb->prop_L, d);
     const int kp = d <= 16 ? 16 : (d <= 32 ? 32 : 64), ks = kp + 4;
-    size_t tail_len = 0;
+    int np_l[2] = {0, 0};                 // operand rows per level, rounded up to 16
     bool dense_prior[2] = {false, false};
     std::vector<double> Rp[2];            // chol(prior precision)' of the levels with a dense prior
     for (int l = 0; l < nl; l++) {
@@ -245,16 +245,17 @@ int build_big_blob(const yg_config &c, const yg_problem *pb, std::vector<char> &
             for (int i = 0; i < d; i++)
                 for (int j = 0; j < d; j++) Rp[l][(size_t)i * d + j] = Lp[(size_t)j * d + i];
         }
-        const size_t rows = (size_t)L.data_dim + (dense_prior[l] ? d : 0);
-        const size_t np = (rows + 15) & ~size_t(15);
-        tail_len += np * ks + np + 2 * (size_t)kp;
+        np_l[l] = (L.data_dim + (dense_prior[l] ? d : 0) + 15) & ~15;
     }
-    tail_len += 2 * (size_t)kp + (dense_L ? (size_t)kp * ks : 0);
-    tail_len = (tail_len + 1) & ~size_t(1);
-    if (big_smem_plan((int)tail_len, ks, kp / 4, dense_L, false).warps < BIG_MIN_WARPS) {
-        yg_set_error("large linear model: %zu bytes of G / data do not fit the shared memory of one SM", sizeof(double) * tail_len);
+    // operands that leave too little shared memory for BIG_MIN_WARPS warps are read from this blob's global copy
+    // (smem_plan.h: big_tensor_plan); inside the envelope that always suffices, so the refusal is a safety check only
+    const BigTensorPlan plan = big_tensor_plan(np_l[0], np_l[1], kp / 4, dense_L, false);
+    if (plan.smem.warps < BIG_MIN_WARPS) {
+        yg_set_error("large linear model: %zu bytes of G / data do not fit the shared memory of one SM",
+                     sizeof(double) * (size_t)plan.resident);
         return YG_ERR_UNSUPPORTED;
     }
+    const size_t tail_len = (size_t)plan.tail;
     blob.assign(sizeof(DevBigHeader) + sizeof(double) * tail_len, 0);
     DevBigHeader *h = reinterpret_cast<DevBigHeader *>(blob.data());
     double *tail = reinterpret_cast<double *>(blob.data() + sizeof(DevBigHeader));
@@ -263,20 +264,29 @@ int build_big_blob(const yg_config &c, const yg_problem *pb, std::vector<char> &
     h->tail_len = (int32_t)tail_len;
     h->proposal = pb->proposal;
     h->dense_L = dense_L ? 1 : 0;
+    h->stream = plan.stream;
+    // every item in the staged prefix in the order below, except the streamed operands: those follow the prefix
+    size_t off = 0, soff = (size_t)plan.resident;
+    auto place = [&](const size_t n, const int bit) {
+        size_t &cur = (plan.stream & bit) ? soff : off;
+        const size_t at = cur;
+        cur += n;
+        return (int32_t)at;
+    };
     if (pb->proposal == YG_PROPOSAL_PCN) {
         const double t = 2.0 * pb->pcn_step;                      // pcn.py:30
         h->pcn_a = sqrt(1.0 - t);
         h->pcn_b = sqrt(t);
     }
-    size_t off = 0;
     for (int l = 0; l < nl; l++) {
         const yg_level &L = pb->level[l];
         BigLevel &B = h->lvl[l];
         const int rows = L.data_dim + (dense_prior[l] ? d : 0);
-        const int np = (rows + 15) & ~15;
+        const int np = np_l[l];
         B.n_data = L.n_data; B.data_dim = L.data_dim; B.np = np; B.n_rows = rows;
-        B.G_off = (int32_t)off;
-        B.bd_off = (int32_t)(off + (size_t)np * ks);
+        B.G_off = place((size_t)np * ks, l == 1 ? BIG_STREAM_G1 : 0);
+        B.bd_off = place((size_t)np, 0);
+        const size_t goff = (size_t)B.G_off;
         // sum_rows ||F - d_row||^2_P = sum_col n P_col (F_col - mean_col)^2 + sum_col P_col sum_rows (d - mean)^2;
         // sqrt(n P_col) is folded into row `col` of G and into b - mean
         double q_const = 0.0;
@@ -291,7 +301,7 @@ int build_big_blob(const yg_config &c, const yg_problem *pb, std::vector<char> &
             }
             const double prec = L.noise_prec[(size_t)r * L.data_dim + r];
             const double sw = sqrt((double)L.n_data * prec);
-            for (int k = 0; k < d; k++) tail[off + (size_t)r * ks + k] = sw * L.G[(size_t)r * d + k];
+            for (int k = 0; k < d; k++) tail[goff + (size_t)r * ks + k] = sw * L.G[(size_t)r * d + k];
             tail[B.bd_off + r] = sw * (L.b[r] - mean);
             q_const += prec * scatter;
         }
@@ -299,34 +309,29 @@ int build_big_blob(const yg_config &c, const yg_problem *pb, std::vector<char> &
             for (int r = 0; r < d; r++) {
                 double rm = 0.0;
                 for (int k = 0; k < d; k++) {
-                    tail[off + (size_t)(L.data_dim + r) * ks + k] = Rp[l][(size_t)r * d + k];
+                    tail[goff + (size_t)(L.data_dim + r) * ks + k] = Rp[l][(size_t)r * d + k];
                     rm += Rp[l][(size_t)r * d + k] * L.prior_mean[k];
                 }
                 tail[B.bd_off + L.data_dim + r] = -rm;
             }
         }
         B.q_const = q_const;
-        off += (size_t)np * ks + np;
-        B.pmean_off = (int32_t)off;
-        for (int k = 0; k < d; k++) tail[off + k] = L.prior_mean[k];
-        off += kp;
-        B.pprec_off = (int32_t)off;
+        B.pmean_off = place(kp, 0);
+        for (int k = 0; k < d; k++) tail[B.pmean_off + k] = L.prior_mean[k];
+        B.pprec_off = place(kp, 0);
         if (!dense_prior[l])
-            for (int k = 0; k < d; k++) tail[off + k] = L.prior_prec[(size_t)k * d + k];
-        off += kp;
+            for (int k = 0; k < d; k++) tail[B.pprec_off + k] = L.prior_prec[(size_t)k * d + k];
     }
     if (nl == 1) h->lvl[1] = h->lvl[0];
-    h->propL_off = (int32_t)off;
-    for (int k = 0; k < d; k++) tail[off + k] = pb->prop_L[(size_t)k * d + k];
-    off += kp;
-    h->pcn_mean_off = (int32_t)off;
+    h->propL_off = place(kp, 0);
+    for (int k = 0; k < d; k++) tail[h->propL_off + k] = pb->prop_L[(size_t)k * d + k];
+    h->pcn_mean_off = place(kp, 0);
     if (pb->proposal == YG_PROPOSAL_PCN && pb->pcn_mean)
-        for (int k = 0; k < d; k++) tail[off + k] = pb->pcn_mean[k];
-    off += kp;
-    h->Ld_off = (int32_t)off;
+        for (int k = 0; k < d; k++) tail[h->pcn_mean_off + k] = pb->pcn_mean[k];
+    h->Ld_off = place(dense_L ? (size_t)kp * ks : 0, BIG_STREAM_LD);
     if (dense_L)
         for (int r = 0; r < d; r++)
-            for (int k = 0; k <= r; k++) tail[off + (size_t)r * ks + k] = pb->prop_L[(size_t)r * d + k];
+            for (int k = 0; k <= r; k++) tail[h->Ld_off + (size_t)r * ks + k] = pb->prop_L[(size_t)r * d + k];
     return YG_OK;
 }
 

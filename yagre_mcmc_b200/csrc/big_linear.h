@@ -15,7 +15,9 @@ struct BigLevel {
 struct DevBigHeader {
     int32_t dim, kp, ks, n_levels;                  // kp in {16, 32, 64} >= dim; ks = kp + 4 (row stride of G)
     int32_t J, tail_len, propL_off, proposal;       // proposal: yg_proposal
-    int32_t pcn_mean_off, dense_L, Ld_off, _pad;    // dense_L: the proposal factor is a full lower triangle Ld[kp][ks]
+    int32_t pcn_mean_off, dense_L, Ld_off, stream;  // dense_L: the proposal factor is a full lower triangle Ld[kp][ks];
+                                                    // stream: BigStream bits (smem_plan.h) of the operands the step
+                                                    // kernel reads from this global copy instead of shared memory
     double pcn_a, pcn_b;                            // sqrt(1 - 2h), sqrt(2h)   (pcn.py:30-35)
     BigLevel lvl[2];
     // followed by double tail[tail_len]: per level
@@ -25,9 +27,12 @@ struct DevBigHeader {
     // A DENSE prior precision P = R'R (R = chol(P)') is folded into the same operands as d more rows:
     //   Gw[data_dim + r] = R_r,  bdw[data_dim + r] = -(R m)_r,  pprec = 0:  ||R (theta - m)||^2 = (theta - m)' P (theta - m).
     // then propL[kp] (diagonal of the factor), pcn_mean[kp] and, for a dense factor, Ld[kp][ks].  Padding is zero.
+    // When the plan streams operands (big_tensor_plan), the same items are laid out without the streamed ones up to
+    // the staged prefix of BigTensorPlan::resident doubles, and the streamed ones follow it, 32-byte aligned, level 1's
+    // G before Ld; the offsets above say where every item is.
     // sum_rows ||F - d_row||^2_P = sum_col w_col (F_col - mean_col)^2 + q_const.
 };
-static_assert(sizeof(DevBigHeader) % 16 == 0, "header must keep 16-byte alignment");
+static_assert(sizeof(DevBigHeader) % 32 == 0, "header must keep the tail on 32-byte sectors (streamed operands)");
 
 // Welford second moment of the large model is diagonal only (like the reference's
 // WelfordAccumulator, statistics/estimation.py:4-58): w_m2 is [d, n] when d > YG_MAX_DIM and the

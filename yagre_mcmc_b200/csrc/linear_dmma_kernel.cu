@@ -263,11 +263,169 @@ YG_DEVFN double logpost_tile(const SmemLevel &L, const int ks, const double (&a)
     return -0.5 * (q + L.q_const) + (-0.5 * quad_sum(pr));
 }
 
+// ---- streamed operands: A fragments read from the global copy of the blob (smem_plan.h: big_tensor_plan) -----------
+// The blob is constant during a launch, so the non-coherent read-only path is legal.  A lane reads 8 bytes and the four
+// t lanes of a row 32 contiguous bytes: whole sectors (every streamed operand starts on a 32-byte boundary of the tail).
+// Volatile for the reason lds_ordered is: the loads keep their place in the DMMA stream.
+YG_DEVFN double ldg_ordered(const double *p)
+{
+    double v;
+    asm volatile("ld.global.nc.f64 %0, [%1];" : "=d"(v) : "l"(p));
+    return v;
+}
+
+// k-steps of A fragments in flight ahead of the DMMA that consumes them, chosen from the sweep over 2, 4, 6 and 8 in
+// profiles/streamed_operand.md (B200, 1,000 W): two-level 64 x 256 at 65,536 chains ran at 2.00, 2.04, 2.01 and
+// 1.99e8 chain-steps/s.  At 4 the streamed two-level instances spill what the resident ones spill (72 B; 88 B in the
+// general instance) and the single-level one nothing; ptxas -v: at 6 the single-level instance spills 104 B, at 8 the
+// two-level ones 168 / 176 B.  YG_STREAM_DEPTH overrides it in the dev builds of that sweep.
+#ifndef YG_STREAM_DEPTH
+#define YG_STREAM_DEPTH 4
+#endif
+constexpr int STREAM_DEPTH = YG_STREAM_DEPTH;
+
+// Where a streamed operand lives, for the bounds-checked build: every index is checked against the tail.
+struct StreamTail {
+    const double *tail;
+    int len;
+    YG_DEVFN const double *at(const double *p) const
+    {
+        YG_CHK(p - tail, len);
+        return p;
+    }
+};
+
+// logpost_tile with G in global memory.  Same DMMAs in the same order on the same operands; the fragments of k-step
+// i + STREAM_DEPTH are requested before the DMMAs of k-step i, across the boundary of 32-row passes too.  A row block
+// that does not exist (after the last pass, or the second half of a trailing 16-row block) re-reads rows of the current
+// pass instead (addresses stay inside G, no branch splits the DMMA stream).
+template <int KQ, typename SIDE>
+YG_DEVFN double logpost_tile_streamed(const SmemLevel &L, const int ks, const double (&a)[KQ], const int g, const int t,
+                                      SIDE &&side, const StreamTail &st)
+{
+    constexpr int D = STREAM_DEPTH < KQ ? STREAM_DEPTH : KQ - 1;       // (only KQ = 16 runs it)
+    double qa = 0.0, qb = 0.0;
+    auto epilogue = [&](const int nb, const double c0, const double c1, const double c2, const double c3) {
+        const double b0 = L.bd[nb + g], b1 = L.bd[nb + 8 + g];
+        const double e0 = c0 + b0, e1 = c1 + b0, e2 = c2 + b1, e3 = c3 + b1;
+        qa = fma(e2, e2, fma(e0, e0, qa));
+        qb = fma(e3, e3, fma(e1, e1, qb));
+    };
+    // k-step i of the row block at nb: rows nb + g, nb + 8 + g, nb + h2 + g, nb + h2 + 8 + g (h2 = 16 for 32 rows)
+    auto fetch = [&](const int nb, const int h2, const int i, double (&f)[4]) {
+        const double *Gb = L.G + (size_t)(nb + g) * ks + t + 4 * i;
+        f[0] = ldg_ordered(st.at(Gb));
+        f[1] = ldg_ordered(st.at(Gb + (size_t)8 * ks));
+        f[2] = ldg_ordered(st.at(Gb + (size_t)h2 * ks));
+        f[3] = ldg_ordered(st.at(Gb + (size_t)(h2 + 8) * ks));
+    };
+    double F[D][4];                            // F[0]: the fragments of the k-step the DMMAs consume next
+#pragma unroll
+    for (int j = 0; j < D; j++) fetch(0, L.np >= 32 ? 16 : 0, j, F[j]);
+    int nb = 0, pass = 0;
+    for (; nb + 32 <= L.np; nb += 32) {
+        double c[2][4] = {{0.0, 0.0, 0.0, 0.0}, {0.0, 0.0, 0.0, 0.0}};
+        const int nn = nb + 32 < L.np ? nb + 32 : nb, hn = nn + 32 <= L.np ? 16 : 0;       // the next row block
+        side.begin(pass++);
+#pragma unroll
+        for (int i = 0; i < KQ; i++) {
+            double N[4];
+            if (i + D < KQ) fetch(nb, 16, i + D, N);
+            else fetch(nn, hn, i + D - KQ, N);
+#pragma unroll
+            for (int m = 0; m < 2; m++) dmma_m16n8k4(c[m][0], c[m][1], c[m][2], c[m][3], F[0][2 * m], F[0][2 * m + 1], a[i]);
+#pragma unroll
+            for (int j = 0; j < D; j++)
+#pragma unroll
+                for (int r = 0; r < 4; r++) F[j][r] = j + 1 < D ? F[j + 1][r] : N[r];
+            side.stage(i);
+        }
+#pragma unroll
+        for (int m = 0; m < 2; m++) epilogue(nb + 16 * m, c[m][0], c[m][1], c[m][2], c[m][3]);
+    }
+    for (; nb < L.np; nb += 16) {              // last 16 rows: its first D k-steps are already in F
+        double c0 = 0.0, c1 = 0.0, c2 = 0.0, c3 = 0.0;
+        side.begin(pass++);
+#pragma unroll
+        for (int i = 0; i < KQ; i++) {
+            double N[4] = {0.0, 0.0, 0.0, 0.0};
+            if (i + D < KQ) fetch(nb, 0, i + D, N);
+            dmma_m16n8k4(c0, c1, c2, c3, F[0][0], F[0][1], a[i]);
+#pragma unroll
+            for (int j = 0; j < D; j++)
+#pragma unroll
+                for (int r = 0; r < 4; r++) F[j][r] = j + 1 < D ? F[j + 1][r] : N[r];
+            side.stage(i);
+        }
+        epilogue(nb, c0, c1, c2, c3);
+    }
+#pragma unroll
+    for (int o = 4; o < 32; o <<= 1) {
+        qa += __shfl_xor_sync(0xffffffffu, qa, o);
+        qb += __shfl_xor_sync(0xffffffffu, qb, o);
+    }
+    const int src = (g << 2) | (g >> 1);
+    const double va = __shfl_sync(0xffffffffu, qa, src), vb = __shfl_sync(0xffffffffu, qb, src);
+    const double q = (g & 1) ? vb : va;
+    double pr = 0.0;
+#pragma unroll
+    for (int i = 0; i < KQ; i++) {
+        const double x = a[i] - L.pmean[4 * i + t];
+        pr = fma(L.pprec[4 * i + t] * x, x, pr);
+    }
+    return -0.5 * (q + L.q_const) + (-0.5 * quad_sum(pr));
+}
+
+// L z of the 8 chains with the dense factor in global memory: the DMMAs of propose's loop in its order, the fragments
+// STREAM_DEPTH k-steps ahead over the whole triangle; the accumulators go to the transpose tile as there.
+template <int KQ>
+YG_DEVFN void lz_streamed(const double *Ld, const int ks, const double (&zv)[KQ], const int g, const int t, double *scr,
+                          const StreamTail &st)
+{
+    constexpr int D = STREAM_DEPTH;
+    static_assert(D <= 8, "the next block of the triangle has at least 8 k-steps");
+    // fragments of k-step i of 16-row block b; block b has the 4 (b + 1) k-steps i with 4 i <= 16 b + 15
+    auto fetch = [&](const int b, const int i, double (&n)[2]) {
+        const double *p = Ld + (size_t)(16 * b + g) * ks + t + 4 * i;
+        n[0] = ldg_ordered(st.at(p));
+        n[1] = ldg_ordered(st.at(p + (size_t)8 * ks));
+    };
+    double F[D][2];
+#pragma unroll
+    for (int j = 0; j < D; j++) fetch(j < 4 ? 0 : 1, j < 4 ? j : j - 4, F[j]);
+#pragma unroll
+    for (int b = 0; b < KQ / 4; b++) {
+        double c0 = 0.0, c1 = 0.0, c2 = 0.0, c3 = 0.0;
+#pragma unroll
+        for (int i = 0; i <= 4 * b + 3; i++) {
+            double N[2] = {0.0, 0.0};
+            if (i + D <= 4 * b + 3) fetch(b, i + D, N);                         // k-step D ahead: this block
+            else if (b + 1 < KQ / 4) fetch(b + 1, i + D - 4 * (b + 1), N);       // or the next one
+            dmma_m16n8k4(c0, c1, c2, c3, F[0][0], F[0][1], zv[i]);
+#pragma unroll
+            for (int j = 0; j < D; j++) {
+                F[j][0] = j + 1 < D ? F[j + 1][0] : N[0];
+                F[j][1] = j + 1 < D ? F[j + 1][1] : N[1];
+            }
+        }
+        const int nb = 16 * b;
+        YG_CHK((2 * t + 1) * ks + nb + 8 + g, 8 * ks);
+        scr[(2 * t) * ks + nb + g] = c0;
+        scr[(2 * t + 1) * ks + nb + g] = c1;
+        scr[(2 * t) * ks + nb + 8 + g] = c2;
+        scr[(2 * t + 1) * ks + nb + 8 + g] = c3;
+    }
+}
+
 // FREE_NOISE = true: the production instance (Philox noise, diagonal proposal factor).  The injected / recorded noise
 // paths of the parity tests and the DENSE proposal factor (p = s + L z with L z as a second small GEMM) live in the
 // FREE_NOISE = false instance, which keeps the step loop of the production one small enough for the instruction cache
 // (stall reason no_instruction in profiles/r01_linear_dmma.md).
-template <int KQ, bool TWO_LEVEL, bool FREE_NOISE>
+// STREAMED = true: the operands of H.stream (smem_plan.h: big_tensor_plan: the target level's G, the dense factor) are
+// read from the global blob, and only the prefix of sp.blob bytes is staged.  Level 0's G -- J evaluations per
+// transition, under which the next proposal's noise is drawn -- always stays in shared memory.  Instantiated at KQ = 16
+// only, the one width whose blobs can outgrow shared memory.
+template <int KQ, bool TWO_LEVEL, bool FREE_NOISE, bool STREAMED = false>
 __global__ void __launch_bounds__(big_max_warps(KQ) * 32, 1) linear_dmma_mh_kernel(const RunArgs a, const DevBigHeader *gh,
                                                                           long long *tile_done, const BigSmemPlan sp)
 {
@@ -277,12 +435,14 @@ __global__ void __launch_bounds__(big_max_warps(KQ) * 32, 1) linear_dmma_mh_kern
     // ---- stage the problem into shared memory -------------------------------------------------
     const DevBigHeader H = *gh;
     const double *gtail = reinterpret_cast<const double *>(gh + 1);
-    for (int i = tid; i < H.tail_len; i += blockDim.x) smem[i] = gtail[i];
+    const int staged = STREAMED ? (int)(sp.blob / sizeof(double)) : H.tail_len;
+    for (int i = tid; i < staged; i += blockDim.x) smem[i] = gtail[i];
     __syncthreads();
+    const StreamTail stail{gtail, H.tail_len};
     SmemLevel Lv[2];
 #pragma unroll
     for (int l = 0; l < 2; l++) {
-        Lv[l].G = smem + H.lvl[l].G_off;
+        Lv[l].G = ((STREAMED && l == 1 && (H.stream & BIG_STREAM_G1)) ? gtail : smem) + H.lvl[l].G_off;
         Lv[l].bd = smem + H.lvl[l].bd_off;
         Lv[l].pmean = smem + H.lvl[l].pmean_off;
         Lv[l].pprec = smem + H.lvl[l].pprec_off;
@@ -299,7 +459,8 @@ __global__ void __launch_bounds__(big_max_warps(KQ) * 32, 1) linear_dmma_mh_kern
     constexpr int ZS = big_zs(KQ);
     const int n_warps = blockDim.x >> 5;
     const bool dense_L = !FREE_NOISE && H.dense_L;
-    const double *Ld = smem + H.Ld_off;            // [kp][ks] lower-triangular proposal factor (dense_L only)
+    const bool ld_streamed = STREAMED && (H.stream & BIG_STREAM_LD);
+    const double *Ld = (ld_streamed ? gtail : smem) + H.Ld_off;      // [kp][ks] lower-triangular factor (dense_L only)
     // the warp's tiles (smem_plan.h): state, transpose buffer of L z (dense_L only), Welford moments (wsm only), noise
     const int wsm = sp.wsm;
     unsigned char *wreg = reinterpret_cast<unsigned char *>(smem) + sp.blob + (size_t)warp * sp.stride;
@@ -454,7 +615,10 @@ __global__ void __launch_bounds__(big_max_warps(KQ) * 32, 1) linear_dmma_mh_kern
                     if (noise_mode == YG_NOISE_RECORD && live) a.z[((n * J + j) * d + k) * N + gr] = zv[i];
                 }
             }
-            if (dense_L) {
+            if (dense_L && ld_streamed) {
+                lz_streamed<KQ>(Ld, ks, zv, g, t, scr, stail);
+                __syncwarp();
+            } else if (dense_L) {
                 // L z of the 8 chains as a GEMM: L is the A operand (16 rows x 4 columns per mma), z -- already in the
                 // B-fragment layout -- the other one; only the k-steps of the lower triangle are issued.  The accumulators
                 // hold (L z)[row][chain]; the scratch tile transposes them back to "lane (g, t) holds chain g, row 4i + t".
@@ -560,7 +724,8 @@ __global__ void __launch_bounds__(big_max_warps(KQ) * 32, 1) linear_dmma_mh_kern
                 const bool moved = (((m >> (4 * g)) & 0xFu) != 0xFu) && live;
                 double lpf = 0.0;
                 if (__any_sync(0xffffffffu, moved)) {
-                    lpf = logpost_tile<KQ>(Lv[1], ks, s, g, t, SideNone{});
+                    lpf = (STREAMED && (H.stream & BIG_STREAM_G1)) ? logpost_tile_streamed<KQ>(Lv[1], ks, s, g, t, SideNone{}, stail)
+                                                                    : logpost_tile<KQ>(Lv[1], ks, s, g, t, SideNone{});
                     if (moved) {
                         if (t == 0) cnt_ev1++;
                         double u;
@@ -718,14 +883,27 @@ template <int KQ>
 int launch_t(yg_ensemble *e, const RunArgs &a, cudaStream_t st)
 {
     const DevBigHeader *hh = reinterpret_cast<const DevBigHeader *>(e->h_problem.data());
-    // warps per CTA: as many as the shared memory left by the problem blob holds (13 at d = 64 x 256, else 16; yg_set_problem
-    // refused a blob that leaves fewer than BIG_MIN_WARPS); Welford moments of the tiles in shared memory when that costs no
-    // warp (and FullDiagnostics asked for them at all)
-    const BigSmemPlan sp = big_smem_plan(hh->tail_len, hh->ks, KQ, hh->dense_L != 0, a.welford != 0);
+    // warps per CTA: as many as the shared memory left by the staged part of the problem blob holds (at most 12 for
+    // d > 32, else 16; yg_set_problem streamed operands until BIG_MIN_WARPS fit); Welford moments of the tiles in shared
+    // memory when that costs no warp (and FullDiagnostics asked for them at all)
+    const bool two = e->cfg.n_levels == 2;
+    const BigTensorPlan tp = big_tensor_plan(hh->lvl[0].np, two ? hh->lvl[1].np : 0, KQ, hh->dense_L != 0, a.welford != 0);
+    const BigSmemPlan sp = tp.smem;
     const bool free_noise = a.noise_mode == YG_NOISE_PHILOX && !hh->dense_L;      // the general instance also knows dense factors
-    auto kern = e->cfg.n_levels == 2
-                    ? (free_noise ? linear_dmma_mh_kernel<KQ, true, true> : linear_dmma_mh_kernel<KQ, true, false>)
-                    : (free_noise ? linear_dmma_mh_kernel<KQ, false, true> : linear_dmma_mh_kernel<KQ, false, false>);
+    decltype(&linear_dmma_mh_kernel<KQ, true, true>) kern;
+    if (tp.stream) {
+        // streamed instances: KQ = 16 only; one level streams only the dense factor (general instance)
+        if constexpr (KQ == 16) {
+            kern = two ? (free_noise ? linear_dmma_mh_kernel<KQ, true, true, true> : linear_dmma_mh_kernel<KQ, true, false, true>)
+                       : linear_dmma_mh_kernel<KQ, false, false, true>;
+        } else {
+            yg_set_error("large linear model: streamed operands need d > 32");
+            return YG_ERR_STATE;
+        }
+    } else {
+        kern = two ? (free_noise ? linear_dmma_mh_kernel<KQ, true, true> : linear_dmma_mh_kernel<KQ, true, false>)
+                   : (free_noise ? linear_dmma_mh_kernel<KQ, false, true> : linear_dmma_mh_kernel<KQ, false, false>);
+    }
     YG_CUDA_CHECK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sp.total));
     const int64_t tiles = (a.n_chains + 7) / 8;
     // persistent grid, every CTA resident (one per SM): the balanced schedule lets warps wait on one another
