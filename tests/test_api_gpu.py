@@ -6,6 +6,7 @@ import pytest
 import torch
 
 import bench_problems as bp
+from support import ensemble
 from yagre_mcmc_b200.parameter import ParameterVector, ScalarParameter
 from yagre_mcmc_b200.model import ForwardModel, LinearModelSolver, LotkaVolterraRK4Solver, LotkaVolterraParameter
 from yagre_mcmc_b200.statistics import (IIDCovarianceMatrix, DiagonalCovarianceMatrix, DenseCovarianceMatrix,
@@ -271,7 +272,6 @@ def _lv_hierarchy():
 def test_lv_two_level_inference_through_builders_equals_direct_backend():
     """The builder path lowers to exactly the arrays of bench_problems.lv_problem, so the trajectory
     equals the one of the bare C-ABI handle with the same seed (bitwise)."""
-    from yagre_mcmc_b200.ensemble import ChainEnsemble, LoweredProblem
     meta, arr, hier, lik, prior = _lv_hierarchy()
     nc, n = 96, 25
     th0 = bp.lv_initial_states(nc)
@@ -284,7 +284,7 @@ def test_lv_two_level_inference_through_builders_equals_direct_backend():
     mc.run(n, LotkaVolterraParameter(th0), verbose=False)
     states = np.asarray(mc.chain.trajectory)
     assert states.shape == (n, nc, 2) and np.array_equal(states[0], th0)
-    ens = ChainEnsemble(LoweredProblem(meta, arr), nc, seed=77)
+    ens = ensemble(meta, arr, nc, seed=77)
     ens.set_state(th0)
     direct = ens.run(n - 1, samples=True)["samples"].permute(0, 2, 1).cpu().numpy()
     assert np.array_equal(states[1:], direct)

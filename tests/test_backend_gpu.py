@@ -9,25 +9,9 @@ import torch
 import bench_problems as bp
 from diag_reference import check_replay_diagnostics, pre_states
 from golden_io import load, rel_err
+from support import LOGPOST_RTOL, ensemble, replay
 
 pytestmark = pytest.mark.gpu
-
-LOGPOST_RTOL = 1e-10      # north_star: 1e-10 relative on log-posterior
-
-
-def _ens(meta, arrays, nc, **kw):
-    from yagre_mcmc_b200.ensemble import ChainEnsemble, LoweredProblem
-    return ChainEnsemble(LoweredProblem(meta, arrays), nc, **kw)
-
-
-def _replay(meta, arrays, th0, out, adaptive=None):
-    """Runs the oracle on the noise the device recorded (chain-major layout)."""
-    from oracle import cport
-    z = out["z"].cpu().numpy().transpose(3, 0, 1, 2)
-    u_c = np.nan_to_num(out["u_c"].cpu().numpy().transpose(2, 0, 1), nan=0.5)
-    u_f = np.nan_to_num(out["u_f"].cpu().numpy().transpose(1, 0), nan=0.5)
-    return cport.run_injected(cport.Problem(meta, arrays, adaptive=adaptive), th0, z, u_c, u_f)     # meta['aem'] is honoured
-
 
 CASES = {
     "lv_two_level": lambda: (bp.lv_problem(True), lambda n: bp.lv_initial_states(n), 300, 30),
@@ -50,12 +34,12 @@ def test_philox_run_replayed_through_oracle(name):
     identical decisions and trajectories, log-posterior within tolerance."""
     (meta, arrays), init, nc, ns = CASES[name]()
     th0 = init(nc)
-    ens = _ens(meta, arrays, nc, seed=99)
+    ens = ensemble(meta, arrays, nc, seed=99)
     ens.set_state(th0)
     lp_init = ens.state()["logpost"].cpu().numpy()
     out = ens.run(ns, samples=True, accepted=True, logpost=True, record=True)
     torch.cuda.synchronize()
-    ref = _replay(meta, arrays, th0, out)
+    ref = replay(meta, arrays, th0, out)
     acc = out["accepted"].cpu().numpy().T
     assert int((acc != ref["accepted"]).sum()) == 0
     traj = out["samples"].cpu().numpy().transpose(2, 0, 1)
@@ -82,7 +66,7 @@ def test_device_philox_matches_host_philox_bitwise():
     from oracle import cport
     meta, arrays = bp.linear_problem(True)
     nc, ns, off = 64, 8, 1000
-    ens = _ens(meta, arrays, nc, seed=4242, chain_offset=off)
+    ens = ensemble(meta, arrays, nc, seed=4242, chain_offset=off)
     ens.set_state(np.zeros((nc, 2)))
     out = ens.run(ns, record=True, samples=False)
     u_c = out["u_c"].cpu().numpy()      # [ns, J, nc]
@@ -109,12 +93,12 @@ def test_sharding_invariance(two_level):
     meta, arrays = bp.lv_problem(two_level, Nc=32, Nf=96)
     nc, ns = 512, 12
     th0 = bp.lv_initial_states(nc)
-    full = _ens(meta, arrays, nc, seed=5)
+    full = ensemble(meta, arrays, nc, seed=5)
     full.set_state(th0)
     a = full.run(ns, samples=True)["samples"].cpu().numpy()
     parts = []
     for (lo, hi, geo) in [(0, 200, dict(blocks_per_sm=2, threads_per_block=256)), (200, nc, dict(rk4_segment=16))]:
-        e = _ens(meta, arrays, hi - lo, seed=5, chain_offset=lo, **geo)
+        e = ensemble(meta, arrays, hi - lo, seed=5, chain_offset=lo, **geo)
         e.set_state(th0[lo:hi])
         parts.append(e.run(ns, samples=True)["samples"].cpu().numpy())
     assert np.array_equal(a, np.concatenate(parts, axis=2))
@@ -133,15 +117,15 @@ def test_resume_is_bit_exact(case):
         (meta, arrays), th0 = bp.gauss2d_problem(), np.tile([-8.0, -7.0], (300, 1))
         adaptive = dict(idle=2, collection=5, eps=1e-4)
     nc = th0.shape[0]
-    a = _ens(meta, arrays, nc, seed=8, adaptive=adaptive)
+    a = ensemble(meta, arrays, nc, seed=8, adaptive=adaptive)
     a.set_state(th0)
     ref = a.run(20, samples=True)["samples"].cpu().numpy()
     ref_state = a.state()
-    b = _ens(meta, arrays, nc, seed=8, adaptive=adaptive)
+    b = ensemble(meta, arrays, nc, seed=8, adaptive=adaptive)
     b.set_state(th0)
     first = b.run(8, samples=True)["samples"].cpu().numpy()
     saved = b.state()
-    c = _ens(meta, arrays, nc, seed=8, adaptive=adaptive)
+    c = ensemble(meta, arrays, nc, seed=8, adaptive=adaptive)
     c.load_state(saved)
     second = c.run(12, samples=True)["samples"].cpu().numpy()
     assert np.array_equal(ref, np.concatenate([first, second], axis=0))
@@ -157,19 +141,19 @@ def test_checkpoint_files_and_trajectory_dump(tmp_path):
     meta, arrays = bp.lv_problem(True, Nc=16, Nf=64)
     nc = 200
     th0 = bp.lv_initial_states(nc)
-    a = _ens(meta, arrays, nc, seed=3, chain_offset=1000)
+    a = ensemble(meta, arrays, nc, seed=3, chain_offset=1000)
     a.set_state(th0)
     ref = a.run(30, samples=True)["samples"]
-    b = _ens(meta, arrays, nc, seed=3, chain_offset=1000)
+    b = ensemble(meta, arrays, nc, seed=3, chain_offset=1000)
     b.set_state(th0)
     first = b.run(10, samples=True)["samples"]
     ck = io.save_checkpoint(str(tmp_path / "ck"), b, extra=dict(note="after 10"))
-    c = _ens(meta, arrays, nc, seed=3, chain_offset=1000)
+    c = ensemble(meta, arrays, nc, seed=3, chain_offset=1000)
     head = io.load_checkpoint(ck, c)
     assert head["step_index"] == 10 and head["extra"]["note"] == "after 10"
     second = c.run(20, samples=True)["samples"]
     assert torch.equal(torch.cat([first, second]), ref)
-    wrong = _ens(meta, arrays, nc, seed=4, chain_offset=1000)
+    wrong = ensemble(meta, arrays, nc, seed=4, chain_offset=1000)
     with pytest.raises(ValueError, match="seed"):
         io.load_checkpoint(ck, wrong)
     f = io.save_trajectory(str(tmp_path / "traj"), ref, thin=1, chain_offset=1000, meta=dict(model="lv"))
@@ -185,11 +169,11 @@ def test_load_state_rejects_misshapen_arrays():
     here is at least as large as that copy, so nothing reads out of bounds whatever the check does)."""
     meta, arrays = bp.linear_problem(True)
     nc = 64
-    a = _ens(meta, arrays, nc, seed=8)
+    a = ensemble(meta, arrays, nc, seed=8)
     a.set_state(np.zeros((nc, 2)))
     a.run(5, samples=False)
     st = a.state()
-    b = _ens(meta, arrays, nc, seed=8)
+    b = ensemble(meta, arrays, nc, seed=8)
     for theta in (st["theta"].t().contiguous(), torch.zeros(3, nc, dtype=torch.float64, device=st["theta"].device)):
         with pytest.raises(ValueError, match="theta"):
             b.load_state(dict(st, theta=theta))
@@ -207,7 +191,7 @@ def test_failed_set_problem_leaves_the_handle_unchanged():
     from yagre_mcmc_b200.ensemble import LoweredProblem
     meta, arrays = bp.big_linear_problem(2, 16, 1)
     nc = 64
-    ens = _ens(meta, arrays, nc, seed=12)
+    ens = ensemble(meta, arrays, nc, seed=12)
     pts = np.random.default_rng(0).standard_normal((8, 2))
     before = ens.logpost(0, pts)
     small_meta, small_arrays = bp.linear_problem(False)
@@ -224,10 +208,10 @@ def test_thinning_and_outputs():
     meta, arrays = bp.lv_problem(True, Nc=16, Nf=64)
     nc = 200
     th0 = bp.lv_initial_states(nc)
-    a = _ens(meta, arrays, nc, seed=3)
+    a = ensemble(meta, arrays, nc, seed=3)
     a.set_state(th0)
     full = a.run(20, samples=True, logpost=True)
-    b = _ens(meta, arrays, nc, seed=3)
+    b = ensemble(meta, arrays, nc, seed=3)
     b.set_state(th0)
     thin = b.run(20, thin=5, samples=True, logpost=True)
     assert torch.equal(full["samples"][4::5], thin["samples"])
@@ -240,7 +224,7 @@ def test_thinning_and_outputs():
 def test_error_paths_follow_reference_exception_types():
     from yagre_mcmc_b200.ensemble import ChainEnsemble, LoweredProblem
     meta, arrays = bp.linear_problem(True)
-    e = ChainEnsemble(LoweredProblem(meta, arrays), 16)
+    e = ensemble(meta, arrays, 16)
     with pytest.raises(RuntimeError):                      # run before set_state
         e.run(3)
     with pytest.raises(ValueError):
@@ -259,7 +243,7 @@ def test_pcn_posterior_moments_match_mrw():
     nc = 8192
     out = []
     for meta, arrays in (bp.lv_pcn_problem(), bp.lv_problem(False)):
-        ens = _ens(meta, arrays, nc, seed=31)
+        ens = ensemble(meta, arrays, nc, seed=31)
         ens.set_state(bp.lv_initial_states(nc))
         ens.run(300, samples=False)
         th = ens.state()["theta"].cpu().numpy()
@@ -276,7 +260,7 @@ def test_big_linear_posterior_moments_and_diagnostics():
     nc, d = 4096, 64
     meta, arrays = bp.big_linear_problem(d, 256, 1)
     mean, cov = bp.linear_gaussian_posterior(arrays, 0)
-    ens = _ens(meta, arrays, nc, seed=41)
+    ens = ensemble(meta, arrays, nc, seed=41)
     ens.set_state(np.tile(mean, (nc, 1)))
     ens.run(1500, samples=False)
     out = ens.run(40, thin=40, samples=True, accepted=True)
@@ -294,15 +278,15 @@ def test_big_linear_posterior_moments_and_diagnostics():
         ens.pooled_stats()
     # sizes beyond the kernel, or features it does not have, are refused loudly
     with pytest.raises(NotImplementedError):
-        _ens(*bp.big_linear_problem(65, 64, 1), 16)
+        ensemble(*bp.big_linear_problem(65, 64, 1), 16)
     dense = dict(arrays)                            # round 2: a dense proposal factor runs (4 warps per SM at this size)
     dense["prop_L"] = 0.02 * np.linalg.cholesky(np.eye(d) + 0.01)
-    e2 = _ens(meta, dense, 64, seed=1)
+    e2 = ensemble(meta, dense, 64, seed=1)
     e2.set_state(np.tile(mean, (64, 1)))
     e2.run(20, samples=False)
     assert e2.counters()["transitions"] == 64 * 20 and e2.last_launch()["block"] == 4 * 32
     with pytest.raises(NotImplementedError):        # per-chain adaptation would need a d x d factor per chain
-        _ens(meta, arrays, 16, adaptive=dict(idle=1, collection=2))
+        ensemble(meta, arrays, 16, adaptive=dict(idle=1, collection=2))
 
 
 def test_logpost_matches_oracle():
@@ -312,7 +296,7 @@ def test_logpost_matches_oracle():
                                 (bp.linear_problem(True), rng.standard_normal((64, 2)) * 2),
                                 (bp.big_linear_problem(32, 96, 2, two_level=True), rng.standard_normal((64, 32))),
                                 (bp.gauss2d_problem(), rng.standard_normal((64, 2)) * 3)]:
-        ens = _ens(meta, arrays, 4)
+        ens = ensemble(meta, arrays, 4)
         pb = cport.Problem(meta, arrays)
         for lvl in range(meta["levels"]):
             got = ens.logpost(lvl, pts).cpu().numpy()
@@ -324,7 +308,7 @@ def test_nonfinite_forward_output_is_rejected():
     """RK4 blows up for extreme parameters: forward output -> +inf, logL -> -inf, proposal rejected
     by the unchanged acceptance rule (policy of the oracle's solver plugin)."""
     meta, arrays = bp.lv_problem(True, Nc=8, Nf=16)
-    ens = _ens(meta, arrays, 32)
+    ens = ensemble(meta, arrays, 32)
     lp = ens.logpost(0, np.tile([6.0, 6.0], (32, 1))).cpu().numpy()
     assert np.all(np.isneginf(lp))
 
@@ -335,7 +319,7 @@ def test_nonfinite_forward_output_is_rejected():
 
 def _aem_run(meta, a, **kw):
     nc, ns = a["u_f"].shape
-    ens = _ens(meta, a, nc, aem=meta["aem"], **kw)
+    ens = ensemble(meta, a, nc, aem=meta["aem"], **kw)
     ens.set_state(a["theta0"])
     inj = dict(z=np.ascontiguousarray(np.transpose(a["z"], (1, 2, 3, 0))),
                u_c=np.ascontiguousarray(np.transpose(a["u_c"], (1, 2, 0))),
@@ -371,10 +355,10 @@ def test_adaptive_error_model_philox_replay_and_resume():
     meta = dict(meta, aem=dict(min_data=8, heuristic=True))
     nc, ns = 500, 300
     th0 = np.zeros((nc, 2))
-    ens = _ens(meta, arrays, nc, seed=77, aem=meta["aem"])
+    ens = ensemble(meta, arrays, nc, seed=77, aem=meta["aem"])
     ens.set_state(th0)
     out = ens.run(ns, samples=True, accepted=True, record=True)
-    ref = _replay(meta, arrays, th0, out)
+    ref = replay(meta, arrays, th0, out)
     acc = out["accepted"].cpu().numpy().T
     assert int((acc != ref["accepted"]).sum()) == 0
     assert rel_err(out["samples"].cpu().numpy().transpose(2, 0, 1), ref["traj"][:, 1:]).max() <= 1e-12
@@ -383,22 +367,22 @@ def test_adaptive_error_model_philox_replay_and_resume():
     np.testing.assert_allclose(st["aem_mean"].cpu().numpy().T, ref["aem_mean"], rtol=1e-9, atol=1e-13)
     assert ens.counters()["coarse_evals"] == int(ref["aem_model_evals"].sum())
     # the error model lifts the fine acceptance rate well above the plain two-level chain's (SURVEY 8f: 0.04 -> 0.35)
-    plain = _ens(bp.linear_problem(True)[0], arrays, nc, seed=77)
+    plain = ensemble(bp.linear_problem(True)[0], arrays, nc, seed=77)
     plain.set_state(th0)
     plain.run(ns, samples=False)
     assert acc[:, 150:].mean() > 2.0 * plain.counters()["accepted"] / (nc * ns)
     # resume: 300 = 120 + save/load + 180, bit exact (cache and error model are part of the state)
-    b = _ens(meta, arrays, nc, seed=77, aem=meta["aem"])
+    b = ensemble(meta, arrays, nc, seed=77, aem=meta["aem"])
     b.set_state(th0)
     first = b.run(120, samples=True)["samples"]
-    c = _ens(meta, arrays, nc, seed=77, aem=meta["aem"])
+    c = ensemble(meta, arrays, nc, seed=77, aem=meta["aem"])
     c.load_state(b.state())
     second = c.run(180, samples=True)["samples"]
     assert torch.equal(torch.cat([first, second]), out["samples"])
     with pytest.raises(ValueError):
-        _ens(meta, arrays, 8, aem=dict(min_data=1))
+        ensemble(meta, arrays, 8, aem=dict(min_data=1))
     with pytest.raises(NotImplementedError):
-        _ens(bp.lv_problem(True)[0], bp.lv_problem(True)[1], 8, aem=dict(min_data=5))
+        ensemble(bp.lv_problem(True)[0], bp.lv_problem(True)[1], 8, aem=dict(min_data=5))
 
 
 # ------------------------------------------------------------------------------------------
@@ -459,7 +443,7 @@ def test_split_moments_and_pooled_stats_match_numpy():
     from yagre_mcmc_b200.parallel import moments_from_stats, split_rhat
     meta, arrays = bp.gauss2d_problem()
     nc, ns = 1000, 400
-    ens = _ens(meta, arrays, nc, seed=2)
+    ens = ensemble(meta, arrays, nc, seed=2)
     ens.set_state(np.tile(bp.GAUSS2D_MEAN, (nc, 1)))
     out = ens.run(ns, samples=True, accepted=True)
     s = out["samples"]
@@ -504,10 +488,10 @@ def test_adaptive_metropolis_matches_oracle_recurrence():
     ad = dict(idle=10, collection=30, eps=1e-4, refresh=3)
     nc, ns = 256, 150
     th0 = np.tile([-3.0, 4.0], (nc, 1))
-    ens = _ens(meta, arrays, nc, seed=21, adaptive=ad)
+    ens = ensemble(meta, arrays, nc, seed=21, adaptive=ad)
     ens.set_state(th0)
     out = ens.run(ns, samples=True, accepted=True, logpost=True, record=True)
-    ref = _replay(meta, arrays, th0, out, adaptive=ad)
+    ref = replay(meta, arrays, th0, out, adaptive=ad)
     acc = out["accepted"].cpu().numpy().T
     # the adapted factor goes through sqrt / divisions whose rounding may differ in the last ulp
     # between nvcc and gcc: decisions may flip only at ties; trajectories agree to 1e-9 otherwise
@@ -524,7 +508,7 @@ def test_adaptive_metropolis_moments_and_acceptance():
     from yagre_mcmc_b200.parallel import moments_from_stats
     meta, arrays = _am_problem()
     nc, ns = 2048, 6000
-    ens = _ens(meta, arrays, nc, seed=19, adaptive=dict(idle=100, collection=500, eps=1e-4))
+    ens = ensemble(meta, arrays, nc, seed=19, adaptive=dict(idle=100, collection=500, eps=1e-4))
     ens.set_state(np.tile([-3.0, 4.0], (nc, 1)))
     ens.run(1500, samples=False)                          # burn-in + adaptation
     s = ens.run(ns, samples=True, accepted=True)
@@ -550,7 +534,7 @@ def test_c5_full_size_properties():
     the fine screen (reference test/test_mlda.py:94-130)."""
     nc, ns = 65536, 40
     meta, arrays = bp.lv_problem(True)
-    ens = _ens(meta, arrays, nc, seed=11)
+    ens = ensemble(meta, arrays, nc, seed=11)
     th0 = bp.lv_initial_states(nc)
     ens.set_state(th0)
     out = ens.run(ns, samples=True, accepted=True)
@@ -574,7 +558,7 @@ def test_c5_full_size_properties():
     assert torch.equal(moved, acc.bool())
 
     meta2, arrays2 = bp.lv_problem(True, Nc=96, Nf=96)
-    ens2 = _ens(meta2, arrays2, 8192, seed=12)
+    ens2 = ensemble(meta2, arrays2, 8192, seed=12)
     ens2.set_state(bp.lv_initial_states(8192))
     ens2.run(30, samples=False)
     c2 = ens2.counters()
@@ -592,7 +576,7 @@ def test_lv_posterior_moments_match_long_reference_runs(two_level):
     meta_r, ref = load("lv_long_twoLevel" if two_level else "lv_long_singleLevel")
     nc = 65536
     meta, arrays = bp.lv_problem(two_level)
-    ens = _ens(meta, arrays, nc, seed=2024)
+    ens = ensemble(meta, arrays, nc, seed=2024)
     ens.set_state(bp.lv_initial_states(nc))
     ens.run(150 if two_level else 400, samples=False)          # burn-in (IAT 4.3 / 17)
     out = ens.run(60, samples=True, thin=20)
@@ -613,7 +597,7 @@ def test_lv_forward_through_logpost_matches_reference_solver():
     computed from the reference solver's forward output (DOP853, tests/golden/lv_forward.npz)."""
     _, a = load("lv_forward")
     meta, arrays = bp.lv_problem(True)
-    ens = _ens(meta, arrays, len(a["thetas"]), seed=1)
+    ens = ensemble(meta, arrays, len(a["thetas"]), seed=1)
     lp = ens.logpost(1, a["thetas"]).cpu().numpy()
     for i, th in enumerate(a["thetas"]):
         r = a["ref_forward"][i] - arrays["L1_data"]
@@ -643,7 +627,7 @@ def test_warp_specialised_small_ensemble_kernel_is_bit_identical(case):
     for nc in (1, 333):
         res = []
         for record in (False, True):
-            ens = _ens(meta, arrays, nc, seed=77, adaptive=am)
+            ens = ensemble(meta, arrays, nc, seed=77, adaptive=am)
             ens.set_state(init(nc))
             o1 = ens.run(120, samples=True, accepted=True, logpost=True, thin=3, record=record)
             o2 = ens.run(37, samples=True, accepted=True, record=record)          # continues (step index, Welford)
@@ -667,7 +651,7 @@ def test_pooled_proposal_covariance():
     from yagre_mcmc_b200.parallel import pooled_proposal_covariance
     nc = 4096
     meta, arrays = bp.gauss2d_problem()
-    ens = _ens(meta, arrays, nc, seed=31)
+    ens = ensemble(meta, arrays, nc, seed=31)
     ens.set_state(np.tile([1.0, 1.5], (nc, 1)))
     ens.run(3000, samples=False)
     c0 = ens.counters()
@@ -684,7 +668,7 @@ def test_pooled_proposal_covariance():
     rate1 = (c1["accepted"] - c0["accepted"]) / (c1["transitions"] - c0["transitions"])
     assert 0.28 < rate1 < 0.42 and abs(rate1 - 0.35) < abs(rate0 - 0.35) + 0.02     # 2-D optimal scaling: ~0.35
     # the same call on an adaptive ensemble restarts every chain's factor from the pooled one
-    ens_a = _ens(meta, arrays, 256, seed=32, adaptive=dict(idle=10 ** 9, collection=10 ** 9, refresh=1, eps=1e-4))
+    ens_a = ensemble(meta, arrays, 256, seed=32, adaptive=dict(idle=10 ** 9, collection=10 ** 9, refresh=1, eps=1e-4))
     ens_a.set_state(np.tile([1.0, 1.5], (256, 1)))
     ens_a.run(10, samples=False)
     ens_a.set_proposal_factor(want)
@@ -696,7 +680,7 @@ def test_pooled_proposal_covariance():
     with pytest.raises((ValueError, RuntimeError)):
         ens.set_proposal_factor(np.array([[1.0, 0.0], [0.0, -1.0]]))
     metap, arraysp = bp.lv_pcn_problem()
-    ens_p = _ens(metap, arraysp, 64, seed=33)
+    ens_p = ensemble(metap, arraysp, 64, seed=33)
     ens_p.set_state(bp.lv_initial_states(64))
     with pytest.raises((NotImplementedError, RuntimeError)):
         ens_p.set_proposal_factor(np.eye(2))
@@ -705,7 +689,7 @@ def test_pooled_proposal_covariance():
 def test_c4_single_level_full_size():
     nc, ns = 65536, 10
     meta, arrays = bp.lv_problem(False)
-    ens = _ens(meta, arrays, nc, seed=13)
+    ens = ensemble(meta, arrays, nc, seed=13)
     ens.set_state(bp.lv_initial_states(nc))
     out = ens.run(ns, samples=True, accepted=True)
     c = ens.counters()
@@ -724,7 +708,7 @@ def test_c3_linear_posterior_moments():
     mean, cov = bp.linear_posterior('f')
     se = np.sqrt(np.diag(cov) / nc)
     meta, arrays = bp.linear_problem(False)
-    ens = _ens(meta, arrays, nc, seed=17)
+    ens = ensemble(meta, arrays, nc, seed=17)
     ens.set_state(np.zeros((nc, 2)))
     ens.run(5000, samples=False)
     th = ens.state()["theta"].cpu().numpy()
@@ -732,7 +716,7 @@ def test_c3_linear_posterior_moments():
     np.testing.assert_allclose(np.cov(th), cov, rtol=0.06, atol=2e-3)
 
     meta, arrays = bp.linear_problem(True)
-    ens = _ens(meta, arrays, nc, seed=17)
+    ens = ensemble(meta, arrays, nc, seed=17)
     ens.set_state(np.zeros((nc, 2)))
     ens.run(30000, samples=False)
     s = ens.run(2000, thin=500, samples=True)["samples"].cpu().numpy()    # [4, d, nc]
@@ -746,7 +730,7 @@ def test_c3_linear_posterior_moments():
 def test_c2_gaussian_target_moments():
     nc = 4096
     meta, arrays = bp.gauss2d_problem()
-    ens = _ens(meta, arrays, nc, seed=23)
+    ens = ensemble(meta, arrays, nc, seed=23)
     ens.set_state(np.tile([-8.0, -7.0], (nc, 1)))
     ens.run(1000, samples=False)
     s = ens.run(500, thin=10, samples=True)["samples"].cpu().numpy()
@@ -769,10 +753,10 @@ def test_lv_edge_shapes_against_oracle(shape):
     nc = 1 if shape == "one_chain" else 97
     meta, arrays = bp.lv_problem(True, **({"Nc": 16, "Nf": 48} | kw))
     th0 = bp.lv_initial_states(nc)
-    ens = _ens(meta, arrays, nc, seed=3)
+    ens = ensemble(meta, arrays, nc, seed=3)
     ens.set_state(th0)
     out = ens.run(15, samples=True, accepted=True, logpost=True, record=True)
-    ref = _replay(meta, arrays, th0, out)
+    ref = replay(meta, arrays, th0, out)
     assert int((out["accepted"].cpu().numpy().T != ref["accepted"]).sum()) == 0
     assert rel_err(out["samples"].cpu().numpy().transpose(2, 0, 1), ref["traj"][:, 1:]).max() <= 1e-12
     lp = out["logpost"].cpu().numpy().transpose(2, 0, 1)
@@ -784,10 +768,10 @@ def test_zero_steps_and_repeated_short_runs():
     meta, arrays = bp.lv_problem(True, Nc=16, Nf=48)
     nc = 130
     th0 = bp.lv_initial_states(nc)
-    a = _ens(meta, arrays, nc, seed=9)
+    a = ensemble(meta, arrays, nc, seed=9)
     a.set_state(th0)
     ref = a.run(12, samples=True)["samples"]
-    b = _ens(meta, arrays, nc, seed=9)
+    b = ensemble(meta, arrays, nc, seed=9)
     b.set_state(th0)
     assert b.run(0, samples=True)["samples"].shape[0] == 0
     parts = [b.run(1, samples=True)["samples"] for _ in range(12)]
@@ -800,7 +784,7 @@ def test_c5_full_ensemble_on_one_gpu():
     CTA chunk boundaries (each CTA walks its 3,543 chains in chunks of <= 1,024)."""
     nc = 524288
     meta, arrays = bp.lv_problem(True)
-    ens = _ens(meta, arrays, nc, seed=21)
+    ens = ensemble(meta, arrays, nc, seed=21)
     th0 = bp.lv_initial_states(nc)
     ens.set_state(th0)
     out = ens.run(4, samples=True, accepted=True)
@@ -811,6 +795,6 @@ def test_c5_full_ensemble_on_one_gpu():
     moved = (out["samples"][0] != torch.as_tensor(th0.T, device="cuda")).any(dim=0)
     assert torch.equal(moved, acc[0].bool())
     # chain-offset keying: chains [1000, 1100) of the big run equal a 100-chain handle with chain_offset 1000
-    sub = _ens(meta, arrays, 100, seed=21, chain_offset=1000)
+    sub = ensemble(meta, arrays, 100, seed=21, chain_offset=1000)
     sub.set_state(th0[1000:1100])
     assert torch.equal(sub.run(4, samples=True)["samples"], out["samples"][:, :, 1000:1100])

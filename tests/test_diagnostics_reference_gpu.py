@@ -11,144 +11,23 @@ import pytest
 import torch
 
 import bench_problems as bp
-from diag_reference import check_pooled, check_welford, pre_states, welford_reference, welford_tolerance
+from diag_reference import welford_reference, welford_tolerance
 from golden_io import load
+from support import check_case, lv_tempered, three_level_gauss
 
 pytestmark = pytest.mark.gpu
-
-
-def _ens(meta, arrays, nc, **kw):
-    from yagre_mcmc_b200.ensemble import ChainEnsemble, LoweredProblem
-    return ChainEnsemble(LoweredProblem(meta, arrays), nc, **kw)
-
-
-def _replay(meta, arrays, th0, out, adaptive=None):
-    from oracle import cport
-    z = out["z"].cpu().numpy().transpose(3, 0, 1, 2)
-    u_c = np.nan_to_num(out["u_c"].cpu().numpy().transpose(2, 0, 1), nan=0.5)
-    u_f = np.nan_to_num(out["u_f"].cpu().numpy().transpose(1, 0), nan=0.5)
-    return cport.run_injected(cport.Problem(meta, arrays, adaptive=adaptive), th0, z, u_c, u_f)
-
-
-def _drive(meta, arrays, th0, plan, record, kw):
-    """Runs plan on a handle: ("run", k) | ("restart", theta) = set_state(theta, keep_diagnostics=True) |
-    ("reload",) = state() loaded into a fresh handle.  Returns the last handle and, per run, its outputs, the state it
-    started from, the restart state before it (or None) and the index of the handle that ran it."""
-    nc = th0.shape[0]
-    ens = _ens(meta, arrays, nc, **kw)
-    ens.set_state(th0)
-    runs, x, restart, handle = [], np.asarray(th0, dtype=np.float64), None, 0
-    for op in plan:
-        if op[0] == "run":
-            out = ens.run(op[1], samples=True, accepted=True, logpost=True, record=record)
-            runs.append(dict(out=out, start=x, restart=restart, handle=handle, launch=ens.last_launch()))
-            x, restart = out["samples"][-1].t().cpu().numpy(), None
-        elif op[0] == "restart":
-            ens.set_state(op[1], keep_diagnostics=True)
-            x = restart = np.asarray(op[1], dtype=np.float64)
-        else:
-            st = ens.state()
-            ens.close()
-            ens = _ens(meta, arrays, nc, **kw)
-            ens.load_state(st)
-            handle += 1
-    torch.cuda.synchronize()
-    return ens, runs
-
-
-def _expected_counts(meta, arrays, runs, adaptive, nc):
-    """Counters of the last handle and the per-chain accept / coarse-accept counts since the reset, from the oracle's
-    replay of every run's recorded noise (its evaluation totals include one initial evaluation per chain per level)."""
-    lv = meta["levels"]
-    want = dict(transitions=0, accepted=0, coarse_evals=0, mid_evals=0, fine_evals=0, coarse_accepted=0)
-    n_acc, c_acc = np.zeros(nc, dtype=np.int64), np.zeros(nc, dtype=np.int64)
-    last = runs[-1]["handle"]
-    for r in runs:
-        ref = _replay(meta, arrays, r["start"], r["out"], adaptive)
-        acc = r["out"]["accepted"].cpu().numpy().T
-        assert np.array_equal(acc, ref["accepted"])
-        n_acc += ref["accepted"].sum(axis=1, dtype=np.int64)
-        c_acc += ref["coarse_accepted"]
-        if r["handle"] != last:
-            continue
-        ev = [int(v) - nc for v in ref["n_evals"]]
-        want["transitions"] += acc.size
-        want["accepted"] += int(ref["accepted"].sum())
-        want["coarse_accepted"] += int(ref["coarse_accepted"].sum())
-        if meta.get("aem"):
-            want["coarse_evals"] += int(ref["aem_model_evals"].sum())
-            want["fine_evals"] += ev[1]
-        elif lv == 1:
-            want["fine_evals"] += ev[0]
-        elif lv == 2:
-            want["coarse_evals"] += ev[0]
-            want["fine_evals"] += ev[1]
-        else:
-            want["coarse_evals"] += ev[0]
-            want["mid_evals"] += ev[1]
-            want["fine_evals"] += ev[2]
-    return want, n_acc, c_acc
-
-
-def _state_np(st):
-    return {k: v.cpu().numpy() for k, v in st.items() if torch.is_tensor(v)}
-
-
-def check_case(meta, arrays, th0, plan, seed=1, adaptive=None, aem=None, ws=None, smem=None, label="", **kw):
-    """The whole check of one case (see the module docstring).  ws: the Philox run must (True) or must not (False)
-    run the warp-specialised kernel; smem: the tensor path's expected dynamic shared memory of every launch."""
-    nc = th0.shape[0]
-    kw = dict(kw, seed=seed, adaptive=adaptive, aem=aem)
-    rec_ens, rec = _drive(meta, arrays, th0, plan, True, kw)
-    ens, free = _drive(meta, arrays, th0, plan, False, kw)
-    # 1. production instances == recording instances, bit for bit
-    for a, b in zip(rec, free):
-        for k in ("samples", "accepted", "logpost"):
-            assert torch.equal(a["out"][k], b["out"][k]), (label, k)
-        if ws is not None:
-            assert a["launch"]["block"] != 64 and (b["launch"]["block"] == 64) == ws, (label, a["launch"], b["launch"])
-        if smem is not None:
-            assert a["launch"]["smem"] == b["launch"]["smem"] == smem, (label, a["launch"], b["launch"], smem)
-    st_rec, st = rec_ens.state(), ens.state()
-    for k, v in st.items():
-        assert (torch.equal(v, st_rec[k]) if torch.is_tensor(v) else v == st_rec[k]), (label, k)
-    c = ens.counters()
-    assert c == rec_ens.counters(), label
-    # 2. Welford moments against the long-double reference of the pre-transition states
-    pre = pre_states(th0, [r["out"]["samples"].cpu().numpy() for r in rec], [r["restart"] for r in rec])
-    s = _state_np(st)
-    check_welford(s["w_mean"], s["w_m2"], c["welford_n"], pre, label)
-    # 3. counts: the accept flags, the oracle replay, the counters
-    flags = sum(r["out"]["accepted"].to(torch.int64).sum(dim=0) for r in rec).cpu().numpy()
-    want, n_acc, c_acc = _expected_counts(meta, arrays, rec, adaptive, nc)
-    assert np.array_equal(s["n_accept"], flags) and np.array_equal(s["n_accept"], n_acc), label
-    got = {k: c[k] for k in want}
-    assert got == want, (label, got, want)
-    if meta["levels"] == 1:
-        assert c["coarse_accepted"] == 0 and not c_acc.any(), label
-    # 4. pooled statistics (d <= 8)
-    if meta["dim"] <= 8:
-        check_pooled(ens.pooled_stats().cpu().numpy(), s, c["welford_n"], pre, label)
-    rec_ens.close()
-    ens.close()
-    return c
 
 
 # ------------------------------------------------------------------------------------------
 # the LV kernel
 # ------------------------------------------------------------------------------------------
-def _lv_tempered():
-    meta, arrays = bp.lv_problem(True)
-    return meta, dict(arrays, L0_tempering=np.array(0.4))
-
-
 LV_CASES = {
     # name: (problem, chains, plan, adaptive)
     "headline": (lambda: bp.lv_problem(True), 65536, [("run", 3)], None),
     "single_level": (lambda: bp.lv_problem(False), 3000, [("run", 6)], None),
     "adaptive_coarse": (lambda: bp.lv_problem(True), 700, [("run", 8)], dict(idle=1, collection=3, eps=1e-6, refresh=2)),
     "pcn": (lambda: bp.lv_pcn_problem(), 1000, [("run", 8)], None),
-    "tempered_level0": (_lv_tempered, 500, [("run", 6)], None),
+    "tempered_level0": (lv_tempered, 500, [("run", 6)], None),
     "300_design_points": (lambda: bp.lv_problem(True, n_data=300, Nc=4, Nf=12, prop_var=2e-4), 97, [("run", 6)], None),
     "one_chain": (lambda: bp.lv_problem(True, Nc=16, Nf=48), 1, [("run", 25)], None),
     "whole_c5_ensemble": (lambda: bp.lv_problem(True), 524288, [("run", 2)], None),
@@ -191,12 +70,6 @@ def test_one_chain_per_thread_kernel_diagnostics_every_capacity(k):
     check_case(meta, arrays, th0, [("run", 12)], seed=5 + k, ws=d <= 2, label=f"d={d} data_dim={dd} two={two} nc={nc}")
 
 
-def _three_level_gauss():
-    _, a = load("mlda3_gauss2d")
-    arrays = {k: a[k] for k in a if k.startswith(("L0_", "L1_", "L2_")) or k == "prop_L"}
-    return dict(model="gauss", dim=2, levels=3, J=6, eq="exact"), arrays
-
-
 def _fixture_problem(name):
     meta, a = load(name)
     return meta, {k: v for k, v in a.items() if k.startswith(("L0_", "L1_", "L2_")) or k == "prop_L"}
@@ -208,7 +81,7 @@ def _gauss2d_start(n):
 
 GENERIC_CASES = {
     # name: (problem, initial states, chains, plan, adaptive, warp-specialised Philox run)
-    "three_level": (_three_level_gauss, _gauss2d_start, 33, [("run", 40)], None, True),
+    "three_level": (three_level_gauss, _gauss2d_start, 33, [("run", 40)], None, True),
     "single_level_adaptive": (bp.gauss2d_problem, _gauss2d_start, 4097, [("run", 30)],
                               dict(idle=3, collection=8, refresh=2, eps=1e-4), True),
     "coarse_adaptive": (lambda: bp.linear_problem(True), lambda n: np.zeros((n, 2)), 1000, [("run", 20)],

@@ -12,7 +12,8 @@ import pytest
 
 import bench_problems as bp
 import logpost_reference as R
-from golden_io import load
+from support import (SCHEDULES, TENSOR, dense_noise_linear, dense_prior_tensor, fixture, lv_tempered,
+                     qconst_tensor, schedule_noise)
 
 from oracle import cport
 
@@ -26,54 +27,6 @@ def _err(got, ref):
     return np.abs(np.asarray(got, dtype=np.longdouble) - ref).astype(np.float64)
 
 
-def _fixture(name):
-    meta, a = load(name)
-    return meta, {k: v for k, v in a.items() if k.startswith(("L0_", "L1_", "L2_")) or k in ("prop_L", "pcn_mean")}
-
-
-def _lv_tempered():
-    meta, arrays = bp.lv_problem(True)
-    return meta, dict(arrays, L0_tempering=np.array(0.4))
-
-
-def _dense_noise_linear():
-    meta, arrays = bp.big_linear_problem(5, 4, 3, two_level=False, seed=12)
-    A = np.random.default_rng(3).standard_normal((4, 4))
-    return meta, dict(arrays, L0_noise_prec=A @ A.T + 4 * np.eye(4), L0_prior_mean=np.full(5, 0.7))
-
-
-def _dense_prior_tensor():
-    rng = np.random.default_rng(11)
-    d, dd = 24, 40
-    meta, arrays = bp.big_linear_problem(d, dd, 2)
-    A = rng.standard_normal((d, d))
-    prec = np.linalg.inv(1.5 * (A @ A.T / d + 0.5 * np.eye(d)))
-    return meta, dict(arrays, L0_prior_prec=0.5 * (prec + prec.T), L0_prior_mean=0.1 * rng.standard_normal(d))
-
-
-def _qconst_tensor():
-    """Misfit dominated by q_const: 2,000 data rows scattered (sd 30) about the model, far beyond the noise (0.05)."""
-    meta, arrays = bp.big_linear_problem(23, 45, 1, seed=5)
-    rng = np.random.default_rng(6)
-    data = arrays["L0_data"][0] + 30.0 * rng.standard_normal((2000, 45))
-    return meta, dict(arrays, L0_data=data)
-
-
-def _near_zero_tensor():
-    """|lp| about 1e-4: noise and prior precisions of 1e-6."""
-    meta, arrays = bp.big_linear_problem(9, 1, 3, seed=8)
-    return meta, dict(arrays, L0_noise_prec=np.full((1, 1), 1e-6), L0_prior_prec=1e-6 * np.eye(9))
-
-
-def _tensor_4_warps():
-    """d = 64, two levels of 176 and 192 rows: the blob (206,208 bytes) and four warps' tiles take 232,320 bytes, within
-    the 227 KiB of one block."""
-    meta, arrays = bp.big_linear_problem(64, 192, 1, two_level=True, J=2, seed=9)
-    r = slice(0, 176)
-    return meta, dict(arrays, L0_data=arrays["L0_data"][:, r], L0_G=arrays["L0_G"][r], L0_b=arrays["L0_b"][r],
-                      L0_noise_prec=arrays["L0_noise_prec"][r, r])
-
-
 def _theta(meta, n, seed, scale=0.3):
     if meta["model"] == "lv":
         return bp.lv_initial_states(n, seed=seed) + np.random.default_rng(seed).uniform(-1, 1, (n, 2)) * 0.5
@@ -82,15 +35,15 @@ def _theta(meta, n, seed, scale=0.3):
 
 GENERIC = {
     "gauss2d": bp.gauss2d_problem,
-    "gauss1d_isclose": lambda: _fixture("mrw_gauss1d"),
-    "gauss3_levels": lambda: _fixture("mlda3_gauss2d"),
+    "gauss1d_isclose": lambda: fixture("mrw_gauss1d"),
+    "gauss3_levels": lambda: fixture("mlda3_gauss2d"),
     "linear_c3": lambda: bp.linear_problem(True),
-    "linear_tempered": lambda: _fixture("mlda_linear_tempered"),
-    "linear_dense_noise_d5": _dense_noise_linear,
+    "linear_tempered": lambda: fixture("mlda_linear_tempered"),
+    "linear_dense_noise_d5": dense_noise_linear,
     "linear_d8_dd8": lambda: bp.big_linear_problem(8, 8, 5, two_level=True, seed=4),
     "lv_two_level": lambda: bp.lv_problem(True),
     "lv_single_level": lambda: bp.lv_problem(False),
-    "lv_tempered": _lv_tempered,
+    "lv_tempered": lv_tempered,
     "lv_pcn": bp.lv_pcn_problem,
     "lv_one_design_point": lambda: bp.lv_problem(True, n_data=1),
     "lv_300_design_points": lambda: bp.lv_problem(True, n_data=300, Nc=16, Nf=48),
@@ -159,18 +112,6 @@ def tensor_logpost_f64(arrays, theta, qc_f32=False, R_f32=False, qc_rel=0.0):
     return -0.5 * (q + q_const) + (-0.5 * (pprec * x * x).sum(axis=1))
 
 
-TENSOR = {
-    "9x1": lambda: bp.big_linear_problem(9, 1, 3, seed=2),
-    "23x45": lambda: bp.big_linear_problem(23, 45, 3),
-    "32x96_two_level": lambda: bp.big_linear_problem(32, 96, 2, two_level=True, J=3),
-    "64x256": lambda: bp.big_linear_problem(64, 256, 1),
-    "dense_prior": _dense_prior_tensor,
-    "q_const_dominated": _qconst_tensor,
-    "near_zero": _near_zero_tensor,
-    "64x176_192_four_warps": _tensor_4_warps,
-}
-
-
 @pytest.mark.parametrize("name", sorted(TENSOR))
 def test_tensor_path_formulation_within_its_bound(name):
     """The folded formulation in double (and the oracle's textbook one) within the tensor-path bound."""
@@ -210,7 +151,7 @@ def _wrong_cases():
     lin_meta, lin = bp.big_linear_problem(5, 4, 3, two_level=False, seed=12)
     lin = dict(lin, L0_prior_mean=np.full(5, 0.7))
     lv_meta, lv = bp.lv_problem(True)
-    tmeta, tarr = _fixture("mlda_linear_tempered")
+    tmeta, tarr = fixture("mlda_linear_tempered")
     tl = [l for l in range(2) if f"L{l}_tempering" in tarr][0]
     other = 1 - tl
     moved = {k: v for k, v in tarr.items() if k != f"L{tl}_tempering"}
@@ -218,8 +159,8 @@ def _wrong_cases():
     h_meta, h_arr = bp.lv_problem(False)
     a, g, T, N = h_arr["L0_lv"]
     h_wrong = dict(h_arr, L0_lv=np.array([a, g, T * N / (N + 1), N]))
-    qc_meta, qc = _qconst_tensor()
-    dp_meta, dp = _dense_prior_tensor()
+    qc_meta, qc = qconst_tensor()
+    dp_meta, dp = dense_prior_tensor()
     return {
         # name: (meta, arrays, level, wrong evaluation (theta -> lp), path)
         "last_data_row_dropped": (lin_meta, lin, 0, lambda th: _oracle(
@@ -266,34 +207,6 @@ def test_c_rk4_covers_a_fresh_measurement():
 # ------------------------------------------------------------------------------------------------------------------
 # the schedules force the chosen decisions in the oracle
 # ------------------------------------------------------------------------------------------------------------------
-def _pcn_linear():
-    meta, arrays = bp.linear_problem(False)
-    return dict(meta, proposal="pcn", pcn_step=0.05), dict(arrays, pcn_mean=np.array([0.3, -0.2]))
-
-
-SCHEDULES = {
-    # name: (problem, chains, steps, initial states)
-    "lv_two_level": (lambda: bp.lv_problem(True), 24, 4, lambda n: bp.lv_initial_states(n)),
-    "lv_single_level": (lambda: bp.lv_problem(False), 24, 5, lambda n: bp.lv_initial_states(n)),
-    "lv_pcn": (bp.lv_pcn_problem, 24, 5, lambda n: bp.lv_initial_states(n)),
-    "gauss_single_level": (bp.gauss2d_problem, 64, 10, lambda n: np.tile([-1.0, 2.0], (n, 1))),
-    "gauss_isclose_1d": (lambda: _fixture("mrw_gauss1d"), 64, 10, lambda n: np.full((n, 1), -1.0)),
-    "linear_pcn": (_pcn_linear, 64, 10, lambda n: np.zeros((n, 2))),
-    "linear_two_level": (lambda: bp.linear_problem(True), 64, 8, lambda n: np.zeros((n, 2))),
-    "linear_tempered_surrogate": (lambda: _fixture("mlda_linear_tempered"), 64, 8, lambda n: np.zeros((n, 2))),
-    "gauss_three_level": (lambda: _fixture("mlda3_gauss2d"), 64, 8, lambda n: np.tile([0.5, 1.0], (n, 1))),
-    "tensor_single_level": (lambda: bp.big_linear_problem(23, 45, 3), 32, 6,
-                            lambda n: 0.01 * np.random.default_rng(2).standard_normal((n, 23))),
-    "tensor_two_level": (lambda: bp.big_linear_problem(32, 96, 2, two_level=True, J=3), 32, 5,
-                         lambda n: 0.01 * np.random.default_rng(3).standard_normal((n, 32))),
-}
-
-
-def schedule_noise(meta, nc, ns, seed):
-    J = int(meta["J"]) if int(meta["levels"]) >= 2 else 1
-    return np.random.default_rng(seed).standard_normal((nc, ns, J, int(meta["dim"])))
-
-
 @pytest.mark.parametrize("eta", [0.0, 1e-7, 1e-3])
 @pytest.mark.parametrize("name", sorted(SCHEDULES))
 def test_forced_schedule_reproduced_by_the_oracle(name, eta):

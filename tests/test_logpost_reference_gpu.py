@@ -15,55 +15,9 @@ import torch
 
 import bench_problems as bp
 import logpost_reference as R
-from test_logpost_reference_cpu import (SCHEDULES, TENSOR, _dense_noise_linear, _fixture, _lv_tempered,
-                                        schedule_noise)
+from support import SCHEDULES, TENSOR, dense_noise_linear, ensemble, fixture, lv_tempered, schedule_noise, value_case
 
 pytestmark = pytest.mark.gpu
-
-
-def _ens(meta, arrays, nc, **kw):
-    from yagre_mcmc_b200.ensemble import ChainEnsemble, LoweredProblem
-    return ChainEnsemble(LoweredProblem(meta, arrays), nc, **kw)
-
-
-def _check_level(meta, arrays, l, theta, got, label):
-    """theta [n, d], got [n]: level l within the bound; -inf exactly where the reference says so."""
-    lp, b = R.logpost_bound(meta, arrays, l, theta)
-    ref = np.asarray(lp, dtype=np.float64)
-    got = np.asarray(got, dtype=np.float64)
-    inf = ref == -np.inf
-    assert np.array_equal(got[inf], ref[inf]), (label, l, "-inf")
-    e = np.abs(got[~inf].astype(np.longdouble) - lp[~inf]).astype(np.float64)
-    assert np.all(e <= b[~inf]), (label, l, float((e / b[~inf]).max()), int(np.argmax(e / b[~inf])))
-
-
-def _check_values(meta, arrays, theta, lp_dev, label):
-    for l in range(int(meta["levels"])):
-        _check_level(meta, arrays, l, theta, lp_dev[l], label)
-
-
-def value_case(meta, arrays, th0, runs=(3, 2), sample=None, stored=None, seed=3, **kw):
-    """Short Philox runs; after each, the state (and the stored steps of `stored` chains of the sample) against the
-    reference, and yg_logpost at the same points."""
-    nc = th0.shape[0]
-    idx = np.arange(nc) if sample is None or sample >= nc else np.sort(
-        np.random.default_rng(seed).choice(nc, sample, replace=False))
-    st_idx = idx if stored is None else idx[:stored]
-    ens = _ens(meta, arrays, nc, seed=seed, **kw)
-    ens.set_state(th0)
-    label = f"{meta['model']} d={meta['dim']} L={meta['levels']} nc={nc}"
-    for k in runs:
-        out = ens.run(k, samples=True, logpost=True)
-        torch.cuda.synchronize()
-        st = ens.state()
-        th = st["theta"].cpu().numpy().T[idx]
-        _check_values(meta, arrays, th, st["logpost"].cpu().numpy()[:, idx], label)
-        sm, lps = out["samples"].cpu().numpy(), out["logpost"].cpu().numpy()
-        for s in range(k):
-            _check_values(meta, arrays, sm[s].T[st_idx], lps[s][:, st_idx], f"{label} step {s}")
-        for l in range(int(meta["levels"])):
-            _check_level(meta, arrays, l, th, ens.logpost(l, th).cpu().numpy(), f"{label} yg_logpost")
-    ens.close()
 
 
 # ------------------------------------------------------------------------------------------------------------------
@@ -74,7 +28,7 @@ LV_VALUES = {
     "headline": (lambda: bp.lv_problem(True), 65536, 2048, 256, {}),
     "single_level": (lambda: bp.lv_problem(False), 3000, 512, 128, {}),
     "pcn": (bp.lv_pcn_problem, 1000, 512, 128, {}),
-    "tempered_level0": (_lv_tempered, 500, None, 128, {}),
+    "tempered_level0": (lv_tempered, 500, None, 128, {}),
     "one_design_point": (lambda: bp.lv_problem(True, n_data=1), 700, None, None, {}),
     "300_design_points": (lambda: bp.lv_problem(True, n_data=300, Nc=16, Nf=48, prop_var=2e-4), 97, None, None, {}),
     "fine_one_segment": (lambda: bp.lv_problem(True), 1024, 256, 64, dict(rk4_segment=512)),
@@ -106,12 +60,12 @@ def test_one_chain_per_thread_logpost_values(k):
 
 
 GENERIC_VALUES = {
-    "three_level_gauss": (lambda: _fixture("mlda3_gauss2d"), lambda n: np.tile([0.5, 1.0], (n, 1)), 33),
-    "isclose_1d": (lambda: _fixture("mrw_gauss1d"), lambda n: np.full((n, 1), -1.0), 100),
+    "three_level_gauss": (lambda: fixture("mlda3_gauss2d"), lambda n: np.tile([0.5, 1.0], (n, 1)), 33),
+    "isclose_1d": (lambda: fixture("mrw_gauss1d"), lambda n: np.full((n, 1), -1.0), 100),
     "one_chain": (lambda: bp.linear_problem(True), lambda n: np.zeros((n, 2)), 1),
     "40001_chains": (lambda: bp.linear_problem(True), lambda n: np.zeros((n, 2)), 40001),
-    "dense_noise_d5": (_dense_noise_linear, lambda n: 0.1 * np.random.default_rng(1).standard_normal((n, 5)), 999),
-    "tempered_surrogate": (lambda: _fixture("mlda_linear_tempered"), lambda n: np.zeros((n, 2)), 500),
+    "dense_noise_d5": (dense_noise_linear, lambda n: 0.1 * np.random.default_rng(1).standard_normal((n, 5)), 999),
+    "tempered_surrogate": (lambda: fixture("mlda_linear_tempered"), lambda n: np.zeros((n, 2)), 500),
     "adaptive_metropolis": (bp.gauss2d_problem, lambda n: np.tile([-1.0, 2.0], (n, 1)), 300),
 }
 
@@ -141,7 +95,7 @@ def _inject(z, sch):
 
 
 def run_forced(meta, arrays, th0, z, sch, **kw):
-    ens = _ens(meta, arrays, th0.shape[0], seed=5, **kw)
+    ens = ensemble(meta, arrays, th0.shape[0], seed=5, **kw)
     ens.set_state(th0)
     out = ens.run(z.shape[1], samples=True, accepted=True, logpost=True, inject=_inject(z, sch))
     torch.cuda.synchronize()

@@ -3,18 +3,13 @@ misfit sum passes the budget from reject_budget (common.cuh).  Skipping must cha
 
 CPU: the budget against accept_rule on near-ties (host build of common.cuh).
 GPU: with skipping on and off, samples, accept flags, log-posteriors, chain state and counters are bit-identical."""
-import os
-import shutil
-import subprocess
-
 import numpy as np
 import pytest
 import torch
 
 import bench_problems as bp
 from golden_io import load
-
-ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+from support import ensemble, host_program
 
 _NEAR_TIE_PROGRAM = r"""
 #include "yagre_mcmc_b200/csrc/common.cuh"
@@ -76,29 +71,12 @@ int main()
 """
 
 
-def _nvcc():
-    found = shutil.which("nvcc")
-    if found:
-        return found
-    path = os.path.join(os.environ.get("CUDA_HOME") or "/usr/local/cuda", "bin", "nvcc")
-    return path if os.path.exists(path) else None
-
-
 def test_reject_budget_never_certifies_an_accept(tmp_path):
     """Near-ties: sums within 1e-16 .. 1e-7 relative of the exact accept / reject boundary, q split over up to 128
     design points and summed in a random order.  A partial sum above the budget must never belong to a proposal that
     accept_rule accepts; beyond a few times the margin the budget must certify.  u == 0, t <= 0, non-finite t, lp or lps:
     no budget."""
-    nvcc = _nvcc()
-    if nvcc is None:
-        pytest.skip("nvcc not found")
-    src = tmp_path / "near_tie.cu"
-    src.write_text(_NEAR_TIE_PROGRAM)
-    exe = tmp_path / "near_tie"
-    subprocess.run([nvcc, "-std=c++17", "-O2", "-I", ROOT, str(src), "-o", str(exe)], check=True,
-                   capture_output=True)
-    edge_bad, cases, violations, certified, missed = map(int, subprocess.run(
-        [str(exe)], check=True, capture_output=True, text=True).stdout.split())
+    edge_bad, cases, violations, certified, missed = map(int, host_program(tmp_path, "near_tie", _NEAR_TIE_PROGRAM).split())
     assert edge_bad == 0
     assert cases > 200000
     assert violations == 0
@@ -110,8 +88,7 @@ def test_reject_budget_never_certifies_an_accept(tmp_path):
 # GPU: skipping on == skipping off
 # ------------------------------------------------------------------------------------------------------------------
 def _run(meta, arrays, th0, early_reject, ns, inject=None, **kw):
-    from yagre_mcmc_b200.ensemble import ChainEnsemble, LoweredProblem
-    ens = ChainEnsemble(LoweredProblem(meta, arrays), th0.shape[0], seed=77, early_reject=early_reject, **kw)
+    ens = ensemble(meta, arrays, th0.shape[0], seed=77, early_reject=early_reject, **kw)
     ens.set_state(th0)
     if inject is None:
         ens.run(ns, samples=False)                 # a second launch continues with a learned order

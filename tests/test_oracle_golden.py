@@ -5,8 +5,7 @@ import pytest
 
 from oracle import cport
 from golden_io import load, rel_err, CHAIN_CASES, MLDA3_CASES, AM_CASES, TEMPERED_CASES
-
-LOGPOST_RTOL = 1e-10     # north_star: 1e-10 relative on log-posterior
+from support import LOGPOST_RTOL
 
 
 @pytest.mark.parametrize("name", CHAIN_CASES + MLDA3_CASES + TEMPERED_CASES)

@@ -5,7 +5,6 @@ covered by the -m gpu tests; here the per-rank vectors are built with numpy in y
 layout so that the reduction, the restore of the per-chain sample count and the R-hat algebra
 are exercised across two real processes."""
 import os
-import socket
 
 import numpy as np
 import pytest
@@ -13,6 +12,7 @@ import torch
 import torch.distributed as dist
 import torch.multiprocessing as mp
 
+from support import free_port
 from yagre_mcmc_b200.parallel import (shard_range, all_reduce_stats, moments_from_stats,
                                       split_rhat_from_moments, pooled_proposal_covariance)
 
@@ -29,12 +29,6 @@ class _RankEnsemble:
 
     def set_proposal_factor(self, L):
         self.L = np.array(L)
-
-
-def _free_port():
-    with socket.socket() as s:
-        s.bind(("127.0.0.1", 0))
-        return s.getsockname()[1]
 
 
 def _ensemble(seed=3, C=48, n=400, d=2):
@@ -78,7 +72,7 @@ def _worker(rank, world, port, q):
 
 @pytest.mark.timeout(180)
 def test_two_rank_pooling_equals_single_process():
-    world, port = 2, _free_port()
+    world, port = 2, free_port()
     ctx = mp.get_context("spawn")
     q = ctx.Queue()
     procs = [ctx.Process(target=_worker, args=(r, world, port, q)) for r in range(world)]

@@ -5,10 +5,9 @@ import pytest
 import torch
 
 from golden_io import load, rel_err, CHAIN_CASES, MLDA3_CASES, TEMPERED_CASES, AM_CASES
+from support import LOGPOST_RTOL, ensemble
 
 pytestmark = pytest.mark.gpu
-
-LOGPOST_RTOL = 1e-10      # north_star: 1e-10 relative on log-posterior
 
 
 def to_device_layout(a):
@@ -20,10 +19,8 @@ def to_device_layout(a):
 
 
 def run_gpu(meta, a, **kw):
-    from yagre_mcmc_b200.ensemble import ChainEnsemble, LoweredProblem
-    pb = LoweredProblem(meta, a)
     nc, ns = a["u_f"].shape
-    ens = ChainEnsemble(pb, nc, **kw)
+    ens = ensemble(meta, a, nc, **kw)
     ens.set_state(a["theta0"])
     st0 = ens.state()
     out = ens.run(ns, samples=True, accepted=True, logpost=True, inject=to_device_layout(a))

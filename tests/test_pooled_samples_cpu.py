@@ -6,7 +6,6 @@ restatement, its bounds against the kernel's formulation in double and against r
 two halves of the chains must pool to the single-rank answer; the device kernel is covered by the -m gpu tests."""
 import ctypes as C
 import os
-import socket
 
 import numpy as np
 import pytest
@@ -15,6 +14,7 @@ import torch.distributed as dist
 import torch.multiprocessing as mp
 
 import pooled_samples_reference as psr
+from support import free_port
 from yagre_mcmc_b200 import _lib
 from yagre_mcmc_b200.parallel import moments_from_stats, shard_range
 
@@ -88,12 +88,6 @@ def test_raw_moments_fail_the_bound_on_offset_data():
     assert ratio > 100.0, ratio
 
 
-def _free_port():
-    with socket.socket() as s:
-        s.bind(("127.0.0.1", 0))
-        return s.getsockname()[1]
-
-
 def _samples(seed=11, ns=30, d=5, nc=40):
     rng = np.random.default_rng(seed)
     return (rng.standard_normal((ns, d, nc)) * np.linspace(0.5, 2.0, d)[None, :, None]
@@ -133,7 +127,7 @@ def _worker(rank, world, port, q):
 
 @pytest.mark.timeout(180)
 def test_two_rank_pooling_from_samples_equals_single_rank():
-    world, port = 2, _free_port()
+    world, port = 2, free_port()
     ctx = mp.get_context("spawn")
     q = ctx.Queue()
     procs = [ctx.Process(target=_worker, args=(r, world, port, q)) for r in range(world)]

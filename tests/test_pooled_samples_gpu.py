@@ -14,16 +14,11 @@ import torch
 import bench_problems as bp
 import diag_reference as dr
 import pooled_samples_reference as psr
+from support import check_closed_form, ensemble, linear_chain
 from yagre_mcmc_b200 import _lib
-from yagre_mcmc_b200.ensemble import ChainEnsemble, LoweredProblem, pooled_sample_stats, iat_ess
+from yagre_mcmc_b200.ensemble import pooled_sample_stats, iat_ess
 from yagre_mcmc_b200.parallel import moments_from_stats
 from yagre_mcmc_b200.parameter import ParameterVector
-from yagre_mcmc_b200.model import ForwardModel, LinearModelSolver
-from yagre_mcmc_b200.statistics import (IIDCovarianceMatrix, Gaussian, CentredGaussianNoise, Data,
-                                        AdditiveGaussianNoiseLikelihood, BayesianRegressionModel,
-                                        BayesianRegressionModelHierarchy)
-from yagre_mcmc_b200.utility import Hierarchy, SharedComponent
-from yagre_mcmc_b200.chain.method import MRWBuilder, MLDABuilder, PCNBuilder
 
 pytestmark = pytest.mark.gpu
 
@@ -104,7 +99,7 @@ def test_agrees_with_welford_path_on_pre_transition_states(case):
     else:
         (meta, arrays), nc, ns = bp.lv_problem(True), 256, 40
         th0 = bp.lv_initial_states(nc)
-    ens = ChainEnsemble(LoweredProblem(meta, arrays), nc, seed=21)
+    ens = ensemble(meta, arrays, nc, seed=21)
     ens.set_state(th0)
     samples = ens.run(ns, samples=True)["samples"]
     traj = torch.cat([torch.from_numpy(th0.T.copy()).cuda()[None], samples])
@@ -123,41 +118,6 @@ def test_agrees_with_welford_path_on_pre_transition_states(case):
     assert w[0] == v[0] == nc and w[1] == v[1] == ns
 
 
-def _linear_chain(d, dd, two_level, nc, seed, thin, store=True, pcn=False):
-    meta, a = bp.big_linear_problem(d, dd, 1, two_level=two_level, J=3)
-    noise = CentredGaussianNoise(IIDCovarianceMatrix(dd, 0.05))
-    prior = Gaussian(ParameterVector(np.zeros(d)), IIDCovarianceMatrix(d, 2.0))
-    levels = 2 if two_level else 1
-    lik = [AdditiveGaussianNoiseLikelihood(Data(a["L0_data"]), ForwardModel(LinearModelSolver(a[f"L{l}_G"], a[f"L{l}_b"])),
-                                           noise) for l in range(levels)]
-    prop = IIDCovarianceMatrix(d, float(a["prop_L"][0, 0]) ** 2)
-    if two_level:
-        b = MLDABuilder()
-        b.bayesModel = BayesianRegressionModelHierarchy(Hierarchy(lik), SharedComponent(prior, 2))
-        b.baseProposalCovariance = prop
-        b.subChainLengths = [3]
-    elif pcn:
-        b = PCNBuilder()
-        b.bayesModel = BayesianRegressionModel(lik[0], prior)
-        b.stepSize = 0.01
-    else:
-        b = MRWBuilder()
-        b.bayesModel = BayesianRegressionModel(lik[0], prior)
-        b.proposalCovariance = prop
-    b.nChains, b.seed, b.thin, b.storeTrajectory = nc, seed, thin, store
-    return b.build_method(), bp.linear_gaussian_posterior(a, levels - 1)
-
-
-def _check_closed_form(out, mean, cov, C, label):
-    """Chains started from exact posterior draws are stationary: each is worth at least one independent draw, so the
-    pooled mean has variance <= Sigma_ii / C and the pooled covariance (Sigma_ii Sigma_jj + Sigma_ij^2) / C."""
-    sm = np.sqrt(np.diag(cov) / C)
-    assert np.all(np.abs(out["mean"] - mean) <= 5 * sm), (label, "mean", np.abs(out["mean"] - mean).max())
-    dg = np.diag(cov)
-    sc = np.sqrt((np.outer(dg, dg) + cov ** 2) / C)
-    assert np.all(np.abs(out["covariance"] - cov) <= 5 * sc), (label, "covariance", (np.abs(out["covariance"] - cov) / sc).max())
-
-
 def _rhat_restated(vec, d):
     v = np.asarray(vec, dtype=np.float64)
     C, n = v[0], v[1]
@@ -173,8 +133,8 @@ def test_tensor_path_pooling_through_the_builders(case):
     d, dd, two = (64, 256, False) if case == "single_64x256" else (32, 96, True)
     C, thin, n1, n2 = 4096, 10, 1001, 10001
     rng = np.random.default_rng(17)
-    mc, (mean, cov) = _linear_chain(d, dd, two, C, seed=5, thin=thin)
-    iso, _ = _linear_chain(d, dd, two, C, seed=5, thin=thin)
+    mc, (mean, cov) = linear_chain(d, dd, two, C, seed=5, thin=thin)
+    iso, _ = linear_chain(d, dd, two, C, seed=5, thin=thin)
     draws1, draws2 = rng.multivariate_normal(mean, cov, size=C), rng.multivariate_normal(mean, cov, size=C)
 
     mc.run(n1, ParameterVector(draws1), verbose=False)
@@ -184,7 +144,7 @@ def test_tensor_path_pooling_through_the_builders(case):
     c = mc.ensemble.counters()
     assert out["n_chains"] == C and out["samples_per_chain"] == traj.shape[0]
     assert abs(out["acceptance_rate"] - c["accepted"] / c["transitions"]) < 1e-12
-    _check_closed_form(out, mean, cov, C, case + " isotropic")
+    check_closed_form(out, mean, cov, C, case + " isotropic")
     vec = pooled_sample_stats(traj).cpu().numpy()
     np.testing.assert_allclose(out["rhat"], _rhat_restated(vec, d), rtol=1e-10)
 
@@ -196,7 +156,7 @@ def test_tensor_path_pooling_through_the_builders(case):
     if d == 64:
         assert mc.ensemble.last_launch()["block"] == 4 * 32          # the dense-factor instance
     out2 = mc.pooled()
-    _check_closed_form(out2, mean, cov, C, case + " pooled dense")
+    check_closed_form(out2, mean, cov, C, case + " pooled dense")
     iat_dense = np.median(iat_ess(mc.chain.trajectory.device_tensor)[0].cpu().numpy())
 
     iso.run(n1, ParameterVector(draws1), verbose=False)
@@ -207,7 +167,7 @@ def test_tensor_path_pooling_through_the_builders(case):
 
 
 def test_refusals():
-    mc, (mean, _) = _linear_chain(64, 256, False, 64, seed=1, thin=5, store=False)
+    mc, (mean, _) = linear_chain(64, 256, False, 64, seed=1, thin=5, store=False)
     mc.run(11, ParameterVector(mean), verbose=False)
     with pytest.raises(NotImplementedError, match="storeTrajectory"):
         mc.pooled()
@@ -215,7 +175,7 @@ def test_refusals():
         mc.pool_proposal_covariance()
     with pytest.raises(NotImplementedError):                          # still no full second moment on the tensor path
         mc.ensemble.pooled_stats()
-    stored, _ = _linear_chain(64, 256, False, 64, seed=1, thin=5)
+    stored, _ = linear_chain(64, 256, False, 64, seed=1, thin=5)
     with pytest.raises(NotImplementedError, match="storeTrajectory"):  # nothing run yet
         stored.pooled()
     stored.run(11, ParameterVector(mean), verbose=False)
@@ -224,7 +184,7 @@ def test_refusals():
         stored.pooled()
     with pytest.raises(ValueError):
         stored.ensemble.rebuild_proposal_factor(np.ones((64, 64)))     # not lower triangular
-    pcn, (mean, _) = _linear_chain(32, 96, False, 64, seed=1, thin=5, pcn=True)
+    pcn, (mean, _) = linear_chain(32, 96, False, 64, seed=1, thin=5, pcn=True)
     pcn.run(11, ParameterVector(mean), verbose=False)
     with np.errstate(divide="ignore", invalid="ignore"):             # R-hat of chains that have not moved: 0 / 0
         assert pcn.pooled()["n_chains"] == 64

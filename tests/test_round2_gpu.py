@@ -7,26 +7,9 @@ import torch
 import bench_problems as bp
 from diag_reference import check_replay_diagnostics, pre_states
 from golden_io import load, rel_err
+from support import LOGPOST_RTOL, ensemble, replay, three_level_gauss
 
 pytestmark = pytest.mark.gpu
-
-LOGPOST_RTOL = 1e-10      # north_star: 1e-10 relative on log-posterior
-
-
-def _ens(meta, arrays, nc, **kw):
-    from yagre_mcmc_b200.ensemble import ChainEnsemble, LoweredProblem
-    return ChainEnsemble(LoweredProblem(meta, arrays), nc, **kw)
-
-
-def _replay(meta, arrays, th0, out, rows=None, adaptive=None):
-    from oracle import cport
-    z = out["z"].cpu().numpy().transpose(3, 0, 1, 2)
-    u_c = np.nan_to_num(out["u_c"].cpu().numpy().transpose(2, 0, 1), nan=0.5)
-    u_f = np.nan_to_num(out["u_f"].cpu().numpy().transpose(1, 0), nan=0.5)
-    if rows is not None:
-        z, u_c, u_f, th0 = z[rows], u_c[rows], u_f[rows], th0[rows]
-    return cport.run_injected(cport.Problem(meta, arrays, adaptive=adaptive), th0, z, u_c, u_f)
-
 
 # ------------------------------------------------------------------------------------------
 # the noise stream keeps advancing across set_state (ADVICE r1, high)
@@ -43,7 +26,7 @@ def test_stream_position_survives_set_state(case):
     else:
         (meta, arrays), th0, n = bp.lv_problem(True), bp.lv_initial_states(300), 12
     nc = th0.shape[0]
-    a = _ens(meta, arrays, nc, seed=5)
+    a = ensemble(meta, arrays, nc, seed=5)
     a.set_state(th0)
     r1 = a.run(n, samples=True)["samples"].clone()
     assert a.counters()["step_index"] == n
@@ -55,11 +38,11 @@ def test_stream_position_survives_set_state(case):
     r3 = a.run(n, samples=True)["samples"]
     assert torch.equal(r1, r3)
     # restart from the end of r1 + run(n)  ==  run(2n) in one go
-    b = _ens(meta, arrays, nc, seed=5)
+    b = ensemble(meta, arrays, nc, seed=5)
     b.set_state(th0)
     full = b.run(2 * n, samples=True)["samples"]
     assert torch.equal(full[:n], r1)
-    c = _ens(meta, arrays, nc, seed=5)
+    c = ensemble(meta, arrays, nc, seed=5)
     c.set_state(th0)
     c.run(n, samples=False)
     end = c.state()["theta"].t().contiguous()
@@ -82,7 +65,7 @@ def test_keep_flags_control_what_a_restart_resets():
     meta, arrays = bp.gauss2d_problem()
     nc = 128
     ad = dict(idle=5, collection=20, eps=1e-4)
-    e = _ens(meta, arrays, nc, seed=3, adaptive=ad)
+    e = ensemble(meta, arrays, nc, seed=3, adaptive=ad)
     th0 = np.tile([-8.0, -7.0], (nc, 1))
     e.set_state(th0)
     e.run(60, samples=False)
@@ -111,11 +94,11 @@ def test_lv_adaptive_philox_run_replayed_through_oracle(two_level):
     ad = dict(idle=6, collection=15, eps=1e-6, refresh=2)
     nc, ns = 700, 30
     th0 = bp.lv_initial_states(nc)
-    ens = _ens(meta, arrays, nc, seed=31, adaptive=ad)
+    ens = ensemble(meta, arrays, nc, seed=31, adaptive=ad)
     ens.set_state(th0)
     out = ens.run(ns, samples=True, accepted=True, logpost=True, record=True)
     torch.cuda.synchronize()
-    ref = _replay(meta, arrays, th0, out, adaptive=ad)
+    ref = replay(meta, arrays, th0, out, adaptive=ad)
     acc = out["accepted"].cpu().numpy().T
     assert int((acc != ref["accepted"]).sum()) == 0
     traj = out["samples"].cpu().numpy().transpose(2, 0, 1)
@@ -134,13 +117,13 @@ def test_lv_adaptive_resume_is_bit_exact():
     ad = dict(idle=4, collection=10, eps=1e-6)
     nc = 200
     th0 = bp.lv_initial_states(nc)
-    a = _ens(meta, arrays, nc, seed=8, adaptive=ad)
+    a = ensemble(meta, arrays, nc, seed=8, adaptive=ad)
     a.set_state(th0)
     ra = a.run(24, samples=True)["samples"]
-    b = _ens(meta, arrays, nc, seed=8, adaptive=ad)
+    b = ensemble(meta, arrays, nc, seed=8, adaptive=ad)
     b.set_state(th0)
     b.run(12, samples=False)
-    c = _ens(meta, arrays, nc, seed=8, adaptive=ad)
+    c = ensemble(meta, arrays, nc, seed=8, adaptive=ad)
     c.load_state(b.state())
     rc = c.run(12, samples=True)["samples"]
     assert torch.equal(ra[12:], rc)
@@ -158,7 +141,7 @@ def test_lv_adaptive_posterior_moments_and_acceptance(two_level):
     _, g = load("lv_long_twoLevel" if two_level else "lv_long_singleLevel")
     meta, arrays = bp.lv_problem(two_level)
     nc = 8192
-    ens = _ens(meta, arrays, nc, seed=77, adaptive=dict(idle=50, collection=200, eps=1e-8, refresh=5))
+    ens = ensemble(meta, arrays, nc, seed=77, adaptive=dict(idle=50, collection=200, eps=1e-8, refresh=5))
     ens.set_state(bp.lv_initial_states(nc))
     ens.run(600, samples=False)
     c0 = ens.counters()
@@ -185,7 +168,7 @@ def test_headline_geometry_direct_replay():
     meta, arrays = bp.lv_problem(True)
     nc, ns = 65536, 50
     th0 = bp.lv_initial_states(nc)
-    ens = _ens(meta, arrays, nc, seed=20261018)
+    ens = ensemble(meta, arrays, nc, seed=20261018)
     ens.set_state(th0)
     out = ens.run(ns, samples=True, accepted=True, logpost=True, record=True)
     torch.cuda.synchronize()
@@ -195,7 +178,7 @@ def test_headline_geometry_direct_replay():
     rows = np.sort(np.random.default_rng(5).choice(nc, 256, replace=False))
     idx = torch.from_numpy(rows).to("cuda")
     sub = {k: out[k].index_select(out[k].dim() - 1, idx) for k in ("z", "u_c", "u_f", "samples", "accepted", "logpost")}
-    ref = _replay(meta, arrays, th0[rows], sub)
+    ref = replay(meta, arrays, th0[rows], sub)
     acc = sub["accepted"].cpu().numpy().T
     assert int((acc != ref["accepted"]).sum()) == 0
     traj = sub["samples"].cpu().numpy().transpose(2, 0, 1)
@@ -209,22 +192,16 @@ def test_headline_geometry_direct_replay():
 # ------------------------------------------------------------------------------------------
 # MLDA with two surrogates / tempered surrogate: Philox runs replayed, statistics
 # ------------------------------------------------------------------------------------------
-def _three_level_gauss():
-    _, a = load("mlda3_gauss2d")
-    arrays = {k: a[k] for k in a if k.startswith(("L0_", "L1_", "L2_")) or k == "prop_L"}
-    return dict(model="gauss", dim=2, levels=3, J=6, eq="exact"), arrays
-
-
 def test_three_level_philox_run_replayed_through_oracle():
-    meta, arrays = _three_level_gauss()
+    meta, arrays = three_level_gauss()
     nc, ns = 1000, 200
     th0 = np.tile([-8.0, -7.0], (nc, 1))
     for seed, record in ((4, True), (4, False)):
-        ens = _ens(meta, arrays, nc, seed=seed)
+        ens = ensemble(meta, arrays, nc, seed=seed)
         ens.set_state(th0)
         out = ens.run(ns, samples=True, accepted=True, logpost=True, record=record)
         if record:
-            ref = _replay(meta, arrays, th0, out)
+            ref = replay(meta, arrays, th0, out)
             acc = out["accepted"].cpu().numpy().T
             assert int((acc != ref["accepted"]).sum()) == 0
             traj = out["samples"].cpu().numpy().transpose(2, 0, 1)
@@ -248,9 +225,9 @@ def test_three_level_posterior_moments():
     container: [[3.86, -0.86], [-0.86, 1.00]], acceptance 0.52-0.53) -- its two-surrogate recursion screens with
     the finest surrogate although the sub-chain ran on the base one, so it does not reproduce the target's
     [[2.4, -0.5], [-0.5, 0.7]]; a drop-in has to match the reference, not the textbook."""
-    meta, arrays = _three_level_gauss()
+    meta, arrays = three_level_gauss()
     nc = 4096
-    ens = _ens(meta, arrays, nc, seed=42)
+    ens = ensemble(meta, arrays, nc, seed=42)
     ens.set_state(np.tile([-8.0, -7.0], (nc, 1)))
     ens.run(500, samples=False)
     c0 = ens.counters()
@@ -267,18 +244,18 @@ def test_tempered_surrogate_philox_replay():
     arrays = {k: a[k] for k in a if k.startswith(("L0_", "L1_")) or k == "prop_L"}
     nc, ns = 500, 150
     th0 = np.zeros((nc, 2))
-    ens = _ens(meta, arrays, nc, seed=6)
+    ens = ensemble(meta, arrays, nc, seed=6)
     ens.set_state(th0)
     out = ens.run(ns, samples=True, accepted=True, logpost=True, record=True)
-    ref = _replay(meta, arrays, th0, out)
+    ref = replay(meta, arrays, th0, out)
     assert int((out["accepted"].cpu().numpy().T != ref["accepted"]).sum()) == 0
     lp = out["logpost"].cpu().numpy().transpose(2, 0, 1)
     assert rel_err(lp[:, :, 0], ref["logpost_L0"][:, 1:]).max() <= LOGPOST_RTOL
     # the tempered surrogate is flatter than the untempered one: a different coarse log-posterior
     plain = dict(arrays); plain.pop("L0_tempering")
-    e2 = _ens(meta, plain, 4, seed=6)
+    e2 = ensemble(meta, plain, 4, seed=6)
     e2.set_state(np.full((4, 2), 0.3))
-    e3 = _ens(meta, arrays, 4, seed=6)
+    e3 = ensemble(meta, arrays, 4, seed=6)
     e3.set_state(np.full((4, 2), 0.3))
     assert not torch.allclose(e2.state()["logpost"][0], e3.state()["logpost"][0])
     assert torch.equal(e2.state()["logpost"][1], e3.state()["logpost"][1])
@@ -291,13 +268,13 @@ def test_lv_tempered_level_through_logpost():
     arrays = dict(arrays); arrays["L0_tempering"] = np.array(0.4)
     nc, ns = 64, 20
     th0 = bp.lv_initial_states(nc)
-    ens = _ens(meta, arrays, nc, seed=2)
+    ens = ensemble(meta, arrays, nc, seed=2)
     ens.set_state(th0)
     pb = cport.Problem(meta, arrays)
     want = np.array([cport.logpost(pb, 0, t) for t in th0])
     np.testing.assert_allclose(ens.state()["logpost"][0].cpu().numpy(), want, rtol=LOGPOST_RTOL)
     out = ens.run(ns, samples=True, accepted=True, logpost=True, record=True)
-    ref = _replay(meta, arrays, th0, out)
+    ref = replay(meta, arrays, th0, out)
     assert int((out["accepted"].cpu().numpy().T != ref["accepted"]).sum()) == 0
     lp = out["logpost"].cpu().numpy().transpose(2, 0, 1)
     assert rel_err(lp[:, :, 0], ref["logpost_L0"][:, 1:]).max() <= LOGPOST_RTOL
@@ -309,13 +286,13 @@ def test_unsupported_combinations_are_refused():
     a3 = dict(arrays)
     a3.update({k.replace("L1_", "L2_"): v for k, v in arrays.items() if k.startswith("L1_")})
     with pytest.raises(NotImplementedError):                   # three levels: one-chain-per-thread kernels only
-        _ens(m3, a3, 8)
+        ensemble(m3, a3, 8)
     bm, ba = bp.big_linear_problem(16, 24, 2)
     with pytest.raises(NotImplementedError):                   # no adaptive proposal on the tensor path
-        _ens(bm, ba, 8, adaptive=dict(idle=1, collection=2))
+        ensemble(bm, ba, 8, adaptive=dict(idle=1, collection=2))
     with pytest.raises(NotImplementedError):                   # no adaptive error model on the tensor path (ADVICE r1)
         bm2, ba2 = bp.big_linear_problem(16, 24, 2, two_level=True, J=2)
-        _ens(bm2, ba2, 8, aem=dict(min_data=3, heuristic=False))
+        ensemble(bm2, ba2, 8, aem=dict(min_data=3, heuristic=False))
 
 
 # ------------------------------------------------------------------------------------------
@@ -352,7 +329,7 @@ def test_dmma_path_normals_match_the_oracle_transform():
     from oracle import cport
     meta, arrays = bp.big_linear_problem(23, 45, 3)
     nc, ns, seed = 96, 40, 4242
-    ens = _ens(meta, arrays, nc, seed=seed, chain_offset=1000)
+    ens = ensemble(meta, arrays, nc, seed=seed, chain_offset=1000)
     ens.set_state(np.zeros((nc, 23)))
     out = ens.run(ns, samples=False, record=True)
     z = out["z"].cpu().numpy()                               # [ns, 1, d, nc]
@@ -382,7 +359,7 @@ def test_dmma_philox_launch_equals_recorded_launch_and_is_shard_invariant(case):
     th0 = 0.01 * np.random.default_rng(3).standard_normal((nc, d))
     runs = []
     for record in (False, True):
-        ens = _ens(meta, arrays, nc, seed=12)
+        ens = ensemble(meta, arrays, nc, seed=12)
         ens.set_state(th0)
         o1 = ens.run(ns, samples=True, accepted=True, logpost=True, record=record)
         o2 = ens.run(5, samples=True, thin=5, record=record)                 # continues: stream position, Welford
@@ -394,7 +371,7 @@ def test_dmma_philox_launch_equals_recorded_launch_and_is_shard_invariant(case):
     for k in ("theta", "logpost", "n_accept", "w_mean", "w_m2"):
         assert torch.equal(runs[0][2][k], runs[1][2][k]), k
     off, m = 8000 if nc > 10000 else 1234, 800
-    sub = _ens(meta, arrays, m, seed=12, chain_offset=off)
+    sub = ensemble(meta, arrays, m, seed=12, chain_offset=off)
     sub.set_state(th0[off:off + m])
     s1 = sub.run(ns, samples=True, accepted=True, logpost=True)
     for k in ("samples", "accepted", "logpost"):
@@ -410,7 +387,7 @@ def test_dmma_philox_launch_equals_recorded_launch_and_is_shard_invariant(case):
     idx = torch.from_numpy(rows).to("cuda")
     o1 = runs[1][0]
     rec = {k: o1[k].index_select(o1[k].dim() - 1, idx) for k in ("z", "u_c", "u_f", "samples", "accepted", "logpost")}
-    ref = _replay(meta, arrays, th0[rows], rec)
+    ref = replay(meta, arrays, th0[rows], rec)
     assert int((rec["accepted"].cpu().numpy().T != ref["accepted"]).sum()) == 0
     assert rel_err(rec["samples"].cpu().numpy().transpose(2, 0, 1), ref["traj"][:, 1:]).max() <= 1e-12
     lp = rec["logpost"].cpu().numpy().transpose(2, 0, 1)
@@ -433,7 +410,7 @@ def test_dmma_path_dense_covariances_posterior_moments():
     arrays["L0_prior_mean"] = 0.1 * rng.standard_normal(d)
     mean, cov = bp.linear_gaussian_posterior(arrays, 0)
     arrays["prop_L"] = np.linalg.cholesky(2.4 ** 2 / d * cov)            # dense, posterior shaped
-    ens = _ens(meta, arrays, nc, seed=3)
+    ens = ensemble(meta, arrays, nc, seed=3)
     ens.set_state(np.tile(mean, (nc, 1)))
     ens.run(400, samples=False)
     c0 = ens.counters()
@@ -448,7 +425,7 @@ def test_dmma_path_dense_covariances_posterior_moments():
     lp = ens.logpost(0, np.tile(mean, (3, 1))).cpu().numpy()
     from oracle import cport
     np.testing.assert_allclose(lp, cport.logpost(cport.Problem(meta, arrays), 0, mean), rtol=1e-10)
-    diag = _ens(*bp.big_linear_problem(d, dd, 2), 64, seed=1)
+    diag = ensemble(*bp.big_linear_problem(d, dd, 2), 64, seed=1)
     with pytest.raises(NotImplementedError):
         diag.set_proposal_factor(arrays["prop_L"])
     ens.set_proposal_factor(0.5 * arrays["prop_L"])                      # a dense handle takes another dense factor
@@ -463,7 +440,7 @@ def test_dmma_acceptance_only_diagnostics_skips_the_moments_and_nothing_else():
     th0 = 0.01 * np.random.default_rng(5).standard_normal((nc, 32))
     res = []
     for welford in (True, False):
-        ens = _ens(meta, arrays, nc, seed=9, welford=welford)
+        ens = ensemble(meta, arrays, nc, seed=9, welford=welford)
         ens.set_state(th0)
         out = ens.run(ns, samples=True, accepted=True, logpost=True)
         res.append((out, ens.state(), ens.counters()))
@@ -486,10 +463,10 @@ def test_dmma_short_launches_compose(shape):
     meta, arrays = bp.big_linear_problem(d, dd, 2, two_level=two, J=2)
     for nc in (5, 2500, 20011):
         th0 = 0.01 * np.random.default_rng(nc).standard_normal((nc, d))
-        a = _ens(meta, arrays, nc, seed=2)
+        a = ensemble(meta, arrays, nc, seed=2)
         a.set_state(th0)
         whole = a.run(6, samples=True, accepted=True)
-        b = _ens(meta, arrays, nc, seed=2)
+        b = ensemble(meta, arrays, nc, seed=2)
         b.set_state(th0)
         parts = [b.run(k, samples=True, accepted=True) for k in (1, 2, 3)]
         assert torch.equal(whole["samples"], torch.cat([p["samples"] for p in parts]))
@@ -558,11 +535,11 @@ def test_seeded_shape_sweep_replayed_through_oracle(k):
     output; MRW, pCN, per-chain adaptive Metropolis, dense proposal factor with a dense prior precision.  Identical
     accept decisions, trajectories to 1e-12, log-posterior to north_star's 1e-10."""
     label, meta, arrays, th0, nc, ns, thin, ad = _sweep_case(k)
-    ens = _ens(meta, arrays, nc, seed=500 + k, adaptive=ad)
+    ens = ensemble(meta, arrays, nc, seed=500 + k, adaptive=ad)
     ens.set_state(th0)
     out = ens.run(ns, thin=thin, samples=True, accepted=True, logpost=True, record=True)
     torch.cuda.synchronize()
-    ref = _replay(meta, arrays, th0, out, adaptive=ad)
+    ref = replay(meta, arrays, th0, out, adaptive=ad)
     acc = out["accepted"].cpu().numpy().T
     assert int((acc != ref["accepted"]).sum()) == 0, label
     traj = out["samples"].cpu().numpy().transpose(2, 0, 1)                  # every thin-th state
@@ -604,7 +581,7 @@ def test_lv_results_do_not_depend_on_launch_geometry(two_level, nc):
             dict(threads_per_block=512, rk4_segment=300), dict(threads_per_block=640, rk4_segment=17)]
     ref = None
     for geo in geos:
-        ens = _ens(meta, arrays, nc, seed=4242, **geo)
+        ens = ensemble(meta, arrays, nc, seed=4242, **geo)
         ens.set_state(th0)
         ens.run(ns, samples=False)
         out = ens.run(ns, samples=True, accepted=True, logpost=True)

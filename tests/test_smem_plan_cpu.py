@@ -5,13 +5,7 @@ up to 320 operand rows per level on one or two levels, dense or diagonal proposa
 Every region is aligned for its element type (the blob end at 16 bytes), lies inside the launch's bytes and overlaps no
 other; the launch stays within 227 KiB, the LV kernel within its 220 KiB / blocks_per_sm budget up to the rounding that
 its cap formula ignores; the tensor path refuses a problem exactly when four warps do not fit."""
-import os
-import shutil
-import subprocess
-
-import pytest
-
-ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+from support import host_program
 
 # The LV cap divides the budget by the unpadded bytes per chain.  Rounding the end of the int arrays up to 16 bytes
 # adds at most 12 bytes (every region before it is a multiple of 4 bytes), padding evald to 16 bytes at most 15.
@@ -115,23 +109,8 @@ int main()
 """
 
 
-def _nvcc():
-    found = shutil.which("nvcc")
-    if found:
-        return found
-    path = os.path.join(os.environ.get("CUDA_HOME") or "/usr/local/cuda", "bin", "nvcc")
-    return path if os.path.exists(path) else None
-
-
 def test_shared_memory_plans(tmp_path):
-    nvcc = _nvcc()
-    if nvcc is None:
-        pytest.skip("nvcc not found")
-    src = tmp_path / "smem_plan.cu"
-    src.write_text(_PROGRAM.replace("SLACK", str(LV_ROUNDING_SLACK)))
-    exe = tmp_path / "smem_plan"
-    subprocess.run([nvcc, "-std=c++17", "-O2", "-I", ROOT, str(src), "-o", str(exe)], check=True, capture_output=True)
-    lines = subprocess.run([str(exe)], check=True, capture_output=True, text=True).stdout.splitlines()
+    lines = host_program(tmp_path, "smem_plan", _PROGRAM.replace("SLACK", str(LV_ROUNDING_SLACK))).splitlines()
     lv_cases, t_cases, t_refused, overlap, misaligned, outside, over, wrong, refusal = map(int, lines[0].split())
     assert lv_cases == 2 * 300 * 4 * 20
     assert t_cases > 100000 and 0 < t_refused < t_cases

@@ -9,13 +9,7 @@ diagonal proposal factor, Welford tiles asked for or not:
       227 KiB; it has at least 4 warps;
   (c) no shape of the envelope is refused.
 And the plans of the shapes profiles/streamed_operand.md measures."""
-import os
-import shutil
-import subprocess
-
-import pytest
-
-ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+from support import host_program
 
 _PROGRAM = r"""
 #include "yagre_mcmc_b200/csrc/common.cuh"
@@ -122,23 +116,8 @@ int main()
 """
 
 
-def _nvcc():
-    found = shutil.which("nvcc")
-    if found:
-        return found
-    path = os.path.join(os.environ.get("CUDA_HOME") or "/usr/local/cuda", "bin", "nvcc")
-    return path if os.path.exists(path) else None
-
-
 def test_streamed_operand_plans(tmp_path):
-    nvcc = _nvcc()
-    if nvcc is None:
-        pytest.skip("nvcc not found")
-    src = tmp_path / "streamed_plan.cu"
-    src.write_text(_PROGRAM)
-    exe = tmp_path / "streamed_plan"
-    subprocess.run([nvcc, "-std=c++17", "-O2", "-I", ROOT, str(src), "-o", str(exe)], check=True, capture_output=True)
-    lines = subprocess.run([str(exe)], check=True, capture_output=True, text=True).stdout.splitlines()
+    lines = host_program(tmp_path, "streamed_plan", _PROGRAM).splitlines()
     cases, streamed, s_g1, s_ld, s_both = map(int, lines[0].split())
     assert cases > 400000 and streamed > 1000
     assert s_g1 > 0 and s_ld > 0 and s_both > 0 and s_g1 + s_ld + s_both == streamed

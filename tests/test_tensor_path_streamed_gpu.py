@@ -17,28 +17,10 @@ import torch
 
 import bench_problems as bp
 from golden_io import rel_err
-from test_diagnostics_reference_gpu import check_case
-from test_logpost_reference_gpu import value_case
-from test_pooled_samples_gpu import _check_closed_form, _linear_chain
+from support import LOGPOST_RTOL, check_case, check_closed_form, ensemble, linear_chain, replay, value_case
 from yagre_mcmc_b200.parameter import ParameterVector
 
 pytestmark = pytest.mark.gpu
-
-LOGPOST_RTOL = 1e-10
-
-
-def _ens(meta, arrays, nc, **kw):
-    from yagre_mcmc_b200.ensemble import ChainEnsemble, LoweredProblem
-    return ChainEnsemble(LoweredProblem(meta, arrays), nc, **kw)
-
-
-def _replay(meta, arrays, th0, out):
-    from oracle import cport
-    z = out["z"].cpu().numpy().transpose(3, 0, 1, 2)
-    u_c = np.nan_to_num(out["u_c"].cpu().numpy().transpose(2, 0, 1), nan=0.5)
-    u_f = np.nan_to_num(out["u_f"].cpu().numpy().transpose(1, 0), nan=0.5)
-    return cport.run_injected(cport.Problem(meta, arrays), th0, z, u_c, u_f)
-
 
 def traj_err(got, ref, dense_L):
     """Trajectory error: relative per coordinate; with a dense factor relative to the larger of the value and the
@@ -126,13 +108,13 @@ def test_streamed_replay_counters_and_diagnostics(name, nc, thin):
     check_case(meta, arrays, th0, [("run", 1), ("run", 2), ("run", 3)], seed=41, smem=smem, label=label)
     # a thinned recorded run replayed through the oracle
     ns = 3 * thin
-    ens = _ens(meta, arrays, nc, seed=43)
+    ens = ensemble(meta, arrays, nc, seed=43)
     ens.set_state(th0)
     out = ens.run(ns, thin=thin, samples=True, accepted=True, logpost=True, record=True)
     torch.cuda.synchronize()
     launch = ens.last_launch()
     assert launch["smem"] == smem and launch["block"] == 32 * warps, (label, launch, warps, smem)
-    ref = _replay(meta, arrays, th0, out)
+    ref = replay(meta, arrays, th0, out)
     acc = out["accepted"].cpu().numpy().T
     assert np.array_equal(acc, ref["accepted"]), label
     got = out["samples"].cpu().numpy().transpose(2, 0, 1)           # [nc, ns / thin, d]
@@ -159,7 +141,7 @@ def test_streamed_philox_equals_recorded_and_shards(name):
     th0 = 0.01 * np.random.default_rng(3).standard_normal((nc, d))
     runs = []
     for record in (False, True):
-        ens = _ens(meta, arrays, nc, seed=12)
+        ens = ensemble(meta, arrays, nc, seed=12)
         ens.set_state(th0)
         runs.append((ens.run(ns, samples=True, accepted=True, logpost=True, record=record), ens.state(), ens.counters()))
     for k in ("samples", "accepted", "logpost"):
@@ -170,7 +152,7 @@ def test_streamed_philox_equals_recorded_and_shards(name):
     off = 8000
     parts = []
     for lo, hi in ((0, off), (off, nc)):
-        sub = _ens(meta, arrays, hi - lo, seed=12, chain_offset=lo)
+        sub = ensemble(meta, arrays, hi - lo, seed=12, chain_offset=lo)
         sub.set_state(th0[lo:hi])
         parts.append(sub.run(ns, samples=True, accepted=True, logpost=True))
     for k in ("samples", "accepted", "logpost"):
@@ -181,10 +163,10 @@ def test_streamed_short_launches_compose():
     meta, arrays, _, _ = _problem("two_64x256")
     for nc in (5, 2500, 20011):
         th0 = 0.01 * np.random.default_rng(nc).standard_normal((nc, 64))
-        a = _ens(meta, arrays, nc, seed=2)
+        a = ensemble(meta, arrays, nc, seed=2)
         a.set_state(th0)
         whole = a.run(6, samples=True, accepted=True, logpost=True)
-        b = _ens(meta, arrays, nc, seed=2)
+        b = ensemble(meta, arrays, nc, seed=2)
         b.set_state(th0)
         parts = [b.run(k, samples=True, accepted=True, logpost=True) for k in (1, 2, 3)]
         for k in ("samples", "accepted", "logpost"):
@@ -208,11 +190,11 @@ def test_streamed_two_level_posterior_moments():
     mean, cov = bp.linear_gaussian_posterior(arrays, 1)
     C = 4096
     th0 = np.random.default_rng(19).multivariate_normal(mean, cov, size=C)
-    ens = _ens(meta, arrays, C, seed=8)
+    ens = ensemble(meta, arrays, C, seed=8)
     ens.set_state(th0)
     s = ens.run(2000, thin=20, samples=True)["samples"].cpu().numpy()     # [100, d, C]
     flat = s.transpose(0, 2, 1).reshape(-1, 64)
-    _check_closed_form(dict(mean=flat.mean(0), covariance=np.cov(flat.T)), mean, cov, C, "two_64x256")
+    check_closed_form(dict(mean=flat.mean(0), covariance=np.cov(flat.T)), mean, cov, C, "two_64x256")
     c = ens.counters()
     assert 0.05 < c["accepted"] / c["transitions"] < 0.95 and c["fine_evals"] < c["coarse_evals"]
 
@@ -222,7 +204,7 @@ def test_streamed_pooled_factor_through_the_builders():
     to the dense factor, whose blob no longer fits (its rebuild was refused while it had to) and streams level 1's G;
     the run after it samples the posterior and replays through the oracle."""
     C, thin = 4096, 10
-    mc, (mean, cov) = _linear_chain(64, 160, True, C, seed=5, thin=thin)
+    mc, (mean, cov) = linear_chain(64, 160, True, C, seed=5, thin=thin)
     draws = np.random.default_rng(23).multivariate_normal(mean, cov, size=C)
     mc.run(501, ParameterVector(draws), verbose=False)
     pooled = mc.pool_proposal_covariance()
@@ -232,14 +214,14 @@ def test_streamed_pooled_factor_through_the_builders():
     assert stream == 1
     mc.run(1001, ParameterVector(draws), verbose=False)
     assert ens.last_launch()["smem"] == smem and ens.last_launch()["block"] == 32 * warps
-    _check_closed_form(mc.pooled(), mean, cov, C, "pooled dense factor")
+    check_closed_form(mc.pooled(), mean, cov, C, "pooled dense factor")
     # a short recorded run on the pooled factor, replayed through the oracle
     th0 = ens.state()["theta"].cpu().numpy().T.copy()
     out = ens.run(4, samples=True, accepted=True, logpost=True, record=True)
     torch.cuda.synchronize()
     p = ens.problem
     meta = dict(model=p.model, dim=p.dim, levels=p.levels, J=p.J, eq=p.eq)
-    ref = _replay(meta, p.arrays, th0, out)
+    ref = replay(meta, p.arrays, th0, out)
     assert np.array_equal(out["accepted"].cpu().numpy().T, ref["accepted"])
     assert traj_err(out["samples"].cpu().numpy().transpose(2, 0, 1), ref["traj"][:, 1:], True) <= 1e-12
     lp = out["logpost"].cpu().numpy().transpose(2, 0, 1)
@@ -260,7 +242,7 @@ def test_every_envelope_problem_is_accepted():
                     if dense_prior:
                         for l in range(meta["levels"]):
                             arrays[f"L{l}_prior_prec"] = 0.5 * np.eye(d) + 0.01
-                    ens = _ens(meta, arrays, 17, seed=1)
+                    ens = ensemble(meta, arrays, 17, seed=1)
                     ens.set_state(np.zeros((17, d)))
                     ens.run(2, samples=False)
                     ens.close()
