@@ -152,6 +152,87 @@ SCHEDULES = {
 }
 
 
+def aem_problem(d, dd, n_data, J, min_data, heuristic, dense_prop=False, dense_prior=False, zero_error_rows=0,
+                seed=0, error_scale=1.0, spread=1.5, prop_scale=2.4, eq="exact"):
+    """Two-level linear model for the adaptive error model, d parameters and dd data components, diagonal noise.
+    The coarse model is the fine one with row k of G and b perturbed at a scale error_scale x noise sd x 10^(spread
+    (k / (dd - 1) - 1)) (so the error variances span 2 spread decades: the heuristic clamps when that ratio passes 50);
+    the last zero_error_rows rows are left identical to the fine level's, so those error components are exactly 0.
+    The proposal is prop_scale / sqrt(d) times the fine posterior's Cholesky factor (dense_prop) or its marginal sds."""
+    rng = np.random.default_rng(seed)
+    truth = rng.standard_normal(d)
+    G_f = rng.standard_normal((dd, d)) / np.sqrt(d)
+    b_f = 0.1 * rng.standard_normal(dd)
+    sd = 0.1 * (1.0 + 0.5 * np.arange(dd) / dd)
+    scale = error_scale * sd * 10.0 ** (spread * (np.arange(dd) / max(dd - 1, 1) - 1.0))
+    G_c = G_f + scale[:, None] * rng.standard_normal((dd, d))
+    b_c = b_f + scale * rng.standard_normal(dd)
+    if zero_error_rows:
+        G_c[dd - zero_error_rows:], b_c[dd - zero_error_rows:] = G_f[dd - zero_error_rows:], b_f[dd - zero_error_rows:]
+    data = truth @ G_f.T + b_f + sd * rng.standard_normal((n_data, dd))
+    prior_prec = np.eye(d) / 4.0
+    if dense_prior:
+        A = rng.standard_normal((d, d))
+        prior_prec = np.linalg.inv(A @ A.T / d + np.eye(d))
+        prior_prec = 0.5 * (prior_prec + prior_prec.T)
+    prior_mean = truth + 0.3 * rng.standard_normal(d)
+    arrays = {}
+    for l, (G, b) in enumerate(((G_c, b_c), (G_f, b_f))):
+        arrays.update({f"L{l}_G": G, f"L{l}_b": b, f"L{l}_data": data, f"L{l}_noise_prec": np.diag(1.0 / sd ** 2),
+                       f"L{l}_prior_mean": prior_mean, f"L{l}_prior_prec": prior_prec})
+    _, cov = bp.linear_gaussian_posterior(arrays, 1)
+    arrays["prop_L"] = prop_scale / np.sqrt(d) * (np.linalg.cholesky(cov) if dense_prop else np.diag(np.sqrt(np.diag(cov))))
+    meta = dict(model="linear", dim=d, levels=2, J=J, eq=eq, aem=dict(min_data=min_data, heuristic=bool(heuristic)))
+    return meta, arrays
+
+
+def aem_start(arrays, nc, seed):
+    """nc initial states drawn from the fine level's posterior."""
+    mean, cov = bp.linear_gaussian_posterior(arrays, 1)
+    return mean + np.random.default_rng(seed).standard_normal((nc, mean.size)) @ np.linalg.cholesky(cov).T
+
+
+# The AEM value sweep: every (capacity(d), capacity(data_dim)) pair of aem_mh_kernel<D, DD> once.
+# name: (aem_problem kwargs, chains, steps, thin)
+AEM_SWEEP = {
+    "1x1": (dict(d=1, dd=1, n_data=129, J=1, min_data=8, heuristic=True, seed=1), 1, 60, 1),
+    "1x3": (dict(d=1, dd=3, n_data=9, J=5, min_data=2, heuristic=True, seed=2), 33, 40, 1),
+    "2x8": (dict(d=2, dd=8, n_data=2, J=2, min_data=3, heuristic=False, zero_error_rows=2, error_scale=0.3, seed=3),
+            4097, 24, 1),
+    "3x2": (dict(d=3, dd=2, n_data=1, J=5, min_data=3, heuristic=True, dense_prop=True, seed=4), 33, 42, 3),
+    "3x3": (dict(d=3, dd=3, n_data=129, J=1, min_data=8, heuristic=False, error_scale=0.1, prop_scale=0.5, seed=5),
+            33, 50, 1),
+    "3x5": (dict(d=3, dd=5, n_data=9, J=2, min_data=2, heuristic=True, zero_error_rows=1, dense_prior=True, seed=6),
+            4097, 24, 1),
+    "5x1": (dict(d=5, dd=1, n_data=2, J=2, min_data=3, heuristic=True, dense_prop=True, dense_prior=True, seed=7),
+            1, 60, 1),
+    "8x3": (dict(d=8, dd=3, n_data=9, J=5, min_data=2, heuristic=True, dense_prop=True, error_scale=0.1, prop_scale=0.5,
+                seed=8), 33, 40, 1),
+    "8x8": (dict(d=8, dd=8, n_data=129, J=2, min_data=8, heuristic=True, zero_error_rows=3, error_scale=0.1,
+                prop_scale=0.5, seed=9), 33, 40, 1),
+}
+
+# Forced-decision cases, at least one per parameter capacity: the heuristic floors without clamping (d2_floor),
+# clamps (d4_clamp) and neither (d8_one_component: one data component, scaling 2).  name: (kwargs, chains, steps)
+AEM_FORCED = {
+    "d2_floor": (dict(d=2, dd=3, n_data=9, J=5, min_data=3, heuristic=True, zero_error_rows=1, error_scale=0.02,
+                      spread=0.0, seed=11), 64, 40),
+    "d4_clamp": (dict(d=3, dd=4, n_data=2, J=3, min_data=2, heuristic=True, seed=12), 64, 40),
+    "d8_one_component": (dict(d=6, dd=1, n_data=129, J=2, min_data=8, heuristic=True, dense_prop=True, seed=13), 64, 40),
+    "d8_no_heuristic": (dict(d=8, dd=5, n_data=9, J=5, min_data=3, heuristic=False, zero_error_rows=1, seed=14), 64, 40),
+}
+
+
+def aem_forced_inputs(name, seed=0):
+    """(meta, arrays, theta0, z, pattern) of an AEM_FORCED case."""
+    kw, nc, ns = AEM_FORCED[name]
+    meta, arrays = aem_problem(**kw)
+    th0 = aem_start(arrays, nc, kw["seed"] + 100 + seed)
+    z = schedule_noise(meta, nc, ns, kw["seed"] + 200 + seed)
+    pattern = R.random_pattern(nc, ns, meta["J"], kw["seed"] + 300 + seed)
+    return meta, arrays, th0, z, pattern
+
+
 def schedule_noise(meta, nc, ns, seed):
     J = int(meta["J"]) if int(meta["levels"]) >= 2 else 1
     return np.random.default_rng(seed).standard_normal((nc, ns, J, int(meta["dim"])))

@@ -546,6 +546,11 @@ int build_blob(const yg_config &c, const yg_problem *pb, std::vector<char> &blob
             yg_set_error("adaptive error model: both levels must share the data dimension (MRW proposal)");
             return YG_ERR_INVALID;
         }
+        if (Lc.tempered && Lc.tempering != 1.0) {
+            // the error model's coarse log-posterior has no tempering factor (likelihood.py:74-84,140-145)
+            yg_set_error("adaptive error model: a tempered level 0 (tempering %g) is not supported", Lc.tempering);
+            return YG_ERR_UNSUPPORTED;
+        }
         for (int i = 0; i < Lc.data_dim; i++)
             for (int j = 0; j < Lc.data_dim; j++)
                 if (i != j && Lc.noise_prec[i * Lc.data_dim + j] != 0.0) {

@@ -541,6 +541,9 @@ __global__ void __launch_bounds__(WS ? WS_THREADS : 128) generic_mh_kernel(const
 // likelihood's LRU(3) cache is reproduced entry for entry, because the reference does NOT
 // invalidate cached log-likelihoods when the error model changes: which value a chain sees for
 // pi_c(state) depends on whether the state is still among the last three parameters queried.
+// ISCLOSE: proposals of a scalar chain are compared with math.isclose (parameter/scalar.py:38-43); a
+// separate instance, launched only for eq_mode == YG_EQ_ISCLOSE (d = 1, capacity 2), so that the
+// exact-equality instances compile as if the rule did not exist.  The cache keys stay exact.
 // ---------------------------------------------------------------------------------------------
 template <int D>
 struct Lru3 {
@@ -601,7 +604,7 @@ YG_DEVFN void lru_add(Lru3<D> &c, const double (&x)[D], double v)
     c.n++;
 }
 
-template <int D, int DD>
+template <int D, int DD, bool ISCLOSE>
 __global__ void __launch_bounds__(128) aem_mh_kernel(const RunArgs a)
 {
     extern __shared__ __align__(16) unsigned char smem_raw[];
@@ -761,6 +764,7 @@ __global__ void __launch_bounds__(128) aem_mh_kernel(const RunArgs a)
             }
         };
         auto equal = [&](const double (&p)[D], const double (&s)[D]) {
+            if (ISCLOSE) return isclose_rule(p[0], s[0]);
             bool eq = true;
 #pragma unroll
             for (int i = 0; i < D; i++)
@@ -911,7 +915,10 @@ int launch_aem_t(yg_ensemble *e, const RunArgs &a, cudaStream_t st)
     const int64_t want = (a.n_chains + threads - 1) / threads;
     const int grid = (int)std::max<int64_t>(1, std::min<int64_t>(want, (int64_t)e->sm_count * 16));
     const size_t smem = (e->h_problem.size() + 15) & ~size_t(15);
-    auto kern = aem_mh_kernel<D, DD>;
+    auto kern = aem_mh_kernel<D, DD, false>;
+    if constexpr (D == 2) {                                   // abi.cu: isclose needs d = 1
+        if (e->cfg.eq_mode == YG_EQ_ISCLOSE) kern = aem_mh_kernel<2, DD, true>;
+    }
     YG_CUDA_CHECK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     kern<<<grid, threads, smem, st>>>(a);
     YG_CUDA_CHECK(cudaGetLastError());
