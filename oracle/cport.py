@@ -83,7 +83,7 @@ class Problem:
             pb.adaptive = 1
             pb.am_idle = int(adaptive.get('idle', 0))
             pb.am_collect = int(adaptive.get('collection', 100))
-            pb.am_refresh = int(adaptive.get('refresh', 1))
+            pb.am_refresh = max(1, int(adaptive.get('refresh', 1)))      # abi.cu make_args: 0 refreshes every step
             pb.am_eps = float(adaptive.get('eps', 1e-4))
             sc = float(adaptive.get('scale') or 0.0)
             pb.am_scale = sc if sc > 0 else 2.4 * 2.4 / int(meta['dim'])

@@ -432,19 +432,21 @@ def _eval(meta, arrays, level, theta, path, n_moves):
     return lp, b
 
 
-def _propose(meta, arrays, s, z):
-    """propose() of the oracle in double: p = s + L z, or pCN's sqrt(1 - 2h) s + sqrt(2h) (m + L z)."""
-    Lp = np.asarray(arrays["prop_L"], dtype=np.float64)
+def _propose(meta, arrays, s, z, L=None):
+    """propose() of the oracle in double: p = s + L z, or pCN's sqrt(1 - 2h) s + sqrt(2h) (m + L z).  L: the problem's
+    factor by default, or one factor per chain [nc, d, d] (adaptive Metropolis); an exact zero of L is skipped, per
+    chain, as the oracle and the kernels skip it."""
+    Lp = np.asarray(arrays["prop_L"] if L is None else L, dtype=np.float64)
     d = s.shape[1]
     acc = np.zeros_like(s)
     for i in range(d):
-        first = True
+        first = np.ones(s.shape[0], dtype=bool)
         for j in range(i + 1):
-            l = Lp[i, j]
-            if l != 0.0 or j == i:
-                t = l * z[:, j]
-                acc[:, i] = t if first else acc[:, i] + t
-                first = False
+            l = Lp[..., i, j]
+            use = (l != 0.0) | (j == i)
+            t = l * z[:, j]
+            acc[:, i] = np.where(use & first, t, np.where(use, acc[:, i] + t, acc[:, i]))
+            first &= ~use
     if meta.get("proposal", "mrw") == "pcn":
         tt = 2.0 * float(meta["pcn_step"])
         a, b = np.sqrt(1.0 - tt), np.sqrt(tt)
@@ -496,7 +498,20 @@ def _decide(delta, err, want, eta, exact_eta):
     return u, out, e_used
 
 
-def forced_schedule(meta, arrays, theta0, z, pattern, eta, exact_eta=False):
+def _follow(delta, err, u):
+    """accept_rule on given uniforms, in long double: u <= min(exp(delta), 1), a NaN delta accepting.  Returns
+    (u, decision, margin): margin = |delta - log u| - err - 8 u (exp's rounding), > 0 where any double-precision
+    evaluation within err of delta decides the same way."""
+    with np.errstate(over='ignore', divide='ignore', invalid='ignore'):
+        dl = np.asarray(delta, dtype=LD)
+        a = np.exp(dl)
+        dec = ~(a < 1) | (np.asarray(u, dtype=LD) <= a)
+        m = np.asarray(np.abs(dl - np.log(np.asarray(u, dtype=LD))), dtype=np.float64) - err - 8.0 * U
+    m = np.where(np.isnan(m) & np.isnan(np.asarray(delta, dtype=np.float64)), np.inf, m)
+    return np.asarray(u, dtype=np.float64), dec, m
+
+
+def forced_schedule(meta, arrays, theta0, z, pattern, eta, exact_eta=False, factor=None, uniforms=None):
     """Simulates chain_step (oracle/yagre_oracle.c: MRW / pCN, two-level delayed acceptance, MLDA with two surrogates)
     in long double on the noise z [nc, ns, J, d] and returns uniforms that force the decisions of `pattern`.
 
@@ -504,10 +519,16 @@ def forced_schedule(meta, arrays, theta0, z, pattern, eta, exact_eta=False):
     eta: the distance of each uniform from its threshold in log space, at least ETA_FACTOR x the bound on the error of
     that delta (the terms' logpost_bound plus the trajectory term of _eval) -- pass 0 for the smallest allowed.
     exact_eta: use eta as given even below that bound (then no decision is certain; for on / off comparisons only).
+    factor: optional per-chain proposal-factor hook, factor(n, j, s) -> L [nc, d, d], called before each proposal
+    (transition n, sub-step j, 0 for one level) with the current (sub-)chain state s [nc, d]: adaptive Metropolis.
+    uniforms: optional dict(u_c, u_f): decide by these uniforms and the long-double deltas instead of placing
+    uniforms (a run playing a kernel on given noise; pattern and eta are ignored).  Then margin_min is the smallest
+    margin of a decision beyond its bound (_follow; > 0: every decision is certain).
 
     Returns dict(u_c [nc, ns, J], u_f [nc, ns], accepted uint8 [nc, ns], coarse_accepted int64 [nc],
     n_accept int64 [nc], evals [3] (as counted by the oracle, without the initial ones), eta_min (smallest eta used
-    at a decision that could go either way), coarse / fine: the decisions actually forced).  Raises Undecidable."""
+    at a decision that could go either way), coarse / fine: the decisions actually forced, traj [nc, ns, d]: the
+    state after each transition, theta: the last one).  Raises Undecidable."""
     levels = int(meta["levels"])
     J = int(meta["J"]) if levels >= 2 else 1
     theta = np.array(theta0, dtype=np.float64)
@@ -525,7 +546,8 @@ def forced_schedule(meta, arrays, theta0, z, pattern, eta, exact_eta=False):
     cacc = np.zeros(nc, dtype=np.int64)
     evals = np.zeros(3, dtype=np.int64)
     coarse_forced = np.zeros((nc, ns, J), dtype=bool)
-    eta_min = np.inf
+    traj = np.zeros((nc, ns, d))
+    eta_min = margin_min = np.inf
     moves = 0
 
     def track(e, dlt):
@@ -534,17 +556,29 @@ def forced_schedule(meta, arrays, theta0, z, pattern, eta, exact_eta=False):
         if fin.any():
             eta_min = min(eta_min, float(e[fin].min()))
 
+    def decide(delta, err, which, idx, live):
+        nonlocal margin_min
+        if uniforms is None:
+            return _decide(delta, err, pattern[which][idx], eta, exact_eta)
+        u, dec, m = _follow(delta, err, uniforms["u_c" if which == "coarse" else "u_f"][idx])
+        if live.any():
+            margin_min = min(margin_min, float(m[live].min()))
+        return u, dec, np.full(nc, np.inf)
+
+    def propose(s, n, j):
+        return _propose(meta, arrays, s, z[:, n, j], None if factor is None else factor(n, j, s))
+
     for n in range(ns):
         if levels == 1:
             moves += 1
-            p = _propose(meta, arrays, theta, z[:, n, 0])
+            p = propose(theta, n, 0)
             eq = _equal(meta, p, theta)
             lpp, bp = _eval(meta, arrays, 0, p, path, moves)
             evals[0] += int((~eq).sum())
             with np.errstate(invalid='ignore'):
                 delta = lpp - lpt[0]
-            u, dec, e = _decide(delta, bp + bt[0] + U * np.abs(np.asarray(delta, dtype=np.float64)),
-                                pattern["fine"][:, n], eta, exact_eta)
+            u, dec, e = decide(delta, bp + bt[0] + U * np.abs(np.asarray(delta, dtype=np.float64)),
+                               "fine", (slice(None), n), ~eq)
             dec &= ~eq
             track(e[~eq], delta[~eq])
             u_f[:, n] = u
@@ -552,18 +586,19 @@ def forced_schedule(meta, arrays, theta0, z, pattern, eta, exact_eta=False):
             theta = np.where(dec[:, None], p, theta)
             lpt[0] = np.where(dec, lpp, lpt[0])
             bt[0] = np.where(dec, bp, bt[0])
+            traj[:, n] = theta
             continue
         s, lpc, bc = theta.copy(), lpt[0].copy(), bt[0].copy()
         for j in range(J):
             moves += 1
-            p = _propose(meta, arrays, s, z[:, n, j])
+            p = propose(s, n, j)
             eq = _equal(meta, p, s)
             lpp, bp = _eval(meta, arrays, 0, p, path, moves)
             evals[0] += int((~eq).sum())
             with np.errstate(invalid='ignore'):
                 delta = lpp - lpc
-            u, dec, e = _decide(delta, bp + bc + U * np.abs(np.asarray(delta, dtype=np.float64)),
-                                pattern["coarse"][:, n, j], eta, exact_eta)
+            u, dec, e = decide(delta, bp + bc + U * np.abs(np.asarray(delta, dtype=np.float64)),
+                               "coarse", (slice(None), n, j), ~eq)
             dec &= ~eq
             track(e[~eq], delta[~eq])
             u_c[:, n, j] = u
@@ -589,7 +624,7 @@ def forced_schedule(meta, arrays, theta0, z, pattern, eta, exact_eta=False):
             delta = ((terms[0] + terms[1]) + terms[2]) + terms[3]
             mag = sum(np.abs(np.asarray(t, dtype=np.float64)) for t in terms)
         mag = np.where(np.isfinite(mag), mag, 0.0)
-        u, dec, e = _decide(delta, bsum + 3.0 * U * mag, pattern["fine"][:, n], eta, exact_eta)
+        u, dec, e = decide(delta, bsum + 3.0 * U * mag, "fine", (slice(None), n), moved)
         dec &= moved
         track(e[moved], delta[moved])
         u_f[:, n] = u
@@ -602,8 +637,9 @@ def forced_schedule(meta, arrays, theta0, z, pattern, eta, exact_eta=False):
         if levels == 3:
             lpt[1] = np.where(dec, lpm, lpt[1])
             bt[1] = np.where(dec, bm, bt[1])
+        traj[:, n] = theta
     return dict(u_c=u_c, u_f=u_f, accepted=acc, coarse_accepted=cacc, n_accept=acc.sum(axis=1, dtype=np.int64),
-                evals=evals, eta_min=eta_min, coarse=coarse_forced, theta=theta)
+                evals=evals, eta_min=eta_min, margin_min=margin_min, coarse=coarse_forced, traj=traj, theta=theta)
 
 
 def random_pattern(nc, ns, J, seed, p=0.5):

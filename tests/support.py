@@ -432,3 +432,114 @@ def check_closed_form(out, mean, cov, C, label):
     dg = np.diag(cov)
     sc = np.sqrt((np.outer(dg, dg) + cov ** 2) / C)
     assert np.all(np.abs(out["covariance"] - cov) <= 5 * sc), (label, "covariance", (np.abs(out["covariance"] - cov) / sc).max())
+
+
+# ------------------------------------------------------------------------------------------------------------------
+# adaptive Metropolis (test_am_reference_cpu, test_am_reference_gpu)
+# ------------------------------------------------------------------------------------------------------------------
+def am_problem(d, dd=2, levels=1, J=3, n_data=4, offset=0.0, spread=0.3, frozen=None, prop_scale=1.0, seed=0):
+    """Linear model G theta + b with d parameters and dd data components, one level or two (level 0 the fine model
+    with G and b perturbed by 5 %).  The posterior sits near `offset` (every coordinate) with spreads of about
+    `spread`; the proposal factor is prop_scale x spread x a random lower-triangular matrix with unit diagonal, with
+    row `frozen` (if given) exactly zero: that coordinate never moves while the chain runs on this factor."""
+    rng = np.random.default_rng(seed)
+    truth = offset + spread * rng.standard_normal(d)
+    G = rng.standard_normal((dd, d)) / np.sqrt(d)
+    b = 0.1 * rng.standard_normal(dd)
+    data = truth @ G.T + b + spread * rng.standard_normal((n_data, dd))
+    fine = dict(G=G, b=b)
+    coarse = dict(G=G * (1.0 + 0.05 * rng.standard_normal(G.shape)), b=b + 0.05 * spread * rng.standard_normal(dd))
+    arrays = {}
+    for l, lv in enumerate([coarse, fine] if levels == 2 else [fine]):
+        arrays.update({f"L{l}_G": lv["G"], f"L{l}_b": lv["b"], f"L{l}_data": data,
+                       f"L{l}_noise_prec": np.eye(dd) / spread ** 2,
+                       f"L{l}_prior_mean": truth + spread * rng.standard_normal(d),
+                       f"L{l}_prior_prec": np.eye(d) / (10.0 * spread) ** 2})
+    L = np.tril(0.3 * rng.standard_normal((d, d)), -1) + np.eye(d)
+    if frozen is not None:
+        L[frozen] = 0.0
+    arrays["prop_L"] = prop_scale * spread * L
+    meta = dict(model="linear", dim=d, levels=levels, J=J if levels == 2 else 1, eq="exact")
+    return meta, arrays
+
+
+def am_start(meta, arrays, nc, seed):
+    """nc initial states near the level-0 prior mean (a spread of a tenth of the proposal's)."""
+    m = np.asarray(arrays["L0_prior_mean"], dtype=np.float64)
+    sd = np.abs(np.diag(np.asarray(arrays["prop_L"]))).max() * 0.1 if m.size else 0.0
+    return m + sd * np.random.default_rng(seed).standard_normal((nc, m.size))
+
+
+def _am_lv(levels, frozen=None):
+    meta, arrays = bp.lv_problem(levels == 2)
+    if frozen is not None:
+        L = np.array(arrays["prop_L"], dtype=np.float64)
+        L[frozen] = 0.0
+        arrays = dict(arrays, prop_L=L)
+    return meta, arrays
+
+
+# The AM value sweep: each case runs at one and at two levels (J from the kwargs), so together they cover every
+# generic_mh_kernel<D, DD, TWO_LEVEL> instance that carries AM; the d = 2 cases run the warp-specialised instance under
+# Philox noise.  name: (am_problem kwargs, adaptive, chains, steps)
+AM_SWEEP = {
+    "2x2": (dict(d=2, dd=2, J=3, seed=1), dict(idle=0, collection=2, refresh=1, eps=1e-4), 64, 24),
+    "2x4": (dict(d=2, dd=3, J=2, seed=2, offset=1e4, spread=1e-3), dict(idle=3, collection=4, refresh=3, eps=1e-9,
+                                                                         scale=0.8), 64, 24),
+    "2x8": (dict(d=2, dd=7, J=2, seed=3), dict(idle=0, collection=1, refresh=0, eps=1e-5), 64, 24),
+    "3x2": (dict(d=3, dd=1, J=3, seed=4), dict(idle=1, collection=5, refresh=2, eps=1e-4), 64, 24),
+    "4x4": (dict(d=4, dd=4, J=2, seed=5), dict(idle=0, collection=3, refresh=1, eps=1e-4, scale=0.5), 64, 24),
+    "3x8": (dict(d=3, dd=6, J=2, seed=6), dict(idle=2, collection=0, refresh=3, eps=1e-4), 64, 24),
+    "5x2": (dict(d=5, dd=2, J=2, seed=7, frozen=2), dict(idle=0, collection=2, refresh=1, eps=1e-4), 64, 24),
+    "8x4": (dict(d=8, dd=3, J=2, seed=8), dict(idle=0, collection=2, refresh=1, eps=1e-4), 64, 24),
+    "8x8": (dict(d=8, dd=8, J=3, seed=9, offset=1e4, spread=1e-3), dict(idle=4, collection=6, refresh=2, eps=1e-9),
+            64, 24),
+}
+
+LAUNCHES = (1, 2, 5)        # the first launches of every forced case; the rest of the steps make the last one
+
+# Forced-decision cases.  name: (problem builder, adaptive, chains, steps, all-rejected chains, forced first accepts)
+# All-rejected chains get noise 1e3 times larger (every proposal lands far in the tail) and a pattern of rejections;
+# with eps = 0 the moving chains accept their first proposals, so that the first refresh sees d + 1 distinct states.
+AM_FORCED = {
+    "d2_collect0_rejected": (lambda: am_problem(2, dd=1, seed=21), dict(idle=0, collection=0, refresh=1, eps=1e-3),
+                             48, 30, 8, 0),
+    "d3_two_level_refresh3": (lambda: am_problem(3, dd=3, levels=2, J=3, seed=22),
+                              dict(idle=4, collection=5, refresh=3, eps=1e-4), 32, 16, 0, 0),
+    "d5_frozen_eps0": (lambda: am_problem(5, dd=6, frozen=4, seed=23), dict(idle=2, collection=8, refresh=0, eps=0.0),
+                       32, 24, 0, 0),
+    "d4_offset_eps0_rejected": (lambda: am_problem(4, dd=2, offset=1e4, spread=1e-3, seed=24),
+                                dict(idle=1, collection=12, refresh=1, eps=0.0, scale=0.5), 48, 30, 8, 8),
+    "d8_two_level_frozen": (lambda: am_problem(8, dd=3, levels=2, J=2, frozen=2, seed=25),
+                            dict(idle=0, collection=1, refresh=1, eps=1e-4, scale=0.3), 32, 20, 0, 0),
+    "lv_two_level": (lambda: _am_lv(2), dict(idle=0, collection=2, refresh=3, eps=1e-6), 16, 8, 0, 0),
+    "lv_one_level_frozen": (lambda: _am_lv(1, frozen=1), dict(idle=0, collection=3, refresh=1, eps=0.0), 16, 12, 0, 0),
+    "gauss_three_level": (three_level_gauss, dict(idle=3, collection=4, refresh=2, eps=1e-5), 32, 8, 0, 0),
+}
+
+
+def am_launches(ns):
+    return list(LAUNCHES) + [ns - sum(LAUNCHES)]
+
+
+def am_forced_inputs(name, seed=0):
+    """(meta, arrays, adaptive, theta0, z, pattern, launches) of an AM_FORCED case."""
+    make, adaptive, nc, ns, n_rej, n_first = AM_FORCED[name]
+    meta, arrays = make()
+    if meta["model"] == "lv":
+        th0 = bp.lv_initial_states(nc, seed=31 + seed)
+    elif meta["model"] == "gauss":
+        th0 = np.tile([0.5, 1.0], (nc, 1)) + 0.01 * np.random.default_rng(31 + seed).standard_normal((nc, 2))
+    else:
+        th0 = am_start(meta, arrays, nc, 31 + seed)
+    z = schedule_noise(meta, nc, ns, 41 + seed)
+    J = z.shape[2]
+    pattern = R.random_pattern(nc, ns, J, 51 + seed)
+    if n_rej:
+        z[:n_rej] *= 1e3
+        pattern["coarse"][:n_rej] = False
+        pattern["fine"][:n_rej] = False
+    if n_first:
+        pattern["coarse"][n_rej:, :n_first] = True
+        pattern["fine"][n_rej:, :n_first] = True
+    return meta, arrays, adaptive, th0, z, pattern, am_launches(ns)

@@ -3,6 +3,7 @@
 #include "ensemble.h"
 #include "big_linear.h"
 #include "smem_plan.h"
+#include <cmath>
 #include <cstdarg>
 #include <cstdio>
 #include <cstring>
@@ -388,6 +389,13 @@ extern "C" int yg_create(const yg_config *cfg, yg_ensemble **out)
     }
     if (cfg->adaptive && (cfg->am_idle_steps < 0 || cfg->am_collection_steps < 0 || cfg->am_refresh < 0)) {
         yg_set_error("adaptive Metropolis: idle / collection steps and the refresh interval must be >= 0");
+        return YG_ERR_INVALID;
+    }
+    // the builder's rule (AMBuilder.regularisationParameter: eps >= 0); a NaN eps or scale would make every refresh
+    // fail, and the chain would silently never adapt.  A scale <= 0 selects the default 2.4^2 / d (make_args).
+    if (cfg->adaptive && (!std::isfinite(cfg->am_eps) || cfg->am_eps < 0.0 || !std::isfinite(cfg->am_scale))) {
+        yg_set_error("adaptive Metropolis: the regularisation eps must be finite and >= 0, and the scale finite "
+                     "(eps=%g, scale=%g)", cfg->am_eps, cfg->am_scale);
         return YG_ERR_INVALID;
     }
     if (cfg->aem) {
