@@ -143,6 +143,43 @@ def big_linear_problem(d=64, data_dim=256, n_data=1, two_level=False, J=2, seed=
     return meta, arrays
 
 
+def big_linear_three_level_problem(d=64, data_dims=(256, 256, 256), n_data=1, J=3, tempering=None, dense_prior=False,
+                                   seed=3, prop_var=None):
+    """MLDA with two surrogates on a GEMM-sized linear model: one smooth operator observed on three grids, level l on
+    data_dims[l] points (coarse, medium, fine; the fine level is the target).  G_l[i, k] = cos(pi (k + 1) x_i + phi_k)
+    sqrt(2 / d) at the grid points x_i of level l, the surrogates' operators perturbed by 5 % and 2 %, one truth,
+    data per level, diagonal noise.  tempering: {level: t} (TemperedUnnormalisedPosterior); dense_prior: a dense prior
+    precision shared by the levels.  The proposal is diagonal."""
+    rng = Generator(Philox(seed))
+    phase = rng.uniform(0.0, np.pi, d)
+    truth = rng.standard_normal(d)
+    noise_var, prior_var = 0.05, 2.0
+    prior_prec = _diag_prec(prior_var, d)
+    prior_mean = np.zeros(d)
+    if dense_prior:
+        A = rng.standard_normal((d, d))
+        cov = prior_var * (A @ A.T / d + 0.5 * np.eye(d))
+        prior_prec = np.linalg.inv(cov)
+        prior_prec = 0.5 * (prior_prec + prior_prec.T)
+        prior_mean = 0.1 * rng.standard_normal(d)
+    arrays = {}
+    for l, (dd, pert) in enumerate(zip(data_dims, (0.05, 0.02, 0.0))):
+        x = (np.arange(dd) + 0.5) / dd
+        G = np.cos(np.pi * np.outer(x, np.arange(1, d + 1)) + phase) * np.sqrt(2.0 / d)
+        G = G + pert * rng.standard_normal((dd, d)) / np.sqrt(d)
+        b = 0.1 * np.sin(2.0 * np.pi * x) + pert * rng.standard_normal(dd)
+        data = np.array([G @ truth + b + np.sqrt(noise_var) * rng.standard_normal(dd) for _ in range(n_data)])
+        arrays.update({f"L{l}_G": G, f"L{l}_b": b, f"L{l}_data": data, f"L{l}_noise_prec": _diag_prec(noise_var, dd),
+                       f"L{l}_prior_mean": prior_mean, f"L{l}_prior_prec": prior_prec})
+    for l, t in (tempering or {}).items():
+        arrays[f"L{l}_tempering"] = np.array(float(t))
+    if prop_var is None:
+        prop_var = 2.4 ** 2 / d * noise_var / max(n_data * data_dims[0] / d, 1.0)
+    arrays["prop_L"] = _iid_L(prop_var, d)
+    meta = dict(model='linear', dim=d, levels=3, J=J, eq='exact', truth=truth.tolist())
+    return meta, arrays
+
+
 def linear_gaussian_posterior(arrays, level):
     """Closed-form Gaussian posterior (mean, covariance) of one level of a lowered linear problem."""
     pre = f"L{level}_"

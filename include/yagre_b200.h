@@ -73,11 +73,12 @@ extern "C" {
 #define YG_MAX_LEVELS 3         /* densities per problem: up to two surrogates + the target */
 #define YG_MAX_DIM 8           /* parameter dimension of the one-chain-per-thread kernels */
 #define YG_MAX_DATA_DIM 8
-/* YG_MODEL_LINEAR beyond those sizes runs on the FP64 tensor path (DMMA GEMM, linear_dmma_kernel.cu): MRW, pCN and
- * two-level delayed acceptance; diagonal measurement noise; diagonal or dense prior precision and proposal factor;
- * every combination up to YG_BIG_MAX_DIM x YG_BIG_MAX_DATA_DIM (an operand that does not fit shared memory -- level
- * 1's G, then the dense factor -- is read from L2; rates measured on a B200 in profiles/streamed_operand.md);
- * no adaptive Metropolis / adaptive error model / third level / tempering;
+/* YG_MODEL_LINEAR beyond those sizes runs on the FP64 tensor path (DMMA GEMM, linear_dmma_kernel.cu): MRW, pCN,
+ * two-level delayed acceptance and MLDA with two surrogates, tempered levels; diagonal measurement noise; diagonal or
+ * dense prior precision and proposal factor; every combination up to YG_BIG_MAX_DIM x YG_BIG_MAX_DATA_DIM per level (an
+ * operand that does not fit shared memory -- level 1's G, level 2's G, then the dense factor -- is read from L2; rates
+ * measured on a B200 in profiles/streamed_operand.md and profiles/three_level_tensor.md);
+ * no adaptive Metropolis / adaptive error model;
  * Welford M2 is then diagonal only ([d, n_chains] instead of [d, d, n_chains]). */
 #define YG_BIG_MAX_DIM 64
 #define YG_BIG_MAX_DATA_DIM 256
@@ -117,7 +118,7 @@ typedef struct yg_level {
     double alpha, gamma, T;
     int32_t rk4_steps;
     /* TemperedUnnormalisedPosterior (chain/target.py:25-43): tempering * logL + logprior when tempered != 0
-     * (regression levels of the one-chain-per-thread and LV kernels; tempering in [0, 1]) */
+     * (regression levels of every kernel; tempering in [0, 1]) */
     int32_t tempered;
     double tempering;
 } yg_level;

@@ -188,27 +188,30 @@ bool is_diagonal(const double *M, int n)
 int build_big_blob(const yg_config &c, const yg_problem *pb, std::vector<char> &blob)
 {
     const int d = c.dim, nl = c.n_levels;
-    if (c.adaptive || c.eq_mode != YG_EQ_EXACT || c.aem || nl > 2) {
-        yg_set_error("large linear model (dim > %d or data_dim > %d): MRW / pCN / two-level delayed acceptance with exact "
-                     "equality only (no adaptive proposal, adaptive error model or third level)", YG_MAX_DIM, YG_MAX_DATA_DIM);
+    if (c.adaptive || c.eq_mode != YG_EQ_EXACT || c.aem || nl > 3) {
+        yg_set_error("large linear model (dim > %d or data_dim > %d): MRW / pCN / MLDA with up to two surrogates with "
+                     "exact equality only (no adaptive proposal or adaptive error model)", YG_MAX_DIM, YG_MAX_DATA_DIM);
         return YG_ERR_UNSUPPORTED;
     }
-    for (int l = 0; l < nl; l++)
-        if (pb->level[l].tempered) {
-            yg_set_error("large linear model: tempered levels are not implemented");
-            return YG_ERR_UNSUPPORTED;
-        }
     const bool dense_L = !is_diagonal(pb->prop_L, d);
     const int kp = d <= 16 ? 16 : (d <= 32 ? 32 : 64), ks = kp + 4;
-    int np_l[2] = {0, 0};                 // operand rows per level, rounded up to 16
-    bool dense_prior[2] = {false, false};
-    std::vector<double> Rp[2];            // chol(prior precision)' of the levels with a dense prior
+    int np_l[3] = {0, 0, 0};              // operand rows per level, rounded up to 16
+    bool dense_prior[3] = {false, false, false};
+    double temper[3] = {1.0, 1.0, 1.0};   // tempering of each level (target.py:40-43)
+    std::vector<double> Rp[3];            // chol(prior precision)' of the levels with a dense prior
     for (int l = 0; l < nl; l++) {
         const yg_level &L = pb->level[l];
         if (!L.data || !L.noise_prec || !L.prior_mean || !L.prior_prec || !L.G || !L.b || L.n_data < 1 ||
             L.data_dim < 1) {
             yg_set_error("level %d: linear level needs data, noise_prec, prior, G and b", l);
             return YG_ERR_INVALID;
+        }
+        if (L.tempered) {
+            if (!(L.tempering >= 0.0 && L.tempering <= 1.0)) {       // tmlda.py:24-29
+                yg_set_error("Invalid tempering parameter at index %d: %g (must be in [0, 1]).", l, L.tempering);
+                return YG_ERR_INVALID;
+            }
+            temper[l] = L.tempering;
         }
         if (L.data_dim > YG_BIG_MAX_DATA_DIM) {
             yg_set_error("level %d: large linear model is limited to data_dim <= %d", l, YG_BIG_MAX_DATA_DIM);
@@ -250,7 +253,7 @@ int build_big_blob(const yg_config &c, const yg_problem *pb, std::vector<char> &
     }
     // operands that leave too little shared memory for BIG_MIN_WARPS warps are read from this blob's global copy
     // (smem_plan.h: big_tensor_plan); inside the envelope that always suffices, so the refusal is a safety check only
-    const BigTensorPlan plan = big_tensor_plan(np_l[0], np_l[1], kp / 4, dense_L, false);
+    const BigTensorPlan plan = big_tensor_plan(np_l[0], np_l[1], kp / 4, dense_L, false, np_l[2]);
     if (plan.smem.warps < BIG_MIN_WARPS) {
         yg_set_error("large linear model: %zu bytes of G / data do not fit the shared memory of one SM",
                      sizeof(double) * (size_t)plan.resident);
@@ -261,7 +264,7 @@ int build_big_blob(const yg_config &c, const yg_problem *pb, std::vector<char> &
     DevBigHeader *h = reinterpret_cast<DevBigHeader *>(blob.data());
     double *tail = reinterpret_cast<double *>(blob.data() + sizeof(DevBigHeader));
     h->dim = d; h->kp = kp; h->ks = ks; h->n_levels = nl;
-    h->J = nl == 2 ? c.sub_chain_length : 1;
+    h->J = nl >= 2 ? c.sub_chain_length : 1;
     h->tail_len = (int32_t)tail_len;
     h->proposal = pb->proposal;
     h->dense_L = dense_L ? 1 : 0;
@@ -285,11 +288,13 @@ int build_big_blob(const yg_config &c, const yg_problem *pb, std::vector<char> &
         const int rows = L.data_dim + (dense_prior[l] ? d : 0);
         const int np = np_l[l];
         B.n_data = L.n_data; B.data_dim = L.data_dim; B.np = np; B.n_rows = rows;
-        B.G_off = place((size_t)np * ks, l == 1 ? BIG_STREAM_G1 : 0);
+        B.G_off = place((size_t)np * ks, l == 1 ? BIG_STREAM_G1 : (l == 2 ? BIG_STREAM_G2 : 0));
         B.bd_off = place((size_t)np, 0);
         const size_t goff = (size_t)B.G_off;
         // sum_rows ||F - d_row||^2_P = sum_col n P_col (F_col - mean_col)^2 + sum_col P_col sum_rows (d - mean)^2;
-        // sqrt(n P_col) is folded into row `col` of G and into b - mean
+        // sqrt(n P_col) is folded into row `col` of G and into b - mean.  A tempered level scales the data rows by
+        // fl(sqrt(t)) and q_const by t (t = 1: both factors are exactly 1, the operands those of an untempered level).
+        const double st = sqrt(temper[l]);
         double q_const = 0.0;
         for (int r = 0; r < L.data_dim; r++) {
             double mean = 0.0;
@@ -301,7 +306,7 @@ int build_big_blob(const yg_config &c, const yg_problem *pb, std::vector<char> &
                 scatter += dd * dd;
             }
             const double prec = L.noise_prec[(size_t)r * L.data_dim + r];
-            const double sw = sqrt((double)L.n_data * prec);
+            const double sw = st * sqrt((double)L.n_data * prec);
             for (int k = 0; k < d; k++) tail[goff + (size_t)r * ks + k] = sw * L.G[(size_t)r * d + k];
             tail[B.bd_off + r] = sw * (L.b[r] - mean);
             q_const += prec * scatter;
@@ -316,7 +321,7 @@ int build_big_blob(const yg_config &c, const yg_problem *pb, std::vector<char> &
                 tail[B.bd_off + L.data_dim + r] = -rm;
             }
         }
-        B.q_const = q_const;
+        B.q_const = temper[l] * q_const;
         B.pmean_off = place(kp, 0);
         for (int k = 0; k < d; k++) tail[B.pmean_off + k] = L.prior_mean[k];
         B.pprec_off = place(kp, 0);
@@ -366,9 +371,8 @@ extern "C" int yg_create(const yg_config *cfg, yg_ensemble **out)
                      "exist on the device", cfg->n_levels);
         return YG_ERR_UNSUPPORTED;
     }
-    if (cfg->n_levels == 3 && (cfg->model == YG_MODEL_LV_RK4 || cfg->aem || cfg->dim > YG_MAX_DIM)) {
-        yg_set_error("three levels: Gaussian targets and the linear model (dim <= %d) only, no adaptive error model",
-                     YG_MAX_DIM);
+    if (cfg->n_levels == 3 && (cfg->model == YG_MODEL_LV_RK4 || cfg->aem)) {
+        yg_set_error("three levels: Gaussian targets and the linear model only, no adaptive error model");
         return YG_ERR_UNSUPPORTED;
     }
     if (cfg->n_levels >= 2 && cfg->sub_chain_length < 1) {

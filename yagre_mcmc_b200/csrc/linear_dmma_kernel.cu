@@ -303,7 +303,7 @@ template <int KQ, typename SIDE>
 YG_DEVFN double logpost_tile_streamed(const SmemLevel &L, const int ks, const double (&a)[KQ], const int g, const int t,
                                       SIDE &&side, const StreamTail &st)
 {
-    constexpr int D = STREAM_DEPTH < KQ ? STREAM_DEPTH : KQ - 1;       // (only KQ = 16 runs it)
+    constexpr int D = STREAM_DEPTH < KQ ? STREAM_DEPTH : KQ - 1;       // (KQ = 16, and 8 for three levels)
     double qa = 0.0, qb = 0.0;
     auto epilogue = [&](const int nb, const double c0, const double c1, const double c2, const double c3) {
         const double b0 = L.bd[nb + g], b1 = L.bd[nb + 8 + g];
@@ -421,11 +421,13 @@ YG_DEVFN void lz_streamed(const double *Ld, const int ks, const double (&zv)[KQ]
 // paths of the parity tests and the DENSE proposal factor (p = s + L z with L z as a second small GEMM) live in the
 // FREE_NOISE = false instance, which keeps the step loop of the production one small enough for the instruction cache
 // (stall reason no_instruction in profiles/r01_linear_dmma.md).
-// STREAMED = true: the operands of H.stream (smem_plan.h: big_tensor_plan: the target level's G, the dense factor) are
-// read from the global blob, and only the prefix of sp.blob bytes is staged.  Level 0's G -- J evaluations per
-// transition, under which the next proposal's noise is drawn -- always stays in shared memory.  Instantiated at KQ = 16
-// only, the one width whose blobs can outgrow shared memory.
-template <int KQ, bool TWO_LEVEL, bool FREE_NOISE, bool STREAMED = false>
+// NL: levels -- 1 (MRW / pCN), 2 (two-level delayed acceptance) or 3 (MLDA with two surrogates: the sub-chain on level
+// 0, the screen on level 1 in place of level 0, generic_kernel.cuh's three-level step).
+// STREAMED = true: the operands of H.stream (smem_plan.h: big_tensor_plan: the G of levels 1 and 2, the dense factor)
+// are read from the global blob, and only the prefix of sp.blob bytes is staged.  Level 0's G -- J evaluations per
+// transition, under which the next proposal's noise is drawn -- always stays in shared memory.  Instantiated at KQ = 16,
+// and for three levels at KQ = 8: the widths whose blobs can outgrow shared memory.
+template <int KQ, int NL, bool FREE_NOISE, bool STREAMED = false>
 __global__ void __launch_bounds__(big_max_warps(KQ) * 32, 1) linear_dmma_mh_kernel(const RunArgs a, const DevBigHeader *gh,
                                                                           long long *tile_done, const BigSmemPlan sp)
 {
@@ -439,10 +441,13 @@ __global__ void __launch_bounds__(big_max_warps(KQ) * 32, 1) linear_dmma_mh_kern
     for (int i = tid; i < staged; i += blockDim.x) smem[i] = gtail[i];
     __syncthreads();
     const StreamTail stail{gtail, H.tail_len};
-    SmemLevel Lv[2];
+    constexpr bool TWO_LEVEL = NL >= 2;             // a sub-chain on level 0 and a screen above it
+    constexpr int NLV = NL < 2 ? 2 : NL;
+    auto g_bit = [](const int l) { return l == 1 ? BIG_STREAM_G1 : (l == 2 ? BIG_STREAM_G2 : 0); };
+    SmemLevel Lv[NLV];
 #pragma unroll
-    for (int l = 0; l < 2; l++) {
-        Lv[l].G = ((STREAMED && l == 1 && (H.stream & BIG_STREAM_G1)) ? gtail : smem) + H.lvl[l].G_off;
+    for (int l = 0; l < NLV; l++) {
+        Lv[l].G = ((STREAMED && (H.stream & g_bit(l))) ? gtail : smem) + H.lvl[l].G_off;
         Lv[l].bd = smem + H.lvl[l].bd_off;
         Lv[l].pmean = smem + H.lvl[l].pmean_off;
         Lv[l].pprec = smem + H.lvl[l].pprec_off;
@@ -455,7 +460,7 @@ __global__ void __launch_bounds__(big_max_warps(KQ) * 32, 1) linear_dmma_mh_kern
     // current state of the warp's 8 chains: [8][ks] doubles after the problem blob; lane (g, t) only ever
     // touches its own slots (row g, columns 4 i + t), so no synchronisation is needed, and the row stride
     // (4 mod 16 doubles) makes the accesses bank-conflict free
-    const int d = H.dim, ks = H.ks, J = TWO_LEVEL ? H.J : 1, n_lvl = TWO_LEVEL ? 2 : 1;
+    const int d = H.dim, ks = H.ks, J = TWO_LEVEL ? H.J : 1, n_lvl = NL;
     constexpr int ZS = big_zs(KQ);
     const int n_warps = blockDim.x >> 5;
     const bool dense_L = !FREE_NOISE && H.dense_L;
@@ -507,6 +512,7 @@ __global__ void __launch_bounds__(big_max_warps(KQ) * 32, 1) linear_dmma_mh_kern
             TH(i) = (k < d) ? __ldcg(a.theta + (int64_t)k * N + gg) : 0.0;
         }
         double lp0 = __ldcg(a.logpost + gg), lp1 = TWO_LEVEL ? __ldcg(a.logpost + N + gg) : 0.0;
+        double lp2 = NL == 3 ? __ldcg(a.logpost + 2 * N + gg) : 0.0;
         unsigned long long nacc = __ldcg(a.n_accept + gg);
 
         // Welford (estimation.py:36-53, diagonal M2) in run-length form: a chain that stays at x for m
@@ -722,10 +728,22 @@ __global__ void __launch_bounds__(big_max_warps(KQ) * 32, 1) linear_dmma_mh_kern
                 for (int i = 0; i < KQ; i++) same = same && (s[i] == TH(i));
                 const unsigned m = __ballot_sync(0xffffffffu, same);
                 const bool moved = (((m >> (4 * g)) & 0xFu) != 0xFu) && live;
-                double lpf = 0.0;
+                double lpf = 0.0, lpm = 0.0;
                 if (__any_sync(0xffffffffu, moved)) {
-                    lpf = (STREAMED && (H.stream & BIG_STREAM_G1)) ? logpost_tile_streamed<KQ>(Lv[1], ks, s, g, t, SideNone{}, stail)
-                                                                    : logpost_tile<KQ>(Lv[1], ks, s, g, t, SideNone{});
+                    if constexpr (NL == 3) {
+                        // the finest surrogate, then the target, from ONE call site (two inlined evaluations spill)
+#pragma unroll 1
+                        for (int l = 1; l < 3; l++) {
+                            const SmemLevel &L = l == 1 ? Lv[1] : Lv[2];
+                            const double v = (STREAMED && (H.stream & g_bit(l)))
+                                                 ? logpost_tile_streamed<KQ>(L, ks, s, g, t, SideNone{}, stail)
+                                                 : logpost_tile<KQ>(L, ks, s, g, t, SideNone{});
+                            if (l == 1) lpm = v; else lpf = v;
+                        }
+                    } else {
+                        lpf = (STREAMED && (H.stream & BIG_STREAM_G1)) ? logpost_tile_streamed<KQ>(Lv[1], ks, s, g, t, SideNone{}, stail)
+                                                                        : logpost_tile<KQ>(Lv[1], ks, s, g, t, SideNone{});
+                    }
                     if (moved) {
                         if (t == 0) cnt_ev1++;
                         double u;
@@ -734,7 +752,9 @@ __global__ void __launch_bounds__(big_max_warps(KQ) * 32, 1) linear_dmma_mh_kern
                             u = philox_uniform(a.seed, gid, step, YG_SUB_FINE);
                             if (noise_mode == YG_NOISE_RECORD && t == 0) a.u_f[n * N + gg] = u;
                         }
-                        const double delta = lpf + lp0 - lps - lp1;     // mlda.py:148-152, this order
+                        // mlda.py:148-152, this order; with two surrogates the screen's coarse density is the FINEST
+                        // surrogate although the sub-chain ran on level 0 (mlda.py:130,146-154)
+                        const double delta = NL == 3 ? lpf + lp1 - lpm - lp2 : lpf + lp0 - lps - lp1;
                         accepted = accept_rule(delta, u);
                     }
                 }
@@ -743,7 +763,7 @@ __global__ void __launch_bounds__(big_max_warps(KQ) * 32, 1) linear_dmma_mh_kern
 #pragma unroll
                     for (int i = 0; i < KQ; i++) TH(i) = s[i];
                     lp0 = lps;
-                    lp1 = lpf;
+                    if (NL == 3) { lp1 = lpm; lp2 = lpf; } else lp1 = lpf;
                 }
             }
             if (live) {
@@ -763,6 +783,7 @@ __global__ void __launch_bounds__(big_max_warps(KQ) * 32, 1) linear_dmma_mh_kern
                     if (a.lp_out && t == 0) {
                         a.lp_out[(o * n_lvl) * N + gr] = lp0;
                         if (TWO_LEVEL) a.lp_out[(o * n_lvl + 1) * N + gr] = lp1;
+                        if (NL == 3) a.lp_out[(o * n_lvl + 2) * N + gr] = lp2;
                     }
                 }
             }
@@ -782,6 +803,7 @@ __global__ void __launch_bounds__(big_max_warps(KQ) * 32, 1) linear_dmma_mh_kern
             if (t == 0) {
                 a.logpost[gr] = lp0;
                 if (TWO_LEVEL) a.logpost[N + gr] = lp1;
+                if (NL == 3) a.logpost[2 * N + gr] = lp2;
                 a.n_accept[gr] = nacc;
             }
         }
@@ -825,12 +847,15 @@ __global__ void __launch_bounds__(big_max_warps(KQ) * 32, 1) linear_dmma_mh_kern
 #undef WM
 #undef WV
     // ---- counters: warp-shuffle reduction, one atomic per warp ----------------------------------
-    unsigned long long v[5] = {cnt_tr, cnt_acc, cnt_ev0, cnt_ev1, cnt_cacc};
+    // slots (yg_get_counters): transitions, accepted, level-0 evaluations, target evaluations, level-1 evaluations of
+    // three levels (the same chains evaluate both upper levels), coarse accepts
+    unsigned long long v[6] = {cnt_tr, cnt_acc, cnt_ev0, cnt_ev1, cnt_ev1, cnt_cacc};
 #pragma unroll
-    for (int k = 0; k < 5; k++) {
+    for (int k = 0; k < 6; k++) {
+        if (NL < 3 && k == 4) continue;
 #pragma unroll
         for (int o = 16; o > 0; o >>= 1) v[k] += __shfl_xor_sync(0xffffffffu, v[k], o);
-        if (lane == 0 && v[k]) atomicAdd(&a.counters[k == 4 ? 5 : k], v[k]);
+        if (lane == 0 && v[k]) atomicAdd(&a.counters[k], v[k]);
     }
 }
 
@@ -886,23 +911,33 @@ int launch_t(yg_ensemble *e, const RunArgs &a, cudaStream_t st)
     // warps per CTA: as many as the shared memory left by the staged part of the problem blob holds (at most 12 for
     // d > 32, else 16; yg_set_problem streamed operands until BIG_MIN_WARPS fit); Welford moments of the tiles in shared
     // memory when that costs no warp (and FullDiagnostics asked for them at all)
-    const bool two = e->cfg.n_levels == 2;
-    const BigTensorPlan tp = big_tensor_plan(hh->lvl[0].np, two ? hh->lvl[1].np : 0, KQ, hh->dense_L != 0, a.welford != 0);
+    const int nl = e->cfg.n_levels;
+    const BigTensorPlan tp = big_tensor_plan(hh->lvl[0].np, nl >= 2 ? hh->lvl[1].np : 0, KQ, hh->dense_L != 0,
+                                             a.welford != 0, nl == 3 ? hh->lvl[2].np : 0);
     const BigSmemPlan sp = tp.smem;
     const bool free_noise = a.noise_mode == YG_NOISE_PHILOX && !hh->dense_L;      // the general instance also knows dense factors
-    decltype(&linear_dmma_mh_kernel<KQ, true, true>) kern;
+    decltype(&linear_dmma_mh_kernel<KQ, 2, true>) kern;
     if (tp.stream) {
-        // streamed instances: KQ = 16 only; one level streams only the dense factor (general instance)
+        // streamed instances: KQ = 16, and KQ = 8 for three levels; one level streams only the dense factor (general
+        // instance)
         if constexpr (KQ == 16) {
-            kern = two ? (free_noise ? linear_dmma_mh_kernel<KQ, true, true, true> : linear_dmma_mh_kernel<KQ, true, false, true>)
-                       : linear_dmma_mh_kernel<KQ, false, false, true>;
+            kern = nl == 3 ? (free_noise ? linear_dmma_mh_kernel<KQ, 3, true, true> : linear_dmma_mh_kernel<KQ, 3, false, true>)
+                 : nl == 2 ? (free_noise ? linear_dmma_mh_kernel<KQ, 2, true, true> : linear_dmma_mh_kernel<KQ, 2, false, true>)
+                           : linear_dmma_mh_kernel<KQ, 1, false, true>;
+        } else if constexpr (KQ == 8) {
+            if (nl != 3) {
+                yg_set_error("large linear model: streamed operands of fewer than three levels need d > 32");
+                return YG_ERR_STATE;
+            }
+            kern = free_noise ? linear_dmma_mh_kernel<KQ, 3, true, true> : linear_dmma_mh_kernel<KQ, 3, false, true>;
         } else {
-            yg_set_error("large linear model: streamed operands need d > 32");
+            yg_set_error("large linear model: streamed operands need d > 16");
             return YG_ERR_STATE;
         }
     } else {
-        kern = two ? (free_noise ? linear_dmma_mh_kernel<KQ, true, true> : linear_dmma_mh_kernel<KQ, true, false>)
-                   : (free_noise ? linear_dmma_mh_kernel<KQ, false, true> : linear_dmma_mh_kernel<KQ, false, false>);
+        kern = nl == 3 ? (free_noise ? linear_dmma_mh_kernel<KQ, 3, true> : linear_dmma_mh_kernel<KQ, 3, false>)
+             : nl == 2 ? (free_noise ? linear_dmma_mh_kernel<KQ, 2, true> : linear_dmma_mh_kernel<KQ, 2, false>)
+                       : (free_noise ? linear_dmma_mh_kernel<KQ, 1, true> : linear_dmma_mh_kernel<KQ, 1, false>);
     }
     YG_CUDA_CHECK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sp.total));
     const int64_t tiles = (a.n_chains + 7) / 8;

@@ -163,19 +163,21 @@ __host__ __device__ inline BigSmemPlan big_smem_plan(int tail_len, int ks, int k
 }
 
 // Operands that the tensor path may leave in the global copy of the blob (read through L2 with ld.global.nc) when the
-// whole blob leaves room for fewer than BIG_MIN_WARPS warps, in the order they are moved out: the target level's G of
-// two levels (evaluated at most once per transition, only when the sub-chain moved; level 0 is evaluated J times), then
-// the dense proposal factor (J times per transition, but only kp x ks).  With both out, every problem of the envelope
-// (d <= 64, data_dim <= 256, dense prior and factor, two levels) fits with BIG_MIN_WARPS warps or more
-// (tests/test_tensor_path_streamed_cpu.py), so level 0's G always stays in shared memory.  bd, pmean, pprec, propL and
-// pcn_mean always stay there too.
-enum BigStream { BIG_STREAM_G1 = 1, BIG_STREAM_LD = 2 };
+// whole blob leaves room for fewer than BIG_MIN_WARPS warps, in the order they are moved out: level 1's G, then level
+// 2's G of three levels (each evaluated at most once per transition, only when the sub-chain moved; level 0 is evaluated
+// J times), then the dense proposal factor (J times per transition, but only kp x ks).  With all of them out, every
+// problem of the envelope (d <= 64, data_dim <= 256 per level, dense prior and factor, up to three levels) fits with
+// BIG_MIN_WARPS warps or more (tests/test_tensor_path_streamed_cpu.py, tests/test_tensor_path_three_level_cpu.py), so
+// level 0's G always stays in shared memory.  bd, pmean, pprec, propL and pcn_mean always stay there too.  Two levels
+// stream only at d > 32; three levels of 256 data rows outgrow shared memory from d = 32 on, so three levels also
+// stream at 16 < d <= 32.
+enum BigStream { BIG_STREAM_G1 = 1, BIG_STREAM_LD = 2, BIG_STREAM_G2 = 4 };
 
 struct BigTensorPlan {
     BigSmemPlan smem;   // the plan of the staged (resident) part of the blob
     int stream;         // BigStream bits of the operands read from global memory
     int resident;       // doubles of the tail staged into shared memory: a prefix of the tail
-    int tail;           // doubles of the whole tail; the streamed operands follow the prefix, G1 before Ld
+    int tail;           // doubles of the whole tail; the streamed operands follow the prefix, G1 before G2 before Ld
 };
 
 // Doubles of the tail of one level (G, b - mean, prior mean and precision) and of the shared part (diagonal factor,
@@ -183,27 +185,29 @@ struct BigTensorPlan {
 __host__ __device__ constexpr int big_level_doubles(int np, int kp) { return np * (kp + 4) + np + 2 * kp; }
 __host__ __device__ constexpr int big_shared_doubles(int kp, bool dense_L) { return 2 * kp + (dense_L ? kp * (kp + 4) : 0); }
 
-// The plan of the tensor path.  np0, np1: operand rows of levels 0 and 1 (multiples of 16; np1 = 0 for one level).
-// Nothing is streamed while the whole blob leaves BIG_MIN_WARPS warps: the plan is then big_smem_plan of the whole
-// blob.  Otherwise operands move out in BigStream's order until it does; the staged prefix is rounded up to 32 bytes, so
-// every streamed operand starts on a whole sector (G rows and Ld rows are ks = 4 mod 16 doubles: 32-byte multiples).
-__host__ __device__ inline BigTensorPlan big_tensor_plan(int np0, int np1, int kq, bool dense_L, bool welford)
+// The plan of the tensor path.  np0, np1, np2: operand rows of levels 0, 1 and 2 (multiples of 16; np1 = 0 for one
+// level, np2 = 0 for fewer than three).  Nothing is streamed while the whole blob leaves BIG_MIN_WARPS warps: the plan is
+// then big_smem_plan of the whole blob.  Otherwise operands move out in BigStream's order until it does; the staged
+// prefix is rounded up to 32 bytes, so every streamed operand starts on a whole sector (G rows and Ld rows are
+// ks = 4 mod 16 doubles: 32-byte multiples).  With np2 = 0 the plan is the two-level one, field for field.
+__host__ __device__ inline BigTensorPlan big_tensor_plan(int np0, int np1, int kq, bool dense_L, bool welford, int np2 = 0)
 {
     const int kp = 4 * kq, ks = kp + 4;
-    const int raw = big_level_doubles(np0, kp) + (np1 ? big_level_doubles(np1, kp) : 0) + big_shared_doubles(kp, dense_L);
+    const int raw = big_level_doubles(np0, kp) + (np1 ? big_level_doubles(np1, kp) : 0) +
+                    (np2 ? big_level_doubles(np2, kp) : 0) + big_shared_doubles(kp, dense_L);
     BigTensorPlan p;
     p.stream = 0;
     p.resident = p.tail = (raw + 1) & ~1;
     p.smem = big_smem_plan(p.resident, ks, kq, dense_L, welford);
-    const int order[2] = {BIG_STREAM_G1, BIG_STREAM_LD};
-    const int size[2] = {np1 * ks, dense_L ? kp * ks : 0};
+    const int order[3] = {BIG_STREAM_G1, BIG_STREAM_G2, BIG_STREAM_LD};
+    const int size[3] = {np1 * ks, np2 * ks, dense_L ? kp * ks : 0};
     int staged = raw;
 #ifdef YG_STREAM_ALWAYS
     const int need = big_max_warps(kq) + 1;     // dev builds (measurement): stream every operand that can be streamed
 #else
     const int need = BIG_MIN_WARPS;
 #endif
-    for (int i = 0; i < 2 && p.smem.warps < need; i++) {
+    for (int i = 0; i < 3 && p.smem.warps < need; i++) {
         if (size[i] == 0) continue;
         p.stream |= order[i];
         staged -= size[i];
